@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # our arm (torchrun launches N ranks for N > 1)
   python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU path (oracle port) on host cores
+  python bench.py --steps K --dump-outputs DIR              # also save what the timed steps computed (DIR/<name>.npy)
 
 A "step" is one training step (forward + discriminator-weighted BCE + backward + gradient all-reduce +
 Adam) of the reference SRFR model on Beauty-shaped synthetic data, config C2 of BASELINE.json:
@@ -37,6 +38,26 @@ sys.path.insert(0, ROOT)
 
 METRIC = "training seqs/sec; full-catalogue top-10 users/sec"
 CFG = dict(kind="SRFR", usernum=22363, itemnum=12101, L=50, D=64, F=16, blocks=2, heads=1, batch=4096)
+DUMP_LIMIT = 64 << 20          # bytes --dump-outputs may write in all
+
+
+def write_outputs(out_dir, arrays):
+    """--dump-outputs: save each array as out_dir/<name>.npy so that two builds can be compared output for output.
+    Floating arrays become float32 (float64 stays float64), integer ids float64 (exact below 2**53).  Raises before writing
+    anything if the arrays exceed DUMP_LIMIT bytes in all; returns the bytes written."""
+    conv = {}
+    for name, a in arrays.items():
+        t = torch.as_tensor(a).detach()
+        if t.dtype != torch.float64:
+            t = t.float() if t.is_floating_point() else t.double()
+        conv[name] = t.cpu().numpy()
+    total = sum(a.nbytes for a in conv.values())
+    if total > DUMP_LIMIT:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in conv.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return total
 
 
 def peaks():
@@ -473,6 +494,13 @@ def run_ours(args):
     clk.start()
     ms = timed(dev_step, args.steps, W)
     clocks = clk.stop()
+    dump = {} if args.dump_outputs and rank == 0 else None
+    if dump is not None:
+        # what the last timed step returns to its caller: the loss (read now: the e2e run below keeps training).  The
+        # parameters are not saved: gradients are summed with float atomics and Adam turns that rounding into +-lr steps
+        # wherever a gradient is ~0 (the key bias of in_proj_bias is 0 analytically), so after a few steps two correct
+        # runs differ there by far more than rounding while the loss agrees to ~1e-6.
+        dump["train_loss"] = tr.loss_dev.reshape(1).cpu()
     ms_e2e = timed(host_step, args.steps, W)
     value = world * B * args.steps / (ms / 1e3)
     e2e = world * B * args.steps / (ms_e2e / 1e3)
@@ -525,7 +553,7 @@ def run_ours(args):
     # ---- catalogue: C3, 1 M items row-sharded, U = 16384 users ----
     cat = None
     if not args.no_catalogue:
-        cat = guarded(bench_catalogue, dev, rank, world, pg, args, pk, timed)
+        cat = guarded(bench_catalogue, dev, rank, world, pg, args, pk, timed, dump)
 
     # ---- gather: K1 on the C3 item table (1 M rows x 64 fp32 = 256 MB > L2), 4 M tokens, every slot valid ----
     gat = None
@@ -569,6 +597,8 @@ def run_ours(args):
             line["cpu_baseline"] = cpu
         if eager is not None:
             line["gpu_eager_baseline"] = eager
+        if dump is not None:
+            write_outputs(args.dump_outputs, dump)
         print(json.dumps(line), flush=True)
     if world > 1:
         # Tear down without dist.destroy_process_group(): with the NCCL all-reduce captured inside live CUDA graphs the
@@ -677,11 +707,12 @@ def bench_scale_kernels(dev, pk):
     return out
 
 
-def bench_catalogue(dev, rank, world, pg, args, pk, timed):
+def bench_catalogue(dev, rank, world, pg, args, pk, timed, dump=None):
     """C3: (a) score + top-k + all-gather + merge on given user representations (the roofline-graded part), (b) the same
     preceded by the sequence encoder on 16 384 Beauty-shaped sequences over the 1 M-item catalogue (SURVEY 8d metric 2:
     encode + score + top-k + all-gather + merge).  The table is row-sharded; the users are split over the ranks for the encode
-    and their representations all-gathered (EV.encode_users)."""
+    and their representations all-gathered (EV.encode_users).  `dump` (a dict) receives the top-10 scores and global item
+    ids of the last timed pass of (a) and (b)."""
     from srfrd_b200 import evaluation as EV, synth, _lib
     N, D, U = 1_000_000, 64, 16384
     lo, hi = EV.CatalogueIndex.shard_bounds(N + 1, rank, world)
@@ -706,6 +737,9 @@ def bench_catalogue(dev, rank, world, pg, args, pk, timed):
     steps = max(3, min(args.steps, 10))
     ms = timed(step, steps, 3)
     ms_enc = timed(step_enc, steps, 3)
+    if dump is not None:
+        dump["catalogue_scores"], dump["catalogue_ids"] = (t.cpu() for t in out["r"])
+        dump["catalogue_encode_scores"], dump["catalogue_encode_ids"] = (t.cpu() for t in out["e"])
     users_s = U * steps / (ms / 1e3)
     flops = 2.0 * U * (hi - lo) * D
     # kernel-only time of the scoring kernel on this rank
@@ -833,7 +867,12 @@ def main():
     ap.add_argument("--no-catalogue", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the C4 / C5 / dropout objects")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, save the loss of the last training step and the top-10 scores / ids of "
+                         "the last catalogue passes as DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs saves what the product's timed path computed: use it with --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     world = int(os.environ.get("WORLD_SIZE", 1))
