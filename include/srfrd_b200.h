@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define SRFRD_ABI_VERSION 5
+#define SRFRD_ABI_VERSION 6
 #if defined(__GNUC__)
 #define SRFRD_API __attribute__((visibility("default")))
 #else
@@ -287,13 +287,24 @@ SRFRD_API int srfrd_layernorm_fwd_rows(const void* x_bf16, int ldx, const float*
                              int ldy, const int* row_index, int64_t n, int H, void* stream);
 /* Causal attention over packed rows (tcgen05; L + 1 <= 128, head width a multiple of 16, one head or 64-column heads). */
 SRFRD_API int srfrd_attention_packed_supported(int L, int H, int heads);
+/* Whether the packed kernels can fold the attention out-projection in (SRFR_model.py:112-113, the out_proj of
+ * F.multi_head_attention_forward): bit 0 forward, bit 1 backward.  Needs one head of at most 128 columns. */
+SRFRD_API int srfrd_attention_packed_oproj_supported(int L, int H, int heads);
+/* Trailing arguments (wo NULL: plain attention, o only): fused out-projection, residual add and LayerNorm, each row
+ * exactly what srfrd_gemm_tn(o, wo, bias = bo, residual = res, ln_out = y, ...) computes:
+ *     r = o wo^T + bo + res,   y = LayerNorm(r) * ln_w + ln_b,   ln_stats = (mean, rstd) per row     (bo, ln_stats nullable)
+ * wo: the [H, H] weight (rows = output features, K-major), ldw its row pitch.  o is still written. */
 SRFRD_API int srfrd_attention_fwd_packed(const void* q, int ldq, const void* k, const void* v, int ldkv, void* o, int ldo,
                                const srfrd_pack_t* pk, int L, int H, int heads, float drop_p, uint64_t seed,
-                               uint32_t stream_id, const float* drop_step, void* stream);
+                               uint32_t stream_id, const float* drop_step, void* stream, const void* wo, int ldw,
+                               const float* bo, const void* res, int ldres, const float* ln_w, const float* ln_b,
+                               float ln_eps, float* ln_stats, void* r, int ldr, void* y, int ldy);
+/* Trailing arguments (dr NULL: dout is read): dout = dr woT^T is computed in the kernel (what srfrd_gemm_tn(dr, woT)
+ * writes) and dout / lddo are ignored.  woT: the transposed [H, H] out-projection weight, ldw its row pitch. */
 SRFRD_API int srfrd_attention_bwd_packed(const void* dout, int lddo, const void* q, int ldq, const void* k, const void* v,
                                int ldkv, void* dq, int lddq, void* dk, void* dv, int lddkv, const srfrd_pack_t* pk,
                                int L, int H, int heads, float drop_p, uint64_t seed, uint32_t stream_id,
-                               const float* drop_step, void* stream);
+                               const float* drop_step, void* stream, const void* dr, int lddr, const void* woT, int ldw);
 /* K4 on the packed layout: h / dh are packed rows; ids, weights stay (B * L) dense and are reached through row_tok. */
 SRFRD_API int srfrd_score_loss_fused_packed(const float* h, int ldh, const float* item_table, const float* fake_table,
                                   const int64_t* pos, const int64_t* neg, const int64_t* prs, const int64_t* nrs,

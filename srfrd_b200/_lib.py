@@ -94,9 +94,11 @@ SIGNATURES = {
                                   f32, u64, u32, vp, vp, vp, i64, vp],
     "srfrd_layernorm_fwd_rows": [vp, i32, vp, vp, f32, vp, i32, vp, i64, i32, vp],
     "srfrd_attention_packed_supported": [i32, i32, i32],
-    "srfrd_attention_fwd_packed": [vp, i32, vp, vp, i32, vp, i32, C.POINTER(PackDesc), i32, i32, i32, f32, u64, u32, vp, vp],
+    "srfrd_attention_packed_oproj_supported": [i32, i32, i32],
+    "srfrd_attention_fwd_packed": [vp, i32, vp, vp, i32, vp, i32, C.POINTER(PackDesc), i32, i32, i32, f32, u64, u32, vp, vp,
+                                   vp, i32, vp, vp, i32, vp, vp, f32, vp, vp, i32, vp, i32],
     "srfrd_attention_bwd_packed": [vp, i32, vp, i32, vp, vp, i32, vp, i32, vp, vp, i32, C.POINTER(PackDesc), i32, i32, i32,
-                                   f32, u64, u32, vp, vp],
+                                   f32, u64, u32, vp, vp, vp, i32, vp, i32],
     "srfrd_score_loss_fused_packed": [vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, vp, vp, i32, vp, vp, vp, vp,
                                       i64, vp],
     "srfrd_embed_bwd_packed": [vp, i32, vp, vp, vp, vp, i64, i32, i32, i32, i32, f32, vp, vp, vp, vp],
@@ -127,7 +129,7 @@ def load() -> C.CDLL:
         fn = getattr(lib, name)            # AttributeError if the symbol is not exported
         fn.argtypes = argtypes
         fn.restype = C.c_int
-    if lib.srfrd_abi_version() != 5:
+    if lib.srfrd_abi_version() != 6:
         raise RuntimeError("srfrd_b200: ABI version mismatch between _lib.py and the built library")
     _lib = lib
     return lib

@@ -49,6 +49,12 @@ struct AttnTc {
   const int* pk_rows;                     // device {M, T', n_tiles}
   const int4* pk_info;
   const int* pk_tile_row0;
+  // fused out-projection (packed layout, heads == 1; SRFR_model.py:112-113, the out_proj of F.multi_head_attention_forward
+  // and the residual + forward LayerNorm that follow it):
+  //   forward : r = o Wo^T + bo + res,  y = LayerNorm(r) * ln_w + ln_b,  ln_stats = (mean, rstd)   (o is still written)
+  //   backward: dO = dr Wo, computed in the kernel instead of read from memory
+  const float *op_bias, *ln_w, *ln_b; float* ln_stats; float ln_eps;
+  bf16 *op_r, *op_y; int ldr, ldy;
 };
 
 // byte offset of element (row r, column c) inside a [128 x 64] bf16 block with the 128-byte swizzle
@@ -199,6 +205,59 @@ __device__ __forceinline__ void store_staged_rows(bf16* dst, int ld, int64_t row
 
 static constexpr int AF_THREADS = 320;   // forward: 8 softmax / epilogue warps + TMA warp + MMA warp
 
+// Forward out-projection epilogue of one tile (OP), run by the 256 epilogue threads: thread (row r, part) takes the
+// 32-column chunks c = 32 part, 32 part + 64, ... of its row, as gemm_tn's LNF epilogue does (half = part), so the
+// partial row sums and their combination are the same.  On entry every thread has stored its share of o from Qs.
+__device__ __forceinline__ void out_proj_epilogue(const AttnTc& p, uint8_t* Qs, uint8_t* Vs, float* xsum, float* xsq,
+                                               const float* sop, uint32_t tacc, uint64_t* proj_full, uint64_t* w_full,
+                                               uint32_t ph, int r, int part, int quarter, int row0, int n_own) {
+  mbar_wait2(proj_full, ph, w_full, ph);   // r accumulator complete, residual tile landed
+  tc_fence_after();
+  float ln_sum = 0.f, ln_sq = 0.f;
+#pragma unroll 1
+  for (int c = part * 32; c < p.hd; c += 64) {
+    uint32_t raw[32];
+    tmem_ld32(tacc + c, raw);
+    uint8_t* blk = Vs + (c >> 6) * OPB;
+    uint4 ax[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+      if (c + 8 * j < p.hd) ax[j] = *reinterpret_cast<const uint4*>(blk + sw128(r, (c & 63) + 8 * j));
+    tmem_ld_wait();
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      if (c + 8 * j >= p.hd) break;
+      float v[8], a[8];
+      unpack_bf16x8(ax[j], a);
+#pragma unroll
+      for (int i = 0; i < 8; ++i) v[i] = (__uint_as_float(raw[8 * j + i]) + sop[c + 8 * j + i]) + a[i];
+      const uint4 pk = make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
+      *reinterpret_cast<uint4*>(blk + sw128(r, (c & 63) + 8 * j)) = pk;   // r in place over the residual
+      lnf_accum8(pk, ln_sum, ln_sq);
+    }
+  }
+  tc_fence_before();
+  xsum[part * TILE + r] = ln_sum;          // (the softmax's exchange arrays: every thread has read them)
+  xsq[part * TILE + r] = ln_sq;
+  named_bar_sync_a(9, 256);                // partner's partial sums visible; every thread has read o out of Qs
+  float mean, rstd, nb;
+  lnf_stats(ln_sum, ln_sq, xsum[(part ^ 1) * TILE + r], xsq[(part ^ 1) * TILE + r], p.hd, p.ln_eps, mean, rstd, nb);
+#pragma unroll 1
+  for (int c = part * 32; c < p.hd; c += 64) {
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      if (c + 8 * j >= p.hd) break;
+      const uint32_t off = (c >> 6) * OPB + sw128(r, (c & 63) + 8 * j);
+      *reinterpret_cast<uint4*>(Qs + off) =
+          lnf_apply8(*reinterpret_cast<const uint4*>(Vs + off), rstd, nb, sop + TILE + c + 8 * j, sop + 2 * TILE + c + 8 * j);
+    }
+  }
+  if (part == 0 && r < n_own && p.ln_stats) *reinterpret_cast<float2*>(p.ln_stats + 2 * (size_t)(row0 + r)) = make_float2(mean, rstd);
+  named_bar_sync_a(9, 256);                // r and y complete in Vs / Qs
+  store_staged_rows(p.op_r, p.ldr, row0, 0, Vs, p.hd, n_own, threadIdx.x);
+  store_staged_rows(p.op_y, p.ldy, row0, 0, Qs, p.hd, n_own, threadIdx.x);
+}
+
 // Forward, two CTAs per SM (smem <= 98 KB, 256 TMEM columns each): a tile is a chain of TMA -> S MMA -> softmax ->
 // PV MMA -> output latencies, so a second resident CTA fills the gaps.  Shared memory is reused in place: P overwrites
 // K (dead once S is complete), O overwrites Q and leaves through a TMA store whose box has exactly spt*L rows.
@@ -209,10 +268,18 @@ static constexpr int AF_THREADS = 320;   // forward: 8 softmax / epilogue warps 
 // 17 k-cycle tile -- single-warp instruction latency, not bandwidth.
 // Warp roles (320 threads): warps 0..7 softmax + epilogue (quarter = warp & 3, part = warp >> 2), warp 8 TMA,
 // warp 9 MMA (control warps have the highest ids: the scheduler favours them).
-template <bool DROP, bool PK>
+// Fused out-projection (OP, packed layout, heads == 1): once the PV MMA has released K's and V's blocks (kv_free), the TMA
+// warp loads Wo (B operand, hd rows x K = hd) into K's blocks and the residual tile into V's; the MMA warp multiplies the
+// staged O (Q's blocks, already the K-major A operand) by Wo^T into S's TMEM columns (dead since the softmax); the epilogue
+// adds bias and residual, writes r in place over the residual, normalises it into Q's blocks (y) and stores o, r, y and
+// the statistics of the tile's owned rows.  Same K order (64 + 16 at hd = 80), add order and LayerNorm arithmetic as
+// gemm_tn's LNF epilogue, so the results are bit-identical to the separate launch.  A tile is then done only when its
+// y has left: q_free alone gates the next item's loads.
+template <bool DROP, bool PK, bool OP>
 __global__ void __launch_bounds__(AF_THREADS, 2)
 attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
-                   const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmO, AttnTc p) {
+                   const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmO,
+                   const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmR, AttnTc p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const int opbytes = p.kblocks * OPB;
@@ -224,13 +291,17 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
   uint64_t* bars = reinterpret_cast<uint64_t*>(ssum + 2 * TILE);
   uint64_t *qk_full = bars, *v_full = bars + 1, *s_full = bars + 2, *p_full = bars + 3, *o_full = bars + 4,
            *kv_free = bars + 5, *q_free = bars + 6;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 8);
+  uint64_t *w_full = bars + 7, *o_staged = bars + 8, *proj_full = bars + 9;   // OP: Wo + residual landed, O staged, r ready
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 10);
+  float* sop = reinterpret_cast<float*>(bars + 16);        // OP: bias, LayerNorm weight, LayerNorm bias [3][TILE]
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
   if (warp == 8 && lane == 0) {
     tma_prefetch_desc(&tmQ); tma_prefetch_desc(&tmK); tma_prefetch_desc(&tmV); tma_prefetch_desc(&tmO);
+    if (OP) { tma_prefetch_desc(&tmW); tma_prefetch_desc(&tmR); }
     mbar_init(qk_full, 1); mbar_init(v_full, 1); mbar_init(s_full, 1); mbar_init(p_full, 8); mbar_init(o_full, 1);
     mbar_init(kv_free, 1); mbar_init(q_free, 1);
+    mbar_init(w_full, 1); mbar_init(o_staged, 1); mbar_init(proj_full, 1);
     fence_barrier_init();
   }
   if (warp == 9) { tmem_alloc(tmem_slot, 256); tmem_relinquish(); }
@@ -250,7 +321,7 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
       const int tile = it / p.heads, h = it % p.heads;
       const int row0 = PK ? __ldg(p.pk_tile_row0 + tile) : tile * p.spt * p.L, col0 = h * p.hd;
       mbar_wait(q_free, ph ^ 1);                   // O of the previous item has left Q's smem
-      mbar_wait(kv_free, ph ^ 1);                  // previous PV MMA is done with P (K's smem) and V
+      if (!OP) mbar_wait(kv_free, ph ^ 1);         // previous PV MMA is done with P (K's smem) and V (OP: implied)
       AT_STAMP(0, it / gridDim.x);
       if (elect_one()) {
         mbar_expect_tx(qk_full, 2 * opbytes);
@@ -265,10 +336,22 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
         //  compute, and the extra live values spill at the 96-register cap that two CTAs per SM impose)
       }
       __syncwarp();
+      if (OP) {
+        mbar_wait(kv_free, ph);                    // this item's PV MMA is done with K's and V's blocks
+        if (elect_one()) {
+          mbar_expect_tx(w_full, p.kblocks * (p.hd * 128 + OPB));
+          for (int kb = 0; kb < p.kblocks; ++kb) {
+            tma_load_2d(Ks + kb * OPB, &tmW, w_full, kb * 64, 0, SRFRD_EVICT_LAST);
+            tma_load_2d(Vs + kb * OPB, &tmR, w_full, kb * 64, row0, SRFRD_EVICT_FIRST);
+          }
+        }
+        __syncwarp();
+      }
     }
   } else if (warp == 9) {
     const uint32_t idS = umma_idesc_bf16(TILE, TILE, 0, 0);
     const uint32_t idO = umma_idesc_bf16(TILE, p.hd, 0, 1);
+    const uint32_t idW = umma_idesc_bf16(TILE, p.hd, 0, 0);       // OP: O Wo^T, both operands K-major
     const uint64_t dQ = umma_smem_desc(smem_u32(Qs), 0, 1024), dK = umma_smem_desc(smem_u32(Ks), 0, 1024);
     const uint64_t dP = umma_smem_desc(smem_u32(Ks), 0, 1024), dV = umma_smem_desc(smem_u32(Vs), OPB, 1024);
     uint32_t ph = 0;
@@ -299,6 +382,19 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
       }
       __syncwarp();
       AT_STAMP(4, it / gridDim.x);
+      if (OP) {                              // r = O Wo^T into S's columns: A = staged O (Q's blocks), B = Wo (K's blocks)
+        mbar_wait2(o_staged, ph, w_full, ph);
+        tc_fence_after();
+        if (elect_one()) {
+          for (int kb = 0; kb < p.kblocks; ++kb) {
+            const int ksteps = min(4, (p.hd - kb * 64) / 16);
+            for (int k = 0; k < ksteps; ++k)
+              umma_bf16(tS, dQ + (uint64_t)(kb * (OPB >> 4) + 2 * k), dK + (uint64_t)(kb * (OPB >> 4) + 2 * k), idW, (kb | k) != 0);
+          }
+          umma_commit(proj_full);
+        }
+        __syncwarp();
+      }
     }
   } else {
     const int quarter = warp & 3, part = warp >> 2;
@@ -308,6 +404,12 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
     const int r_first = quarter * 32;
     // packed layout: a sequence has at most L + 1 rows, so a row's window starts at most L columns before it
     const int c_lo = PK ? (max(0, r_first - p.L) >> 5) : min(((r_first / p.L) * p.L) >> 5, quarter), c_hi = quarter;
+    if (OP)                                // read by the epilogue only after several barriers of these 256 threads
+      for (int i = threadIdx.x; i < TILE; i += 256) {
+        sop[i] = (p.op_bias && i < p.hd) ? __ldg(p.op_bias + i) : 0.f;
+        sop[TILE + i] = i < p.hd ? __ldg(p.ln_w + i) : 0.f;
+        sop[2 * TILE + i] = i < p.hd ? __ldg(p.ln_b + i) : 0.f;
+      }
     uint32_t ph = 0;
     for (int it = blockIdx.x; it < n_items; it += gridDim.x, ph ^= 1) {
       const int tile = it / p.heads, h = it % p.heads;
@@ -414,8 +516,11 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
       named_bar_sync_a(9, 256);
       if (warp == 0) AT_STAMP(8, it / gridDim.x);
       if (PK) {
+        if (OP && warp == 0 && lane == 0) mbar_arrive(o_staged);   // the out-projection MMA may read O
         const int n_own = __ldg(p.pk_tile_row0 + tile + 1) - pk_row0;
         store_staged_rows(p.o, p.ldo, pk_row0, h * p.hd, Qs, p.hd, n_own, threadIdx.x);
+        if (OP) out_proj_epilogue(p, Qs, Vs, smax, ssum, sop, tS + lane_off, proj_full, w_full, ph, ri.r, part, quarter,
+                                  pk_row0, n_own);
         named_bar_sync_a(9, 256);                  // every thread has read its chunks: Q's smem may be refilled
         if (warp == 0 && lane == 0) mbar_arrive(q_free);
       } else if (warp == 0 && lane == 0) {
@@ -439,12 +544,16 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
 // TMEM round trip), and exchange row max, row sum and delta = sum_j P_ij dP_ij through shared memory.  dQ / dK / dV
 // leave through TMA stores from the (dead) dO / K / Q operand blocks.
 // Warp roles (320 threads): warps 0..7 softmax + epilogue (quarter = warp & 3, part = warp >> 2), warp 8 TMA, warp 9 MMA.
-template <bool DROP, bool PK>
+// Fused out-projection (OP, packed layout, heads == 1): tmDO maps dr instead of dO.  The dr tile lands in P's blocks (dead
+// until the softmax backward), Wo^T (B operand, hd rows x K = hd) is loaded once into its own blocks, and the MMA warp
+// computes dO = dr Wo into TMEM columns [384, 384 + hd) before S; the epilogue warps write it as bf16 into dO's blocks
+// (the layout a TMA load would have left) and the dP MMA follows.  Same K order and rounding as gemm_tn without bias.
+template <bool DROP, bool PK, bool OP>
 __global__ void __launch_bounds__(AF_THREADS, 1)
 attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                    const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmDO,
                    const __grid_constant__ CUtensorMap tmDQ, const __grid_constant__ CUtensorMap tmDK,
-                   const __grid_constant__ CUtensorMap tmDV, AttnTc p) {
+                   const __grid_constant__ CUtensorMap tmDV, const __grid_constant__ CUtensorMap tmWT, AttnTc p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const int opbytes = p.kblocks * OPB;
@@ -457,13 +566,18 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
   float* xch = reinterpret_cast<float*>(Gs + 2 * OPB);   // [3 values][2 parts][128 rows]: max, sum, delta numerator
   uint64_t* bars = reinterpret_cast<uint64_t*>(xch + 6 * TILE);
   uint64_t *in_full = bars, *in_free = bars + 1, *sdp_full = bars + 2, *ds_full = bars + 3, *out_full = bars + 4;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 6);
+  uint64_t *w_full = bars + 5, *do_full = bars + 6, *do_staged = bars + 7;    // OP: Wo^T landed, dr Wo done, dO staged
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 8);
+  uint8_t* Ws = smem + (4 * p.kblocks + 4) * OPB + 4096;  // OP: Wo^T, kblocks x [hd x 64] (after xch and the barriers)
+  const int wblk = p.hd * 128;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
   if (warp == 8 && lane == 0) {
     tma_prefetch_desc(&tmQ); tma_prefetch_desc(&tmK); tma_prefetch_desc(&tmV); tma_prefetch_desc(&tmDO);
     tma_prefetch_desc(&tmDQ); tma_prefetch_desc(&tmDK); tma_prefetch_desc(&tmDV);
+    if (OP) tma_prefetch_desc(&tmWT);
     mbar_init(in_full, 1); mbar_init(in_free, 1); mbar_init(sdp_full, 1); mbar_init(ds_full, 8); mbar_init(out_full, 1);
+    mbar_init(w_full, 1); mbar_init(do_full, 1); mbar_init(do_staged, 8);
     fence_barrier_init();
   }
   if (warp == 9) { tmem_alloc(tmem_slot, 512); tmem_relinquish(); }
@@ -478,8 +592,16 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
   // S and dP live in columns [0,128) and [128,256); once the softmax backward has consumed them the same
   // columns receive dK and dV, and dQ goes to [256, 256+hd).
   const uint32_t tS = tmem_base, tDP = tmem_base + 128, tDK = tmem_base, tDV = tmem_base + 128, tDQ = tmem_base + 256;
+  const uint32_t tDO = tmem_base + 384;    // OP: dO = dr Wo (hd <= 128 columns)
 
   if (warp == 8) {
+    if (OP) {
+      if (elect_one()) {
+        mbar_expect_tx(w_full, p.kblocks * wblk);
+        for (int kb = 0; kb < p.kblocks; ++kb) tma_load_2d(Ws + kb * wblk, &tmWT, w_full, kb * 64, 0, SRFRD_EVICT_LAST);
+      }
+      __syncwarp();
+    }
     uint32_t ph = 0;
     for (int it = blockIdx.x; it < n_items; it += gridDim.x, ph ^= 1) {
       const int tile = it / p.heads, h = it % p.heads;
@@ -491,7 +613,7 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
           tma_load_2d(Qs + kb * OPB, &tmQ, in_full, col0 + kb * 64, row0, SRFRD_EVICT_FIRST);
           tma_load_2d(Ks + kb * OPB, &tmK, in_full, col0 + kb * 64, row0, SRFRD_EVICT_FIRST);
           tma_load_2d(Vs + kb * OPB, &tmV, in_full, col0 + kb * 64, row0, SRFRD_EVICT_FIRST);
-          tma_load_2d(Ds + kb * OPB, &tmDO, in_full, col0 + kb * 64, row0, SRFRD_EVICT_FIRST);
+          tma_load_2d((OP ? Ps : Ds) + kb * OPB, &tmDO, in_full, col0 + kb * 64, row0, SRFRD_EVICT_FIRST);   // OP: dr
         }
         if (!(p.debug & 256) && it + (int)gridDim.x < n_items) {        // next item's operands: HBM -> L2 while this one computes
           const int itn = it + gridDim.x;
@@ -517,16 +639,39 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
     const uint64_t mK = umma_smem_desc(smem_u32(Ks), OPB, 1024), mQ = umma_smem_desc(smem_u32(Qs), OPB, 1024);
     const uint64_t mD = umma_smem_desc(smem_u32(Ds), OPB, 1024), mG = umma_smem_desc(smem_u32(Gs), OPB, 1024);
     const uint64_t mP = umma_smem_desc(smem_u32(Ps), OPB, 1024);
+    const uint64_t kP = umma_smem_desc(smem_u32(Ps), 0, 1024), kW = umma_smem_desc(smem_u32(Ws), 0, 1024);   // OP: dr, Wo^T
+    const uint32_t idW = umma_idesc_bf16(TILE, p.hd, 0, 0);
+    if (OP) { mbar_wait(w_full, 0); }
     uint32_t ph = 0;
     for (int it = blockIdx.x; it < n_items; it += gridDim.x, ph ^= 1) {
       mbar_wait(in_full, ph);                // (implies the previous item's dK / dV were read out of the S / dP columns)
       tc_fence_after();
+      if (OP) {                              // dO = dr Wo first (it gates dP), then S while the epilogue stages dO
+        if (elect_one()) {
+          for (int kb = 0; kb < p.kblocks; ++kb) {
+            const int ksteps = min(4, (p.hd - kb * 64) / 16);
+            for (int k = 0; k < ksteps; ++k)
+              umma_bf16(tDO, kP + (uint64_t)(kb * (OPB >> 4) + 2 * k), kW + (uint64_t)(kb * (wblk >> 4) + 2 * k), idW, (kb | k) != 0);
+          }
+          umma_commit(do_full);
+          for (int kb = 0; kb < p.kblocks; ++kb) {
+            const int ksteps = min(4, (p.hd - kb * 64) / 16);
+            for (int k = 0; k < ksteps; ++k) {
+              const uint64_t o = (uint64_t)(kb * (OPB >> 4) + 2 * k);
+              umma_bf16(tS, kQ + o, kK + o, idKK, (kb | k) != 0);
+            }
+          }
+        }
+        __syncwarp();
+        mbar_wait(do_staged, ph);
+        tc_fence_after();
+      }
       if (elect_one()) {
         for (int kb = 0; kb < p.kblocks; ++kb) {
           const int ksteps = min(4, (p.hd - kb * 64) / 16);
           for (int k = 0; k < ksteps; ++k) {
             const uint64_t o = (uint64_t)(kb * (OPB >> 4) + 2 * k);
-            umma_bf16(tS, kQ + o, kK + o, idKK, (kb | k) != 0);
+            if (!OP) umma_bf16(tS, kQ + o, kK + o, idKK, (kb | k) != 0);
             umma_bf16(tDP, kD + o, kV + o, idKK, (kb | k) != 0);
           }
         }
@@ -565,6 +710,30 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
       const int c0 = c_lo + part, c1 = c_lo + part + 2;
       const int lo0 = (c0 <= c_hi) ? ri.jlo - c0 * 32 : (1 << 20);
       const int lo1 = (c1 <= c_hi) ? ri.jlo - c1 * 32 : (1 << 20);
+      if (OP) {                              // dO -> bf16 into dO's blocks (gemm_tn's rounding: + 0 bias, then bf16)
+        mbar_wait(do_full, ph);
+        tc_fence_after();
+#pragma unroll 1
+        for (int c = part * 32; c < p.hd; c += 64) {
+          uint32_t ro[32];
+          tmem_ld32(tDO + lane_off + c, ro);
+          tmem_ld_wait();
+          uint8_t* blk = Ds + (c >> 6) * OPB;
+#pragma unroll
+          for (int u = 0; u < 4; ++u) {
+            if (c + 8 * u >= p.hd) break;
+            float v[8];
+#pragma unroll
+            for (int j = 0; j < 8; ++j) v[j] = __uint_as_float(ro[8 * u + j]) + 0.f;
+            *reinterpret_cast<uint4*>(blk + sw128(ri.r, (c & 63) + 8 * u)) =
+                make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
+          }
+        }
+        tc_fence_before();
+        fence_proxy_async();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(do_staged);
+      }
       mbar_wait(sdp_full, ph);
       tc_fence_after();
       uint32_t s0[32], s1[32], g0[32], g1[32];
@@ -784,16 +953,18 @@ extern "C" int srfrd_attention_fwd(const void* q, int ldq, const void* k, const 
   const size_t smem = (size_t)(2 * p.kblocks + (p.kblocks > 2 ? p.kblocks : 2)) * OPB + 4 * TILE * sizeof(float) + 1024 + 256;
   static bool attr = false;
   if (!attr) {
-    SRFRD_CUDA(cudaFuncSetAttribute(attn_fwd_tc_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 113 * 1024));
-    SRFRD_CUDA(cudaFuncSetAttribute(attn_fwd_tc_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 113 * 1024));
+    SRFRD_CUDA(cudaFuncSetAttribute(attn_fwd_tc_kernel<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 113 * 1024));
+    SRFRD_CUDA(cudaFuncSetAttribute(attn_fwd_tc_kernel<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 113 * 1024));
     attr = true;
   }
   int grid = p.n_tiles * heads;
   if (grid > 2 * num_sms()) grid = 2 * num_sms();
   if (p.drop_thresh)
-    SRFRD_CUDA(launch_pdl(attn_fwd_tc_kernel<true, false>, dim3(grid), dim3(AF_THREADS), smem, (cudaStream_t)stream, tmQ, tmK, tmV, tmO, p));
+    SRFRD_CUDA(launch_pdl(attn_fwd_tc_kernel<true, false, false>, dim3(grid), dim3(AF_THREADS), smem, (cudaStream_t)stream, tmQ, tmK, tmV, tmO,
+                          tmO, tmO, p));
   else
-    SRFRD_CUDA(launch_pdl(attn_fwd_tc_kernel<false, false>, dim3(grid), dim3(AF_THREADS), smem, (cudaStream_t)stream, tmQ, tmK, tmV, tmO, p));
+    SRFRD_CUDA(launch_pdl(attn_fwd_tc_kernel<false, false, false>, dim3(grid), dim3(AF_THREADS), smem, (cudaStream_t)stream, tmQ, tmK, tmV, tmO,
+                          tmO, tmO, p));
   SRFRD_LAUNCH_CHECK();
   return 0;
 }
@@ -828,18 +999,18 @@ extern "C" int srfrd_attention_bwd(const void* dout, int lddo, const void* q, in
   const size_t smem = (size_t)(4 * p.kblocks + 4) * OPB + 6 * TILE * sizeof(float) + 1024 + 256;
   static bool attr = false;
   if (!attr) {
-    SRFRD_CUDA(cudaFuncSetAttribute(attn_bwd_tc_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    SRFRD_CUDA(cudaFuncSetAttribute(attn_bwd_tc_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    SRFRD_CUDA(cudaFuncSetAttribute(attn_bwd_tc_kernel<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    SRFRD_CUDA(cudaFuncSetAttribute(attn_bwd_tc_kernel<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     attr = true;
   }
   int grid = p.n_tiles * heads;
   if (grid > num_sms()) grid = num_sms();
   if (p.drop_thresh)
-    SRFRD_CUDA(launch_pdl(attn_bwd_tc_kernel<true, false>, dim3(grid), dim3(AF_THREADS), smem, (cudaStream_t)stream, tmQ, tmK, tmV,
-                          tmDO, tmDQ, tmDK, tmDV, p));
+    SRFRD_CUDA(launch_pdl(attn_bwd_tc_kernel<true, false, false>, dim3(grid), dim3(AF_THREADS), smem, (cudaStream_t)stream, tmQ, tmK, tmV,
+                          tmDO, tmDQ, tmDK, tmDV, tmDV, p));
   else
-    SRFRD_CUDA(launch_pdl(attn_bwd_tc_kernel<false, false>, dim3(grid), dim3(AF_THREADS), smem, (cudaStream_t)stream, tmQ, tmK, tmV,
-                          tmDO, tmDQ, tmDK, tmDV, p));
+    SRFRD_CUDA(launch_pdl(attn_bwd_tc_kernel<false, false, false>, dim3(grid), dim3(AF_THREADS), smem, (cudaStream_t)stream, tmQ, tmK, tmV,
+                          tmDO, tmDQ, tmDK, tmDV, tmDV, p));
   SRFRD_LAUNCH_CHECK();
   return 0;
 }
@@ -857,34 +1028,77 @@ extern "C" int srfrd_attention_packed_supported(int L, int H, int heads) {
   return packed_supported(L, H, heads, 8, 8) && !getenv("SRFRD_ATTN_SIMT");
 }
 
+// Shared memory of the packed kernels (1024 B of slack for the 1024-byte alignment of the operand blocks)
+static size_t fwd_smem(int kblocks, bool op) {
+  return (size_t)(2 * kblocks + (kblocks > 2 ? kblocks : 2)) * OPB + 4 * TILE * sizeof(float) + 1024 + 256 +
+         (op ? 3 * TILE * sizeof(float) : 0);
+}
+static size_t bwd_smem(int kblocks, int hd, bool op) {
+  return op ? (size_t)(4 * kblocks + 4) * OPB + 4096 + (size_t)kblocks * hd * 128 + 1024
+            : (size_t)(4 * kblocks + 4) * OPB + 6 * TILE * sizeof(float) + 1024 + 256;
+}
+static constexpr size_t FWD_SMEM_MAX = 113 * 1024;       // two CTAs per SM
+static constexpr size_t BWD_SMEM_MAX = 227 * 1024;
+
+// Which packed kernels can fold the attention out-projection in: bit 0 forward, bit 1 backward.  One head (a CTA owns
+// whole rows, so the LayerNorm of the forward epilogue sees all columns), at most 128 columns (the kernels' operand
+// blocks and TMEM plan), and the shared-memory plan has to fit.
+static int oproj_supported(int L, int H, int heads) {
+  if (!packed_supported(L, H, heads, 8, 8) || heads != 1 || H > 128) return 0;
+  const int kblocks = (H + 63) / 64;
+  return (fwd_smem(kblocks, true) <= FWD_SMEM_MAX ? 1 : 0) | (bwd_smem(kblocks, H, true) <= BWD_SMEM_MAX ? 2 : 0);
+}
+
+extern "C" int srfrd_attention_packed_oproj_supported(int L, int H, int heads) {
+  return getenv("SRFRD_ATTN_SIMT") ? 0 : oproj_supported(L, H, heads);
+}
+
 extern "C" int srfrd_attention_fwd_packed(const void* q, int ldq, const void* k, const void* v, int ldkv, void* o, int ldo,
                                           const srfrd_pack_t* pk, int L, int H, int heads, float drop_p, uint64_t seed,
-                                          uint32_t stream_id, const float* drop_step, void* stream) {
+                                          uint32_t stream_id, const float* drop_step, void* stream, const void* wo, int ldw,
+                                          const float* bo, const void* res, int ldres, const float* ln_w, const float* ln_b,
+                                          float ln_eps, float* ln_stats, void* r, int ldr, void* y, int ldy) {
   SRFRD_REQUIRE(q && k && v && o && pk && pk->rows && pk->row_info && pk->tile_row0, "attention_fwd_packed: null pointer");
   SRFRD_REQUIRE(packed_supported(L, H, heads, ldq, ldkv) && ldo % 8 == 0 && ((uintptr_t)o & 15) == 0,
                 "attention_fwd_packed: unsupported shape (L=%d H=%d heads=%d)", L, H, heads);
+  const bool op = wo != nullptr;
+  if (op) {
+    SRFRD_REQUIRE(oproj_supported(L, H, heads) & 1, "attention_fwd_packed: no fused out-projection for H=%d heads=%d", H, heads);
+    SRFRD_REQUIRE(res && ln_w && ln_b && r && y, "attention_fwd_packed: fused out-projection needs residual, LayerNorm, r and y");
+    SRFRD_REQUIRE(ldw % 8 == 0 && ldw >= H && ldres % 8 == 0 && ldr % 8 == 0 && ldy % 8 == 0 &&
+                      (((uintptr_t)res | (uintptr_t)r | (uintptr_t)y | (uintptr_t)wo) & 15) == 0,
+                  "attention_fwd_packed: bad out-projection operands");
+  }
   AttnTc p = {};
   if (int rc = fill(p, 1, L, H, heads, drop_p, seed, stream_id, drop_step)) return rc;
   p.T = pk->cap;
   p.o = (bf16*)o; p.ldo = ldo; p.tma_o = 1;
   p.pk_rows = pk->rows; p.pk_info = (const int4*)pk->row_info; p.pk_tile_row0 = pk->tile_row0;
-  CUtensorMap tmQ, tmK, tmV;
+  CUtensorMap tmQ, tmK, tmV, tmW, tmR;
   if (int rc = make_tmap_bf16_2d(&tmQ, q, p.T, H, ldq, TILE, 64)) return rc;
   if (int rc = make_tmap_bf16_2d(&tmK, k, p.T, H, ldkv, TILE, 64)) return rc;
   if (int rc = make_tmap_bf16_2d(&tmV, v, p.T, H, ldkv, TILE, 64)) return rc;
-  const size_t smem = (size_t)(2 * p.kblocks + (p.kblocks > 2 ? p.kblocks : 2)) * OPB + 4 * TILE * sizeof(float) + 1024 + 256;
+  tmW = tmQ; tmR = tmQ;
+  if (op) {
+    if (int rc = make_tmap_bf16_2d(&tmW, wo, H, H, ldw, H, 64)) return rc;        // the whole [H x H] weight in one box row
+    if (int rc = make_tmap_bf16_2d(&tmR, res, p.T, H, ldres, TILE, 64)) return rc;
+    p.op_bias = bo; p.ln_w = ln_w; p.ln_b = ln_b; p.ln_stats = ln_stats; p.ln_eps = ln_eps;
+    p.op_r = (bf16*)r; p.op_y = (bf16*)y; p.ldr = ldr; p.ldy = ldy;
+  }
+  const size_t smem = fwd_smem(p.kblocks, op);
   static bool attr = false;
   if (!attr) {
-    SRFRD_CUDA(cudaFuncSetAttribute(attn_fwd_tc_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 113 * 1024));
-    SRFRD_CUDA(cudaFuncSetAttribute(attn_fwd_tc_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 113 * 1024));
+    SRFRD_CUDA(cudaFuncSetAttribute(attn_fwd_tc_kernel<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, FWD_SMEM_MAX));
+    SRFRD_CUDA(cudaFuncSetAttribute(attn_fwd_tc_kernel<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, FWD_SMEM_MAX));
+    SRFRD_CUDA(cudaFuncSetAttribute(attn_fwd_tc_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FWD_SMEM_MAX));
+    SRFRD_CUDA(cudaFuncSetAttribute(attn_fwd_tc_kernel<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FWD_SMEM_MAX));
     attr = true;
   }
   int64_t grid = (pk->cap / 64 + 1) * heads;               // more tiles than this cannot exist
   if (grid > 2 * num_sms()) grid = 2 * num_sms();
-  if (p.drop_thresh)
-    SRFRD_CUDA(launch_pdl(attn_fwd_tc_kernel<true, true>, dim3((unsigned)grid), dim3(AF_THREADS), smem, (cudaStream_t)stream, tmQ, tmK, tmV, tmQ, p));
-  else
-    SRFRD_CUDA(launch_pdl(attn_fwd_tc_kernel<false, true>, dim3((unsigned)grid), dim3(AF_THREADS), smem, (cudaStream_t)stream, tmQ, tmK, tmV, tmQ, p));
+  auto kern = p.drop_thresh ? (op ? attn_fwd_tc_kernel<true, true, true> : attn_fwd_tc_kernel<true, true, false>)
+                            : (op ? attn_fwd_tc_kernel<false, true, true> : attn_fwd_tc_kernel<false, true, false>);
+  SRFRD_CUDA(launch_pdl(kern, dim3((unsigned)grid), dim3(AF_THREADS), smem, (cudaStream_t)stream, tmQ, tmK, tmV, tmQ, tmW, tmR, p));
   SRFRD_LAUNCH_CHECK();
   return 0;
 }
@@ -892,38 +1106,48 @@ extern "C" int srfrd_attention_fwd_packed(const void* q, int ldq, const void* k,
 extern "C" int srfrd_attention_bwd_packed(const void* dout, int lddo, const void* q, int ldq, const void* k, const void* v,
                                           int ldkv, void* dq, int lddq, void* dk, void* dv, int lddkv, const srfrd_pack_t* pk,
                                           int L, int H, int heads, float drop_p, uint64_t seed, uint32_t stream_id,
-                                          const float* drop_step, void* stream) {
-  SRFRD_REQUIRE(dout && q && k && v && dq && dk && dv && pk && pk->rows && pk->row_info && pk->tile_row0,
+                                          const float* drop_step, void* stream, const void* dr, int lddr, const void* woT,
+                                          int ldw) {
+  const bool op = dr != nullptr;
+  SRFRD_REQUIRE((op ? (woT != nullptr) : (dout != nullptr)) && q && k && v && dq && dk && dv && pk && pk->rows &&
+                    pk->row_info && pk->tile_row0,
                 "attention_bwd_packed: null pointer");
-  SRFRD_REQUIRE(packed_supported(L, H, heads, ldq, ldkv) && lddo % 8 == 0 && lddq % 8 == 0 && lddkv % 8 == 0 &&
+  SRFRD_REQUIRE(packed_supported(L, H, heads, ldq, ldkv) && (op || lddo % 8 == 0) && lddq % 8 == 0 && lddkv % 8 == 0 &&
                     (((uintptr_t)dq | (uintptr_t)dk | (uintptr_t)dv) & 15) == 0,
                 "attention_bwd_packed: unsupported shape (L=%d H=%d heads=%d)", L, H, heads);
+  if (op) {
+    SRFRD_REQUIRE(oproj_supported(L, H, heads) & 2, "attention_bwd_packed: no fused out-projection for H=%d heads=%d", H, heads);
+    SRFRD_REQUIRE(lddr % 8 == 0 && ldw % 8 == 0 && ldw >= H && (((uintptr_t)dr | (uintptr_t)woT) & 15) == 0,
+                  "attention_bwd_packed: bad out-projection operands");
+  }
   AttnTc p = {};
   if (int rc = fill(p, 1, L, H, heads, drop_p, seed, stream_id, drop_step)) return rc;
   p.T = pk->cap;
   p.dq = (bf16*)dq; p.dk = (bf16*)dk; p.dv = (bf16*)dv; p.lddq = lddq; p.lddkv = lddkv; p.tma_o = 1;
   p.pk_rows = pk->rows; p.pk_info = (const int4*)pk->row_info; p.pk_tile_row0 = pk->tile_row0;
   { const char* l2 = getenv("SRFRD_L2_PREFETCH"); if (l2 && atoi(l2) == 0) p.debug |= 256; }
-  CUtensorMap tmQ, tmK, tmV, tmDO;
+  CUtensorMap tmQ, tmK, tmV, tmDO, tmWT;
   if (int rc = make_tmap_bf16_2d(&tmQ, q, p.T, H, ldq, TILE, 64)) return rc;
   if (int rc = make_tmap_bf16_2d(&tmK, k, p.T, H, ldkv, TILE, 64)) return rc;
   if (int rc = make_tmap_bf16_2d(&tmV, v, p.T, H, ldkv, TILE, 64)) return rc;
-  if (int rc = make_tmap_bf16_2d(&tmDO, dout, p.T, H, lddo, TILE, 64)) return rc;
-  const size_t smem = (size_t)(4 * p.kblocks + 4) * OPB + 6 * TILE * sizeof(float) + 1024 + 256;
+  if (int rc = make_tmap_bf16_2d(&tmDO, op ? dr : dout, p.T, H, op ? lddr : lddo, TILE, 64)) return rc;   // OP: dr
+  tmWT = tmQ;
+  if (op) if (int rc = make_tmap_bf16_2d(&tmWT, woT, H, H, ldw, H, 64)) return rc;
+  const size_t smem = bwd_smem(p.kblocks, p.hd, op);
   static bool attr = false;
   if (!attr) {
-    SRFRD_CUDA(cudaFuncSetAttribute(attn_bwd_tc_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    SRFRD_CUDA(cudaFuncSetAttribute(attn_bwd_tc_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    SRFRD_CUDA(cudaFuncSetAttribute(attn_bwd_tc_kernel<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, BWD_SMEM_MAX));
+    SRFRD_CUDA(cudaFuncSetAttribute(attn_bwd_tc_kernel<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, BWD_SMEM_MAX));
+    SRFRD_CUDA(cudaFuncSetAttribute(attn_bwd_tc_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, BWD_SMEM_MAX));
+    SRFRD_CUDA(cudaFuncSetAttribute(attn_bwd_tc_kernel<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, BWD_SMEM_MAX));
     attr = true;
   }
   int64_t grid = (pk->cap / 64 + 1) * heads;
   if (grid > num_sms()) grid = num_sms();
-  if (p.drop_thresh)
-    SRFRD_CUDA(launch_pdl(attn_bwd_tc_kernel<true, true>, dim3((unsigned)grid), dim3(AF_THREADS), smem, (cudaStream_t)stream, tmQ, tmK, tmV,
-                          tmDO, tmQ, tmQ, tmQ, p));
-  else
-    SRFRD_CUDA(launch_pdl(attn_bwd_tc_kernel<false, true>, dim3((unsigned)grid), dim3(AF_THREADS), smem, (cudaStream_t)stream, tmQ, tmK, tmV,
-                          tmDO, tmQ, tmQ, tmQ, p));
+  auto kern = p.drop_thresh ? (op ? attn_bwd_tc_kernel<true, true, true> : attn_bwd_tc_kernel<true, true, false>)
+                            : (op ? attn_bwd_tc_kernel<false, true, true> : attn_bwd_tc_kernel<false, true, false>);
+  SRFRD_CUDA(launch_pdl(kern, dim3((unsigned)grid), dim3(AF_THREADS), smem, (cudaStream_t)stream, tmQ, tmK, tmV, tmDO, tmQ, tmQ,
+                        tmQ, tmWT, p));
   SRFRD_LAUNCH_CHECK();
   return 0;
 }

@@ -98,6 +98,45 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
   __nv_bfloat162 t = __floats2bfloat162_rn(lo, hi);
   return *reinterpret_cast<uint32_t*>(&t);
 }
+__device__ __forceinline__ void unpack_bf16x8(const uint4& u, float* f) {
+  const uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const __nv_bfloat162 t = *reinterpret_cast<const __nv_bfloat162*>(&w[i]);
+    f[2 * i] = __low2float(t);
+    f[2 * i + 1] = __high2float(t);
+  }
+}
+
+// LayerNorm of a result row in a GEMM epilogue (gemm_tn's LNF kernels, the attention kernel's fused out-projection): the
+// statistics are those of the ROUNDED bf16 values (what a separate LayerNorm kernel would read back).  Each thread
+// accumulates its own columns, the threads of a row then combine their partial (sum, sum of squares).
+__device__ __forceinline__ void lnf_accum8(const uint4& pk, float& sum, float& sq) {
+  const uint32_t pw[4] = {pk.x, pk.y, pk.z, pk.w};
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const float lo = __uint_as_float(pw[i] << 16), hi = __uint_as_float(pw[i] & 0xffff0000u);
+    sum += lo + hi;
+    sq = fmaf(lo, lo, fmaf(hi, hi, sq));
+  }
+}
+// (own partial sums, the row partner's) -> mean, rstd and nb = -mean * rstd over n columns
+__device__ __forceinline__ void lnf_stats(float sum, float sq, float osum, float osq, int n, float eps, float& mean,
+                                          float& rstd, float& nb) {
+  const float invn = 1.f / (float)n;
+  mean = (sum + osum) * invn;
+  const float var = fmaxf((sq + osq) * invn - mean * mean, 0.f);
+  rstd = rsqrtf(var + eps);
+  nb = -mean * rstd;
+}
+// 8 rounded values -> 8 normalised, scaled and shifted bf16 values (w, b: the LayerNorm weight / bias of these columns)
+__device__ __forceinline__ uint4 lnf_apply8(const uint4& x, float rstd, float nb, const float* w, const float* b) {
+  float f[8], y[8];
+  unpack_bf16x8(x, f);
+#pragma unroll
+  for (int i = 0; i < 8; ++i) y[i] = fmaf(fmaf(f[i], rstd, nb), w[i], b[i]);
+  return make_uint4(pack_bf16x2(y[0], y[1]), pack_bf16x2(y[2], y[3]), pack_bf16x2(y[4], y[5]), pack_bf16x2(y[6], y[7]));
+}
 __device__ __forceinline__ void red_add_f32(float* addr, float v) {
   asm volatile("red.global.add.f32 [%0], %1;" ::"l"(addr), "f"(v) : "memory");
 }

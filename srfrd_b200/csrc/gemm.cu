@@ -83,16 +83,6 @@ static constexpr int TN_RING = 16;                       // tile-id ring between
 // byte offset of the 16-byte chunk j (8 bf16 columns) of row r inside a 128-byte-swizzled [128 x 64] bf16 block
 __device__ __forceinline__ uint32_t sw128_chunk(int r, int j) { return (uint32_t)(r * 128 + ((j ^ (r & 7)) << 4)); }
 
-__device__ __forceinline__ void unpack_bf16x8(const uint4& u, float* f) {
-  const uint32_t w[4] = {u.x, u.y, u.z, u.w};
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const __nv_bfloat162 t = *reinterpret_cast<const __nv_bfloat162*>(&w[i]);
-    f[2 * i] = __low2float(t);
-    f[2 * i + 1] = __high2float(t);
-  }
-}
-
 __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
@@ -421,15 +411,7 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             if (s.tma_out) {
               const uint4 pk = make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
               *reinterpret_cast<uint4*>(blkp + sw128_chunk(r, cj + j)) = pk;
-              if (LNF) {                                 // row statistics of the ROUNDED values (what a LayerNorm kernel would read)
-                const uint32_t pw[4] = {pk.x, pk.y, pk.z, pk.w};
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                  const float lo = __uint_as_float(pw[i] << 16), hi = __uint_as_float(pw[i] & 0xffff0000u);
-                  ln_sum += lo + hi;
-                  ln_sq = fmaf(lo, lo, fmaf(hi, hi, ln_sq));
-                }
-              }
+              if (LNF) lnf_accum8(pk, ln_sum, ln_sq);    // row statistics of the ROUNDED values (common.cuh)
             } else if (row_ok) {
               const int n = nc + 8 * j;
               if (e.out_bf16)
@@ -462,10 +444,8 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           uint8_t* ybuf = smY + set * s.buf_blocks * EPI_BLK_BYTES;
           // one-pass statistics: the two warps of a row exchange (sum, sum of squares) of their columns
           const float2 other = *reinterpret_cast<const float2*>(sxch + ((set * 2 + (half ^ 1)) * BLOCK_M + r) * 2);
-          const float invn = 1.f / (float)bn;
-          const float mean = (ln_sum + other.x) * invn;
-          const float var = fmaxf((ln_sq + other.y) * invn - mean * mean, 0.f);
-          const float rstd = rsqrtf(var + e.ln_eps), nb = -mean * rstd;
+          float mean, rstd, nb;
+          lnf_stats(ln_sum, ln_sq, other.x, other.y, bn, e.ln_eps, mean, rstd, nb);
 #pragma unroll 1
           for (int c = half * 32; c < bn; c += 64) {
             const int cj = (c & 63) >> 3;
@@ -473,14 +453,10 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
               if (c + 8 * j >= bn) break;
-              float f[8], y[8];
               const uint32_t off = boff + sw128_chunk(r, cj + j);
-              unpack_bf16x8(*reinterpret_cast<const uint4*>(buf + off), f);
               const float* w = sln + c + 8 * j;
-#pragma unroll
-              for (int i = 0; i < 8; ++i) y[i] = fmaf(fmaf(f[i], rstd, nb), w[i], w[MAX_LN + i]);
               *reinterpret_cast<uint4*>(ybuf + off) =
-                  make_uint4(pack_bf16x2(y[0], y[1]), pack_bf16x2(y[2], y[3]), pack_bf16x2(y[4], y[5]), pack_bf16x2(y[6], y[7]));
+                  lnf_apply8(*reinterpret_cast<const uint4*>(buf + off), rstd, nb, w, w + MAX_LN);
             }
           }
           if (half == 0 && row_ok && e.ln_stats) *reinterpret_cast<float2*>(e.ln_stats + 2 * (size_t)row) = make_float2(mean, rstd);

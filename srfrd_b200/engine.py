@@ -597,6 +597,7 @@ class HotPath:
         x = [ws[f"x{i}"][:T] for i in range(nb + 1)]
         row_ids = plan.row_ids
         fuse_ln = Hp <= 128 and os.environ.get("SRFRD_FUSE_LN", "1") != "0"
+        fuse_oproj = self._fuse_oproj(hyb, L, fuse_ln) & 1
         with ops.row_limit(plan.rows):
             ops.embed_ln_fwd_packed(P.view(s.item_key), P.view(s.pos_key), aux_table, s.mode, seq, aux_ids, s.item_scale,
                                     P.view("attention_layernorms.0.weight"), P.view("attention_layernorms.0.bias"), LN_EPS,
@@ -611,7 +612,13 @@ class HotPath:
                                       LN_EPS, y_bf16=Q, stats=ws[f"st1_{i}"][:T], H=H)
                 ops.gemm_tn(Q, self.sh[f"wq{i}"], out_bf16=q, bias=self.bias("bq", i))
                 self._join()
-                if hyb is None:
+                if fuse_oproj:              # out-projection, residual and LayerNorm in the attention kernel's epilogue
+                    ops.attention_fwd_packed(q, kv[:, :Hp], kv[:, Hp:], o, plan, L, H, s.num_heads, p_drop, seed, 10 + 4 * i, step,
+                                             wo=self.sh[f"wo{i}"], bias=self.bias("bo", i), residual=Q, r=r, y=y,
+                                             ln_w=P.view(f"forward_layernorms.{i}.weight"),
+                                             ln_b=P.view(f"forward_layernorms.{i}.bias"), ln_eps=LN_EPS,
+                                             ln_stats=ws[f"st2_{i}"][:T])
+                elif hyb is None:
                     ops.attention_fwd_packed(q, kv[:, :Hp], kv[:, Hp:], o, plan, L, H, s.num_heads, p_drop, seed, 10 + 4 * i, step)
                 else:       # dense-layout attention between an unpack and a pack copy
                     qd, kvd, od = hyb[f"qd{i}"][:B * L], hyb[f"kvd{i}"][:B * L], hyb[f"od{i}"][:B * L]
@@ -620,7 +627,9 @@ class HotPath:
                         ops.attention_fwd(qd, kvd[:, :Hp], kvd[:, Hp:], od, B, L, H, s.num_heads, p_drop, seed, 10 + 4 * i, step,
                                           stats=ws.get(f"ast{i}"))
                     ops.pack_rows([(od, o, Hp, 0)], plan)
-                if fuse_ln:
+                if fuse_oproj:
+                    pass                    # r, y and their statistics came out of the attention kernel
+                elif fuse_ln:
                     ops.gemm_tn(o, self.sh[f"wo{i}"], out_bf16=r, bias=self.bias("bo", i), residual=Q, ln_out=y,
                                 ln_w=P.view(f"forward_layernorms.{i}.weight"), ln_b=P.view(f"forward_layernorms.{i}.bias"),
                                 ln_eps=LN_EPS, ln_stats=ws[f"st2_{i}"][:T])
@@ -660,6 +669,14 @@ class HotPath:
                               version=self.fwd_version, plan=plan, hyb=hyb, live=live)
         return ws["hfin"][:T]
 
+    def _fuse_oproj(self, hyb, L, fuse_ln) -> int:
+        """Bit 0 / 1: the packed attention forward / backward takes the out-projection (tile layout, one head, the
+        fused-LayerNorm width, and the kernel's shared-memory plan fits); otherwise the separate gemm_tn launches."""
+        s = self.spec
+        if hyb is not None or s.num_heads != 1 or not fuse_ln or s.Hp != s.H:
+            return 0
+        return ops.attention_packed_oproj_supported(L, s.H, s.num_heads)
+
     def _backward_packed(self, dh: torch.Tensor) -> None:
         s, P, sv = self.spec, self.P, self.saved
         plan, hyb, live = sv["plan"], sv.get("hyb"), sv.get("live")
@@ -673,6 +690,7 @@ class HotPath:
         GM = lambda name: P.mat(name, grad=True)
         x = [ws[f"x{i}"][:T] for i in range(nb + 1)]
         dz_top = ws[f"gdz_{nb - 1}"][:T]
+        fuse_oproj = self._fuse_oproj(hyb, L, Hp <= 128 and os.environ.get("SRFRD_FUSE_LN", "1") != "0") & 2
         with ops.row_limit(plan.rows):
             if s.kind == "SRFR":
                 gc = ws["gc"][:T]
@@ -712,8 +730,12 @@ class HotPath:
                 with self._branch():
                     ops.gemm_wgrad(dr, o, GM(f"attention_layers.{i}.out_proj.weight"),
                                    G(f"attention_layers.{i}.out_proj.bias"), Mo=H, No=H)
-                ops.gemm_tn(dr, self.sh[f"woT{i}"], out_bf16=gC)
-                if hyb is None:
+                if not fuse_oproj:
+                    ops.gemm_tn(dr, self.sh[f"woT{i}"], out_bf16=gC)
+                if fuse_oproj:              # dO = dr Wo inside the attention kernel
+                    ops.attention_bwd_packed(None, q, kv[:, :Hp], kv[:, Hp:], dq, dkv[:, :Hp], dkv[:, Hp:], plan, L, H,
+                                             s.num_heads, p_drop, seed, 10 + 4 * i, step, dr=dr, woT=self.sh[f"woT{i}"])
+                elif hyb is None:
                     ops.attention_bwd_packed(gC, q, kv[:, :Hp], kv[:, Hp:], dq, dkv[:, :Hp], dkv[:, Hp:], plan, L, H,
                                              s.num_heads, p_drop, seed, 10 + 4 * i, step)
                 else:

@@ -365,17 +365,29 @@ def layernorm_fwd_rows(x, w, b, eps, y_f32, row_index, n, H):
          n, H, _stream())
 
 
-def attention_fwd_packed(q, k, v, o, plan: PackedPlan, L, H, heads, drop_p=0.0, seed=0, stream_id=0, drop_step=None):
+def attention_packed_oproj_supported(L: int, H: int, heads: int) -> int:
+    """Bit 0: attention_fwd_packed can take the out-projection (wo=...); bit 1: attention_bwd_packed can (dr=...)."""
+    return int(_lib.load().srfrd_attention_packed_oproj_supported(int(L), int(H), int(heads)))
+
+
+def attention_fwd_packed(q, k, v, o, plan: PackedPlan, L, H, heads, drop_p=0.0, seed=0, stream_id=0, drop_step=None,
+                         wo=None, bias=None, residual=None, r=None, y=None, ln_w=None, ln_b=None, ln_eps=0.0, ln_stats=None):
+    """With wo: also r = o @ wo^T + bias + residual, y = LayerNorm(r) (ln_w, ln_b, ln_eps; (mean, rstd) -> ln_stats),
+    the rows gemm_tn(o, wo, out_bf16=r, bias=bias, residual=residual, ln_out=y, ...) would write."""
     _lib.require_device()
+    st = lambda t: 0 if t is None else t.stride(0)
     call("srfrd_attention_fwd_packed", _p(q), q.stride(0), _p(k), _p(v), k.stride(0), _p(o), o.stride(0), C.byref(plan.desc),
-         L, H, heads, float(drop_p), int(seed), int(stream_id), _p(drop_step), _stream())
+         L, H, heads, float(drop_p), int(seed), int(stream_id), _p(drop_step), _stream(), _p(wo), st(wo), _p(bias),
+         _p(residual), st(residual), _p(ln_w), _p(ln_b), float(ln_eps), _p(ln_stats), _p(r), st(r), _p(y), st(y))
 
 
 def attention_bwd_packed(dout, q, k, v, dq, dk, dv, plan: PackedPlan, L, H, heads, drop_p=0.0, seed=0, stream_id=0,
-                         drop_step=None):
-    call("srfrd_attention_bwd_packed", _p(dout), dout.stride(0), _p(q), q.stride(0), _p(k), _p(v), k.stride(0), _p(dq),
+                         drop_step=None, dr=None, woT=None):
+    """With dr (dout None): dout = dr @ woT^T is computed inside the kernel (what gemm_tn(dr, woT) would write)."""
+    st = lambda t: 0 if t is None else t.stride(0)
+    call("srfrd_attention_bwd_packed", _p(dout), st(dout), _p(q), q.stride(0), _p(k), _p(v), k.stride(0), _p(dq),
          dq.stride(0), _p(dk), _p(dv), dk.stride(0), C.byref(plan.desc), L, H, heads, float(drop_p), int(seed),
-         int(stream_id), _p(drop_step), _stream())
+         int(stream_id), _p(drop_step), _stream(), _p(dr), st(dr), _p(woT), st(woT))
 
 
 def score_loss_fused_packed(h, item_table, fake_table, pos, neg, prs, nrs, w_pos, w_neg, norm, loss_acc, dh, d_item, d_fake,
