@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define SRFRD_ABI_VERSION 6
+#define SRFRD_ABI_VERSION 7
 #if defined(__GNUC__)
 #define SRFRD_API __attribute__((visibility("default")))
 #else
@@ -193,10 +193,25 @@ SRFRD_API int srfrd_adam_step(float* p, float* g, float* m, float* v, int64_t n,
 
 /* The tail of a training step in ONE launch: srfrd_adam_tick + srfrd_adam_step + srfrd_loss_finalize (acc2 nullable).
  * state8 = {step, 1-beta1^step, 1-beta2^step, uint32 step bits (seed of dropout / sampler), int scratch counter, -, -, -}:
- * every block derives the new state from the old one, the last block to finish publishes it. */
+ * every block derives the new state from the old one, the last block to finish publishes it.
+ * Optional l2_emb regulariser (replaces: trainer.py:31-39, loss += l2_emb * torch.norm(param) for every parameter):
+ * l2_seg = the device segment table of srfrd_param_l2, l2_coef / l2_reg its outputs.  Each element's gradient becomes
+ * g + l2_coef[t] * p (t = the tensor holding it, p before this update) and loss[0] gains l2_reg[0]; needs acc2 and
+ * n % 4 == 0.  l2_seg = NULL (l2_n_seg, l2_coef, l2_reg ignored) is the plain step. */
 SRFRD_API int srfrd_adam_step_fused(float* p, float* g, float* m, float* v, int64_t n, float lr, float beta1, float beta2,
                           float eps, float* state8, int zero_grad, float* acc2, const float* norm2, float* loss,
-                          void* stream);
+                          void* stream, const int64_t* l2_seg, int l2_n_seg, const float* l2_coef, const float* l2_reg);
+
+/* ---- l2_emb regulariser: per-tensor L2 norms of the flat parameter buffer (replaces: trainer.py:37-39) ----
+ * seg = {offset, numel} per parameter tensor (int64 pairs, offsets 4-aligned and increasing, the gaps between tensors
+ * are never read), at most 256 tensors.  Writes coef[t] = l2 / ||p_t|| (0 when ||p_t|| == 0, as torch's gradient of the
+ * norm of a zero tensor is 0) and reg[0] = l2 * sum_t ||p_t||.  The buffer is cut into fixed 8192-float chunks that do
+ * not cross tensors; sums of squares are accumulated and reduced in fp64 in a fixed order (no float atomics), so the
+ * outputs are bit-identical across launches and ranks.  srfrd_param_l2_plan (host arithmetic on a HOST copy of seg)
+ * returns the chunk count; ws = n_chunks + 1 doubles, zero-initialised once (word 0 is a counter the kernel leaves 0). */
+SRFRD_API int srfrd_param_l2_plan(const int64_t* seg_host, int n_seg, int64_t* n_chunks);
+SRFRD_API int srfrd_param_l2(const float* p, const int64_t* seg, int n_seg, int64_t n_chunks, float l2, float* coef,
+                   float* reg, double* ws, void* stream);
 
 /* ---- K8/K9: full-catalogue scoring fused with a streaming per-row top-10 ----
  * replaces: SRFR_model.py:144-152 predict() called with label = arange(1, N+1) + the double argsort of
@@ -377,10 +392,13 @@ SRFRD_API int srfrd_pack_rows(const srfrd_repack_part_t* parts, int n_parts, con
  * through release / acquire flags in each rank's signal words.  grad / param / signal pointer arrays are DEVICE arrays of
  * `world` peer-mapped pointers (torch.distributed._symmetric_memory buffer_ptrs_dev); buckets and parameter buffers hold
  * n + 4 floats; local4 = 4 zero-initialised device words (epoch, grid barrier).  Replaces an NCCL all-reduce of the bucket
- * followed by srfrd_adam_step_fused on every rank; with world == 1 it is the same arithmetic as srfrd_adam_step_fused. */
+ * followed by srfrd_adam_step_fused on every rank; with world == 1 it is the same arithmetic as srfrd_adam_step_fused.
+ * l2_seg / l2_n_seg / l2_coef / l2_reg: the optional l2_emb term of srfrd_adam_step_fused, added once to the SUMMED
+ * gradient of the owned slice (the slice is cut on float4 boundaries, not tensors); rank 0 adds l2_reg[0] to the loss. */
 SRFRD_API int srfrd_dp_adam_step(float* const* grad_ptrs_dev, float* const* param_ptrs_dev, uint32_t* const* signal_ptrs_dev,
                        int rank, int world, int64_t n, float* m, float* v, float lr, float beta1, float beta2, float eps,
-                       float* state8, const float* norm2, uint32_t* local4, void* stream);
+                       float* state8, const float* norm2, uint32_t* local4, void* stream, const int64_t* l2_seg,
+                       int l2_n_seg, const float* l2_coef, const float* l2_reg);
 
 #ifdef __cplusplus
 }

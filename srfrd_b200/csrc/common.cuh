@@ -366,4 +366,41 @@ __host__ __device__ __forceinline__ uint32_t umma_idesc_bf16(int M, int N, int a
 int make_tmap_bf16_2d(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols, uint64_t ld,
                       uint32_t box_rows, uint32_t box_cols);
 
+// ---- l2_emb regulariser: segment table of the flat parameter buffer (loss_scatter_adam.cu, dp_adam.cu)
+static constexpr int L2_THREADS = 256;            // threads of srfrd_param_l2 = the most tensors it supports
+
+// Segment lookup of the Adam variants that add the regulariser's gradient: s_off[t] = float4 index where tensor t starts.
+// A thread's grid-stride indices only increase, so it finds its first segment by binary search and then walks forward.
+struct L2Segments {
+  const int64_t* seg;        // device {offset, numel} per tensor (offsets 4-aligned, increasing)
+  int n_seg;
+  const float* coef;         // l2 / ||p_t|| per tensor (srfrd_param_l2)
+  const float* reg;          // l2 * sum_t ||p_t||, added to the published loss
+};
+
+// The tables live in a function-scope shared buffer, so a kernel's plain (l2-off) instantiation allocates none of it.
+struct L2Smem { int64_t off[L2_THREADS]; float coef[L2_THREADS]; };
+__device__ __forceinline__ L2Smem& l2_smem() { __shared__ L2Smem s; return s; }
+
+__device__ __forceinline__ void l2_load_starts(const L2Segments& l2s, int64_t* s_off, float* s_coef) {
+  for (int t = threadIdx.x; t < l2s.n_seg; t += blockDim.x) {
+    s_off[t] = l2s.seg[2 * t] >> 2;
+    s_coef[t] = l2s.coef[t];
+  }
+}
+
+__device__ __forceinline__ int l2_find(const int64_t* s_off, int n_seg, int64_t i4) {
+  int lo = 0, hi = n_seg - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (s_off[mid] <= i4) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+__device__ __forceinline__ int l2_advance(const int64_t* s_off, int n_seg, int t, int64_t i4) {
+  while (t + 1 < n_seg && s_off[t + 1] <= i4) ++t;
+  return t;
+}
+
 }  // namespace srfrd

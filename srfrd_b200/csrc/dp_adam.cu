@@ -62,13 +62,23 @@ struct DpAdam {
   float* state;              // local Adam state8
   const float* norm;         // local (already all-reduced) weight sums
   uint32_t* local;           // local words: [0] epoch, [1] grid arrival counter, [2] exit flag, [3] entry flag
+  L2Segments l2s;            // l2_emb regulariser (L2 instantiation only)
 };
 
+// L2: g += coef[tensor] * p on the reduced gradient (added once, after the sum over ranks) and rank 0 adds reg to the loss.
+template <bool L2>
 __global__ void __launch_bounds__(DP_THREADS, 1) dp_adam_kernel(DpAdam p) {
   __shared__ float s_bc[2];
   __shared__ uint32_t s_epoch;
   pdl_prologue_done();
   const int tid = threadIdx.x;
+  int64_t* s_off = nullptr;
+  float* s_coef = nullptr;
+  if constexpr (L2) {
+    s_off = l2_smem().off;
+    s_coef = l2_smem().coef;
+    l2_load_starts(p.l2s, s_off, s_coef);
+  }
   if (tid == 0) {
     s_epoch = p.local[0];
     const float step = p.state[0] + 1.f;
@@ -102,6 +112,8 @@ __global__ void __launch_bounds__(DP_THREADS, 1) dp_adam_kernel(DpAdam p) {
     gp[r] = r < p.world ? reinterpret_cast<float4*>(p.grad[r]) : nullptr;
     pp_[r] = r < p.world ? reinterpret_cast<float4*>(p.param[r]) : nullptr;
   }
+  int sg = 0;
+  if constexpr (L2) sg = l2_find(s_off, p.l2s.n_seg, lo + (int64_t)blockIdx.x * blockDim.x + tid);
   for (int64_t i = lo + (int64_t)blockIdx.x * blockDim.x + tid; i < hi; i += (int64_t)gridDim.x * blockDim.x) {
     float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
@@ -113,6 +125,12 @@ __global__ void __launch_bounds__(DP_THREADS, 1) dp_adam_kernel(DpAdam p) {
     float4 w = pp_[p.rank][i];
     float4 mm = reinterpret_cast<float4*>(p.m)[i], vv = reinterpret_cast<float4*>(p.v)[i];
     float* wa = &w.x; float* ga = &g.x; float* ma = &mm.x; float* va = &vv.x;
+    if constexpr (L2) {
+      sg = l2_advance(s_off, p.l2s.n_seg, sg, i);
+      const float c = s_coef[sg];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) ga[j] += c * wa[j];
+    }
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       ma[j] = p.beta1 * ma[j] + (1.f - p.beta1) * ga[j];
@@ -130,7 +148,8 @@ __global__ void __launch_bounds__(DP_THREADS, 1) dp_adam_kernel(DpAdam p) {
   if (p.rank == 0 && blockIdx.x == 0 && tid == 0) {
     float a = 0.f, b = 0.f;
     for (int r = 0; r < p.world; ++r) { a += __ldcg(p.grad[r] + p.n); b += __ldcg(p.grad[r] + p.n + 1); }
-    const float loss = (p.norm[0] > 0.f ? a / p.norm[0] : 0.f) + (p.norm[1] > 0.f ? b / p.norm[1] : 0.f);
+    float loss = (p.norm[0] > 0.f ? a / p.norm[0] : 0.f) + (p.norm[1] > 0.f ? b / p.norm[1] : 0.f);
+    if constexpr (L2) loss = loss + p.l2s.reg[0];
     for (int r = 0; r < p.world; ++r) { p.param[r][p.n] = loss; p.grad[r][p.n] = 0.f; p.grad[r][p.n + 1] = 0.f; }
   }
   // ---- 4. all blocks of this rank done -> exit barrier across ranks -> release this rank's blocks
@@ -162,18 +181,26 @@ using namespace srfrd;
 
 extern "C" int srfrd_dp_adam_step(float* const* grad_ptrs_dev, float* const* param_ptrs_dev, uint32_t* const* signal_ptrs_dev,
                                   int rank, int world, int64_t n, float* m, float* v, float lr, float beta1, float beta2,
-                                  float eps, float* state8, const float* norm2, uint32_t* local4, void* stream) {
+                                  float eps, float* state8, const float* norm2, uint32_t* local4, void* stream,
+                                  const int64_t* l2_seg, int l2_n_seg, const float* l2_coef, const float* l2_reg) {
   SRFRD_REQUIRE(grad_ptrs_dev && param_ptrs_dev && signal_ptrs_dev && m && v && state8 && norm2 && local4, "dp_adam_step: null pointer");
+  const bool l2 = l2_seg != nullptr;
+  SRFRD_REQUIRE(!l2 || (l2_coef && l2_reg && l2_n_seg >= 1 && l2_n_seg <= L2_THREADS),
+                "dp_adam_step: the l2 term needs coef, reg and 1..%d segments", L2_THREADS);
   SRFRD_REQUIRE(world >= 1 && world <= DP_MAX_WORLD && rank >= 0 && rank < world, "dp_adam_step: bad rank %d / world %d", rank, world);
   SRFRD_REQUIRE(n > 0 && n % 4 == 0, "dp_adam_step: n must be a positive multiple of 4");
   DpAdam p;
   p.grad = grad_ptrs_dev; p.param = param_ptrs_dev; p.sig = signal_ptrs_dev; p.rank = rank; p.world = world; p.n = n;
   p.m = m; p.v = v; p.lr = lr; p.beta1 = beta1; p.beta2 = beta2; p.eps = eps; p.state = state8; p.norm = norm2; p.local = local4;
+  p.l2s = L2Segments{l2_seg, l2_n_seg, l2_coef, l2_reg};
   const int64_t slice4 = (n / 4 + world - 1) / world;
   int64_t grid = (slice4 + DP_THREADS - 1) / DP_THREADS;
   if (grid < 1) grid = 1;
   if (grid > num_sms()) grid = num_sms();            // every block must be resident (in-kernel grid barrier)
-  SRFRD_CUDA(launch_pdl(dp_adam_kernel, dim3((unsigned)grid), dim3(DP_THREADS), 0, (cudaStream_t)stream, p));
+  if (l2)
+    SRFRD_CUDA(launch_pdl(dp_adam_kernel<true>, dim3((unsigned)grid), dim3(DP_THREADS), 0, (cudaStream_t)stream, p));
+  else
+    SRFRD_CUDA(launch_pdl(dp_adam_kernel<false>, dim3((unsigned)grid), dim3(DP_THREADS), 0, (cudaStream_t)stream, p));
   SRFRD_LAUNCH_CHECK();
   return 0;
 }

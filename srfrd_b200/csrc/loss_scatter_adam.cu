@@ -349,14 +349,115 @@ __global__ void adam_tick_kernel(float* state, float beta1, float beta2) {
   state[3] = __uint_as_float(__float_as_uint(state[3]) + 1u);
 }
 
+// ---------------------------------------------------------------------------------------------
+// l2_emb regulariser (trainer.py:31-39: loss += l2 * torch.norm(p) for every parameter tensor p).  One launch computes,
+// for each tensor t of the flat parameter buffer, coef[t] = l2 / ||p_t|| (0 when the norm is 0: torch's gradient of the
+// norm of a zero tensor is 0) and reg = l2 * sum_t ||p_t||.  Deterministic: the buffer is cut into fixed chunks of
+// L2_CHUNK floats that never cross a tensor boundary; each chunk's sum of squares is reduced in fp64 by one block in a
+// fixed order, and the last block to finish sums the chunks of each tensor in chunk order.  No float atomics, so every
+// data-parallel replica computes bit-identical coefficients from bit-identical parameters.
+static constexpr int64_t L2_CHUNK = 8192;          // floats per chunk: 8 float4 per thread
+
+// chunk starts of each segment (exclusive prefix of ceil(numel / L2_CHUNK)); s_c0[n_seg] = total
+__device__ __forceinline__ void l2_chunk_prefix(const int64_t* seg, int n_seg, int64_t* s_c0) {
+  const int t = threadIdx.x;
+  s_c0[t + 1] = t < n_seg ? (seg[2 * t + 1] + L2_CHUNK - 1) / L2_CHUNK : 0;
+  if (t == 0) s_c0[0] = 0;
+  __syncthreads();
+  for (int d = 1; d < L2_THREADS; d <<= 1) {            // Hillis-Steele inclusive scan over s_c0[1..]
+    const int64_t a = t >= d ? s_c0[t + 1 - d] : 0;
+    __syncthreads();
+    s_c0[t + 1] += a;
+    __syncthreads();
+  }
+}
+
+__device__ __forceinline__ double block_sum_f64(double x, double* s_red) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+  if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = x;
+  __syncthreads();
+  double s = 0.0;
+  if (threadIdx.x == 0)
+    for (int w = 0; w < L2_THREADS / 32; ++w) s += s_red[w];
+  __syncthreads();
+  return s;                                             // valid in thread 0
+}
+
+// ws: [0] = uint32 blocks-done counter (zero between launches), [1 .. n_chunks] = fp64 chunk sums of squares
+__global__ void __launch_bounds__(L2_THREADS) param_l2_kernel(const float* __restrict__ p, const int64_t* __restrict__ seg,
+                                                               int n_seg, int64_t n_chunks, float l2, float* coef, float* reg,
+                                                               double* ws) {
+  __shared__ int64_t s_c0[L2_THREADS + 1];
+  __shared__ double s_red[L2_THREADS / 32];
+  __shared__ double s_norm[L2_THREADS];
+  __shared__ bool s_last;
+  pdl_prologue_done();
+  l2_chunk_prefix(seg, n_seg, s_c0);
+  double* part = ws + 1;
+  for (int64_t c = blockIdx.x; c < n_chunks; c += gridDim.x) {
+    int lo = 0, hi = n_seg - 1;                         // segment t holding chunk c: s_c0[t] <= c < s_c0[t + 1]
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if (s_c0[mid] <= c) lo = mid; else hi = mid - 1;
+    }
+    const int64_t off = seg[2 * lo], numel = seg[2 * lo + 1];
+    const int64_t b = (c - s_c0[lo]) * L2_CHUNK;        // chunk start within the segment
+    const int64_t e = min(numel, b + L2_CHUNK);
+    const float4* p4 = reinterpret_cast<const float4*>(p + off);
+    double acc = 0.0;
+#pragma unroll
+    for (int k = 0; k < (int)(L2_CHUNK / 4 / L2_THREADS); ++k) {
+      const int64_t j = b + 4 * ((int64_t)k * L2_THREADS + threadIdx.x);   // first float of this float4
+      if (j < e) {
+        const float4 x = __ldcg(p4 + j / 4);
+        const float xs[4] = {x.x, x.y, x.z, x.w};
+#pragma unroll
+        for (int q = 0; q < 4; ++q)
+          if (j + q < e) acc = fma((double)xs[q], (double)xs[q], acc);   // never reads the zero padding as data
+      }
+    }
+    const double s = block_sum_f64(acc, s_red);
+    if (threadIdx.x == 0) part[c] = s;
+  }
+  // ---- last block: per-segment sums in chunk order, then the fixed-order total
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) s_last = atomicAdd(reinterpret_cast<unsigned*>(ws), 1u) == gridDim.x - 1;
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int t = warp; t < n_seg; t += L2_THREADS / 32) {
+    double s = 0.0;
+    for (int64_t c = s_c0[t] + lane; c < s_c0[t + 1]; c += 32) s += __ldcg(part + c);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if (lane == 0) {
+      const double nrm = sqrt(s);
+      s_norm[t] = nrm;
+      coef[t] = nrm > 0.0 ? (float)((double)l2 / nrm) : 0.f;
+    }
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double tot = 0.0;
+    for (int t = 0; t < n_seg; ++t) tot += s_norm[t];
+    reg[0] = (float)((double)l2 * tot);
+    *reinterpret_cast<unsigned*>(ws) = 0u;
+  }
+}
+
 // One launch for the tail of a training step: Adam tick (step counters, bias corrections), the dense Adam update, and
 // the loss read-out.  Every block derives the NEW step state from the old one (thread 0: two pow() per block), the last
 // block to finish publishes it -- by then every block has read the old state -- and block 0 finalises the loss.
 // state8 = {step, 1 - beta1^step, 1 - beta2^step, uint32 step bits, int blocks-done counter, -, -, -}.
+// L2: g += coef[tensor] * p (the gradient of l2 * ||p_t||, from the parameters before this update) and loss += reg.
+template <bool L2>
 __global__ void __launch_bounds__(256) adam_fused_kernel(float* __restrict__ p, float* __restrict__ g, float* __restrict__ m,
                                                          float* __restrict__ v, int64_t n, float lr, float beta1, float beta2,
                                                          float eps, float* state, int zero_grad, float* acc, const float* norm,
-                                                         float* loss) {
+                                                         float* loss, L2Segments l2s) {
   __shared__ float s_bc[2];
   pdl_prologue_done();
   if (threadIdx.x == 0) {
@@ -367,17 +468,33 @@ __global__ void __launch_bounds__(256) adam_fused_kernel(float* __restrict__ p, 
   if (blockIdx.x == 0 && threadIdx.x == 32 && acc) {
     const float a = norm[0] > 0.f ? acc[0] / norm[0] : 0.f;
     const float b = norm[1] > 0.f ? acc[1] / norm[1] : 0.f;
-    loss[0] = a + b;
+    if constexpr (L2) loss[0] = a + b + l2s.reg[0];
+    else loss[0] = a + b;
     acc[0] = 0.f; acc[1] = 0.f;
+  }
+  int64_t* s_off = nullptr;
+  float* s_coef = nullptr;
+  if constexpr (L2) {
+    s_off = l2_smem().off;
+    s_coef = l2_smem().coef;
+    l2_load_starts(l2s, s_off, s_coef);
   }
   __syncthreads();
   const float step_size = lr / s_bc[0];
   const float inv_sqrt_bc2 = rsqrtf(s_bc[1]);
   const int64_t n4 = n >> 2;
+  int t = 0;
+  if constexpr (L2) t = l2_find(s_off, l2s.n_seg, (int64_t)blockIdx.x * blockDim.x + threadIdx.x);
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
     float4 pp = reinterpret_cast<float4*>(p)[i], gg = reinterpret_cast<float4*>(g)[i];
     float4 mm = reinterpret_cast<float4*>(m)[i], vv = reinterpret_cast<float4*>(v)[i];
     float* pa = &pp.x; float* ga = &gg.x; float* ma = &mm.x; float* va = &vv.x;
+    if constexpr (L2) {
+      t = l2_advance(s_off, l2s.n_seg, t, i);
+      const float c = s_coef[t];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) ga[j] += c * pa[j];
+    }
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       ma[j] = beta1 * ma[j] + (1.f - beta1) * ga[j];
@@ -624,15 +741,52 @@ extern "C" int srfrd_adam_step(float* p, float* g, float* m, float* v, int64_t n
 
 extern "C" int srfrd_adam_step_fused(float* p, float* g, float* m, float* v, int64_t n, float lr, float beta1, float beta2,
                                      float eps, float* state8, int zero_grad, float* acc2, const float* norm2, float* loss,
-                                     void* stream) {
+                                     void* stream, const int64_t* l2_seg, int l2_n_seg, const float* l2_coef,
+                                     const float* l2_reg) {
   SRFRD_REQUIRE(p && g && m && v && state8, "adam_step_fused: null pointer");
   SRFRD_REQUIRE(!acc2 || (norm2 && loss), "adam_step_fused: the loss read-out needs norm and loss");
   SRFRD_REQUIRE((((uintptr_t)p | (uintptr_t)g | (uintptr_t)m | (uintptr_t)v) & 15) == 0, "adam_step_fused: buffers must be 16-byte aligned");
+  const bool l2 = l2_seg != nullptr;
+  SRFRD_REQUIRE(!l2 || (l2_coef && l2_reg && acc2), "adam_step_fused: the l2 term needs coef, reg and the loss read-out");
+  SRFRD_REQUIRE(!l2 || (l2_n_seg >= 1 && l2_n_seg <= L2_THREADS && n % 4 == 0),
+                "adam_step_fused: l2 needs 1..%d segments and n a multiple of 4", L2_THREADS);
   int64_t blocks = (n / 4 + 255) / 256;
   if (blocks < 1) blocks = 1;
   if (blocks > num_sms() * 8) blocks = num_sms() * 8;
-  SRFRD_CUDA(launch_pdl(adam_fused_kernel, dim3((unsigned)blocks), dim3(256), 0, (cudaStream_t)stream, p, g, m, v, n, lr, beta1,
-                        beta2, eps, state8, zero_grad, acc2, norm2, loss));
+  const L2Segments l2s{l2_seg, l2_n_seg, l2_coef, l2_reg};
+  if (l2)
+    SRFRD_CUDA(launch_pdl(adam_fused_kernel<true>, dim3((unsigned)blocks), dim3(256), 0, (cudaStream_t)stream, p, g, m, v, n,
+                          lr, beta1, beta2, eps, state8, zero_grad, acc2, norm2, loss, l2s));
+  else
+    SRFRD_CUDA(launch_pdl(adam_fused_kernel<false>, dim3((unsigned)blocks), dim3(256), 0, (cudaStream_t)stream, p, g, m, v, n,
+                          lr, beta1, beta2, eps, state8, zero_grad, acc2, norm2, loss, l2s));
+  SRFRD_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int srfrd_param_l2_plan(const int64_t* seg_host, int n_seg, int64_t* n_chunks) {
+  SRFRD_REQUIRE(seg_host && n_chunks, "param_l2_plan: null pointer");
+  SRFRD_REQUIRE(n_seg >= 1 && n_seg <= L2_THREADS, "param_l2_plan: %d segments (1..%d supported)", n_seg, L2_THREADS);
+  int64_t c = 0, end = 0;
+  for (int t = 0; t < n_seg; ++t) {
+    const int64_t off = seg_host[2 * t], numel = seg_host[2 * t + 1];
+    SRFRD_REQUIRE(off % 4 == 0 && off >= end && numel >= 0, "param_l2_plan: segment %d must start 4-aligned after the last", t);
+    end = off + numel;
+    c += (numel + L2_CHUNK - 1) / L2_CHUNK;
+  }
+  *n_chunks = c;
+  return 0;
+}
+
+extern "C" int srfrd_param_l2(const float* p, const int64_t* seg, int n_seg, int64_t n_chunks, float l2, float* coef,
+                              float* reg, double* ws, void* stream) {
+  SRFRD_REQUIRE(p && seg && coef && reg && ws, "param_l2: null pointer");
+  SRFRD_REQUIRE(((uintptr_t)p & 15) == 0, "param_l2: the parameter buffer must be 16-byte aligned");
+  SRFRD_REQUIRE(n_seg >= 1 && n_seg <= L2_THREADS && n_chunks >= 0, "param_l2: bad segment / chunk count");
+  int64_t grid = n_chunks < 1 ? 1 : n_chunks;
+  if (grid > num_sms() * 8) grid = num_sms() * 8;
+  SRFRD_CUDA(launch_pdl(param_l2_kernel, dim3((unsigned)grid), dim3(L2_THREADS), 0, (cudaStream_t)stream, p, seg, n_seg,
+                        n_chunks, l2, coef, reg, ws));
   SRFRD_LAUNCH_CHECK();
   return 0;
 }

@@ -151,6 +151,11 @@ class FlatParams:
         self.grad = self.grad_bucket[:off]
         self.grad_tail = self.grad_bucket[off:]
 
+    def segments(self) -> List[Tuple[int, int]]:
+        """(offset, numel) of every parameter tensor, in the reference's registration order (= model.parameters());
+        the zero padding between tensors belongs to none of them."""
+        return [(off, int(math.prod(shape))) for off, shape in self.offsets.values()]
+
     def view(self, name: str, grad: bool = False) -> torch.Tensor:
         off, shape = self.offsets[name]
         buf = self.grad if grad else self.data

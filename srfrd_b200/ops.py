@@ -216,11 +216,40 @@ def adam_step(p, g, m, v, lr, beta1, beta2, eps, state3, zero_grad=True):
          _p(state3), int(zero_grad), _stream())
 
 
-def adam_step_fused(p, g, m, v, lr, beta1, beta2, eps, state8, zero_grad=True, acc2=None, norm2=None, loss=None):
-    """adam_tick + adam_step + loss_finalize in one launch (state8: 8 floats, see the header)."""
+def adam_step_fused(p, g, m, v, lr, beta1, beta2, eps, state8, zero_grad=True, acc2=None, norm2=None, loss=None,
+                    l2: Optional["ParamL2"] = None):
+    """adam_tick + adam_step + loss_finalize in one launch (state8: 8 floats, see the header).  With ``l2`` (after its
+    ``launch``) the gradient gains the l2_emb term and the loss its value."""
     _lib.require_device()
     call("srfrd_adam_step_fused", _p(p), _p(g), _p(m), _p(v), p.numel(), float(lr), float(beta1), float(beta2), float(eps),
-         _p(state8), int(zero_grad), _p(acc2), _p(norm2), _p(loss), _stream())
+         _p(state8), int(zero_grad), _p(acc2), _p(norm2), _p(loss), _stream(), *_l2_args(l2))
+
+
+class ParamL2:
+    """The l2_emb regulariser's per-tensor norms over a flat parameter buffer (srfrd_param_l2): ``segments`` = the
+    (offset, numel) of every parameter tensor in the buffer.  ``launch(p)`` writes ``coef[t] = l2 / ||p_t||`` (0 for a
+    zero tensor) and ``reg[0] = l2 * sum_t ||p_t||``, deterministically; the Adam entry points take the object to add
+    ``coef[t] * p`` to the gradient and ``reg`` to the loss."""
+
+    def __init__(self, segments, l2: float, device):
+        host = (C.c_int64 * (2 * len(segments)))(*[int(x) for s in segments for x in s])
+        n_chunks = C.c_int64(0)
+        call("srfrd_param_l2_plan", host, len(segments), C.byref(n_chunks))
+        self.n_seg, self.n_chunks, self.l2 = len(segments), int(n_chunks.value), float(l2)
+        self.seg = torch.tensor([int(x) for s in segments for x in s], dtype=torch.int64).to(device)
+        self.coef = torch.zeros(self.n_seg, dtype=torch.float32, device=device)
+        self.reg = torch.zeros(1, dtype=torch.float32, device=device)
+        self.ws = torch.zeros(self.n_chunks + 1, dtype=torch.float64, device=device)
+
+    def launch(self, p: torch.Tensor):
+        _lib.require_device()
+        _chk(p, torch.float32, "p")
+        call("srfrd_param_l2", _p(p), _p(self.seg), self.n_seg, self.n_chunks, self.l2, _p(self.coef), _p(self.reg),
+             _p(self.ws), _stream())
+
+
+def _l2_args(l2: Optional[ParamL2]):
+    return (None, 0, None, None) if l2 is None else (_p(l2.seg), l2.n_seg, _p(l2.coef), _p(l2.reg))
 
 
 def catalogue_topk_plan(U, n_rows, row_lo, D, n_split) -> int:
@@ -406,12 +435,13 @@ def embed_bwd_packed(dx0, seq, aux_ids, plan: PackedPlan, D, F, mode, item_scale
 
 
 def dp_adam_step(grad_ptrs_dev: int, param_ptrs_dev: int, signal_ptrs_dev: int, rank, world, n, m, v, lr, beta1, beta2, eps,
-                 state8, norm2, local4):
+                 state8, norm2, local4, l2: Optional[ParamL2] = None):
     """Reduce-scatter + Adam + all-gather over peer memory in one launch (csrc/dp_adam.cu); the *_ptrs_dev arguments are
-    device addresses of arrays of `world` peer-mapped pointers (symmetric memory handles' buffer_ptrs_dev)."""
+    device addresses of arrays of `world` peer-mapped pointers (symmetric memory handles' buffer_ptrs_dev).  ``l2``: the
+    l2_emb term of adam_step_fused, added once to the reduced gradient."""
     _lib.require_device()
     call("srfrd_dp_adam_step", grad_ptrs_dev, param_ptrs_dev, signal_ptrs_dev, int(rank), int(world), int(n), _p(m), _p(v),
-         float(lr), float(beta1), float(beta2), float(eps), _p(state8), _p(norm2), _p(local4), _stream())
+         float(lr), float(beta1), float(beta2), float(eps), _p(state8), _p(norm2), _p(local4), _stream(), *_l2_args(l2))
 
 
 def _parts(parts):

@@ -6,7 +6,8 @@
 ``FusedTrainer``  -- the B200-first step: ids and discriminator weights are copied to static device buffers,
                      then ONE captured CUDA graph runs forward -> fused weighted BCE (forward+backward, no
                      ``nonzero`` sync, trainer.py:36) -> backward -> [gradient all-reduce] -> flat Adam ->
-                     bf16 shadow refresh.  The loss stays on the device until the caller asks for it.
+                     bf16 shadow refresh; with l2_emb > 0 the per-tensor norms of the regulariser run on a side
+                     stream next to the forward.  The loss stays on the device until the caller asks for it.
 """
 from __future__ import annotations
 
@@ -91,13 +92,15 @@ class FusedTrainer:
     use_graph    : capture the step in a CUDA graph after the first (eager) step.
     packed       : run the encoder on the packed token layout (csrc/pack.cu) -- pad slots, ~88 % of a Beauty-shaped batch,
                    are not computed; results equal the dense path (None = on when the shape supports it).
+    l2_emb       : the reference's regulariser (trainer.py:31-39): the loss gains l2_emb * sum_p ||p||_2 over every tensor
+                   of model.parameters() (plain norm, not squared) and each gradient l2_emb * p / ||p|| (0 for a zero
+                   tensor), both from the parameters before the step's update.  The norm gradient reaches every row of the
+                   embedding tables, the pad row included, so rows no batch touches drift under Adam as in the reference.
+                   Fixed for the trainer's lifetime (a captured graph holds it).
     """
 
     def __init__(self, model, lr: float = 1e-3, betas=(0.9, 0.98), eps: float = 1e-8, process_group=None,
                  use_graph: bool = True, l2_emb: float = 0.0, packed: Optional[bool] = None):
-        if l2_emb != 0.0:
-            raise NotImplementedError("FusedTrainer implements the reference default l2_emb = 0.0 (trainer.py:123); "
-                                      "use simulate() with a torch optimizer for l2_emb != 0")
         self.model = model
         self._dp = None
         if process_group is not None and torch.distributed.get_world_size(process_group) > 1:
@@ -121,9 +124,20 @@ class FusedTrainer:
         self._graph_key = None
         self._eager_key = None
         self._has_w = (False, False)
+        self.l2_emb = float(l2_emb)
+        self._l2 = self._setup_l2(model) if self.l2_emb != 0.0 else None
         self.P.grad_bucket.zero_()
         self.eng.refresh_shadows()
         self.steps = 0
+
+    def _setup_l2(self, model) -> ops.ParamL2:
+        """The regulariser's segment table: every tensor of model.parameters() is one segment of the flat buffer."""
+        segs = self.P.segments()
+        base = self.P.data.data_ptr()
+        mine = sorted((p.data_ptr(), p.numel()) for p in model.parameters())
+        assert mine == [(base + 4 * off, n) for off, n in segs], \
+            "srfrd_b200: l2_emb: the flat parameter segments do not cover exactly model.parameters()"
+        return ops.ParamL2(segs, self.l2_emb, self.eng.device)
 
     # ------------------------------------------------------------------
     @staticmethod
@@ -203,6 +217,11 @@ class FusedTrainer:
             ops.weight_sums(pos, w_pos, w_neg, norm)
             if self.pg is not None:
                 parallel.allreduce_sum_(norm, self.pg)
+            if self._l2 is not None:
+                # the norms of the parameters the previous step left behind, next to the forward pass; the join below
+                # orders them before Adam (in the fused data-parallel kernel, peers overwrite this buffer once this rank
+                # reaches its entry barrier, which only stream order can delay)
+                self._l2.launch(P.data)
         packed = self.packed and eng.packed_ok(B, L)
         # packed token layout: pad slots (88 % of a C2 batch) get no rows; slots whose POSITIVE id is set keep one even if
         # their input is a pad, because the loss reads their hidden state
@@ -227,13 +246,13 @@ class FusedTrainer:
             # peer memory (csrc/dp_adam.cu) instead of an NCCL all-reduce followed by the same Adam on every rank
             d = self._dp
             ops.dp_adam_step(d["g"], d["p"], d["s"], d["rank"], d["world"], P.numel, self.m, self.v, self.lr, self.betas[0],
-                             self.betas[1], self.eps, eng.step_state, norm, d["local"])
+                             self.betas[1], self.eps, eng.step_state, norm, d["local"], l2=self._l2)
         else:
             if self.pg is not None:
                 parallel.allreduce_sum_(P.grad_bucket, self.pg)           # ONE NCCL sum over NVLink: gradients + loss sums
             # Adam tick + dense Adam + loss read-out (consumes acc: zero again for the next step) in one launch
             ops.adam_step_fused(P.data, P.grad, self.m, self.v, self.lr, self.betas[0], self.betas[1], self.eps,
-                                eng.step_state, zero_grad=True, acc2=acc, norm2=norm, loss=loss)
+                                eng.step_state, zero_grad=True, acc2=acc, norm2=norm, loss=loss, l2=self._l2)
         eng.refresh_shadows()
 
     # ------------------------------------------------------------------

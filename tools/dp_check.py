@@ -1,5 +1,6 @@
 """Multi-GPU check (run under torchrun): G-rank data-parallel FusedTrainer == 1-rank on the concatenated batch,
-and row-sharded catalogue top-10 (NCCL all-gather + merge) == unsharded top-10."""
+and row-sharded catalogue top-10 (NCCL all-gather + merge) == unsharded top-10.
+`--l2 X` trains both with l2_emb = X (the regulariser's gradient is added once, after the reduction over ranks)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -29,12 +30,13 @@ batches = [smp.next_batch(64 * world) for _ in range(6)]
 m_dp, m_one = make_model(), make_model()
 P.broadcast_parameters(m_dp.flat_parameters().data, 0)
 use_graph = os.environ.get("DP_CHECK_GRAPH", "0") == "1"
-tr_dp = FusedTrainer(m_dp, process_group=dist.group.WORLD, use_graph=use_graph)
+l2_emb = float(sys.argv[sys.argv.index("--l2") + 1]) if "--l2" in sys.argv else 0.0
+tr_dp = FusedTrainer(m_dp, process_group=dist.group.WORLD, use_graph=use_graph, l2_emb=l2_emb)
 if rank == 0:
-    print("fused reduce-scatter/Adam/all-gather kernel:", tr_dp._dp is not None, "graph:", use_graph)
-tr_one = FusedTrainer(m_one, use_graph=False)
+    print("fused reduce-scatter/Adam/all-gather kernel:", tr_dp._dp is not None, "graph:", use_graph, "l2_emb:", l2_emb)
+tr_one = FusedTrainer(m_one, use_graph=False, l2_emb=l2_emb)
 ok = True
-for nb in batches:
+for i, nb in enumerate(batches):
     full = {k: torch.from_numpy(v).to(dev) for k, v in nb.items()}
     w = discriminator_weights(full["pos"], full["p_fake"], "soft")
     l1 = float(tr_one.step(full, w_pos=w))
@@ -43,6 +45,11 @@ for nb in batches:
     if rank == 0:
         print(f"loss single {l1:.6f}  dp{world} {l2:.6f}")
     ok &= abs(l1 - l2) < 2e-3
+    if i == 0:                      # the first step's parameters, before Adam amplifies bf16 noise into sign flips
+        d0 = float((m_one.flat_parameters().data - m_dp.flat_parameters().data).abs().max())
+        if rank == 0:
+            print(f"param drift after the first step {d0:.2e}")
+        ok &= d0 < 2e-3
 a, b = m_one.flat_parameters().data, m_dp.flat_parameters().data
 drift = float((a - b).abs().max())
 # replicas must be bit-identical (every element is computed by exactly one rank and written everywhere)
