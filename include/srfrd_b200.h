@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define SRFRD_ABI_VERSION 7
+#define SRFRD_ABI_VERSION 8
 #if defined(__GNUC__)
 #define SRFRD_API __attribute__((visibility("default")))
 #else
@@ -213,21 +213,32 @@ SRFRD_API int srfrd_param_l2_plan(const int64_t* seg_host, int n_seg, int64_t* n
 SRFRD_API int srfrd_param_l2(const float* p, const int64_t* seg, int n_seg, int64_t n_chunks, float l2, float* coef,
                    float* reg, double* ws, void* stream);
 
-/* ---- K8/K9: full-catalogue scoring fused with a streaming per-row top-10 ----
+/* ---- K8/K9: full-catalogue scoring fused with a streaming per-row top-k, 1 <= k <= SRFRD_TOPK_KMAX ----
  * replaces: SRFR_model.py:144-152 predict() called with label = arange(1, N+1) + the double argsort of
  * utils.py:591, i.e. rank by (score desc, item id asc).
+ * List length rule: every list below is L = max(k, 10) entries long -- the (U, chunks, L) partial lists, the packed
+ * wire row of 2L words and the input lists of srfrd_merge_topk / srfrd_merge_topk_packed.  k <= 10 runs the top-10
+ * kernels (a smaller k is the prefix of the top-10, exact under the tie-break); k > 10 runs their k-list variants,
+ * which only the unit form serves (n_split * D <= 256) and whose per-row lists must fit shared memory: the plan refuses
+ * a k above srfrd_catalogue_topk_kmax(D, n_split) (64 at D = 64 and at D = 128 with one split, 48 at D = 256).
  * feats: bf16 (n_split stacked blocks of u_pad rows, D); table: bf16 (n_rows, D); candidates are local
- * rows [row_lo, n_rows) with global id = id_base + row.  Writes (U, chunks, 10) partial lists that
- * srfrd_merge_topk reduces (also used for the cross-GPU all-gather merge). */
-SRFRD_API int srfrd_catalogue_topk_plan(int64_t U, int64_t n_rows, int64_t row_lo, int D, int n_split, int* chunks_out);
+ * rows [row_lo, n_rows) with global id = id_base + row.  Writes (U, chunks, L) partial lists whose chunk 0 holds each
+ * user's exact local top-k, sorted, (-inf, -1) past the end, the other chunks emptied (ids -1); srfrd_merge_topk reduces
+ * them (also used for the cross-GPU merge).  For k > 10 the merge inputs must be such sorted lists. */
+#define SRFRD_TOPK_KMAX 64
+SRFRD_API int srfrd_catalogue_topk_plan(int64_t U, int64_t n_rows, int64_t row_lo, int D, int n_split, int* chunks_out,
+                                        int k);
+/* largest k the plan accepts for this width and split (10 where only the tile form runs) */
+SRFRD_API int srfrd_catalogue_topk_kmax(int D, int n_split, int* kmax_out);
 SRFRD_API int srfrd_catalogue_topk(const void* feats_bf16, int64_t U, int64_t u_pad, int n_split, const void* table_bf16,
                          int64_t n_rows, int64_t row_lo, int64_t id_base, int D, int ld_feats, int ld_table,
-                         int chunks, float* part_scores, int* part_ids, float* packed_out, void* stream);
+                         int chunks, float* part_scores, int* part_ids, float* packed_out, void* stream, int k);
 SRFRD_API int srfrd_merge_topk(const float* scores, const int* ids, int64_t U, int nlists, int k, float* out_scores,
                      int64_t* out_ids, void* stream);
-/* Row-sharded scoring: packed_out (nullable, (U, 20) fp32 words) receives each user's final local list as 10 fp32 scores
- * followed by 10 int32 global ids -- 80 B per user, the send buffer of ONE all-gather; srfrd_merge_topk_packed merges the
- * gathered (nlists, U, 20) buffer (list l of user u at word (l * U + u) * 20) into the global top-k, identical on every rank. */
+/* Row-sharded scoring: packed_out (nullable, (U, 2L) fp32 words) receives each user's final local list as L fp32 scores
+ * followed by L int32 global ids -- 8L B per user (80 B at k <= 10), the send buffer of ONE all-gather;
+ * srfrd_merge_topk_packed merges the gathered (nlists, U, 2L) buffer (list l of user u at word (l * U + u) * 2L) into the
+ * global top-k, identical on every rank. */
 SRFRD_API int srfrd_merge_topk_packed(const float* packed, int64_t U, int nlists, int k, float* out_scores,
                             int64_t* out_ids, void* stream);
 

@@ -81,8 +81,9 @@ SIGNATURES = {
     "srfrd_adam_step_fused": [vp, vp, vp, vp, i64, f32, f32, f32, f32, vp, i32, vp, vp, vp, vp, vp, i32, vp, vp],
     "srfrd_param_l2_plan": [C.POINTER(i64), i32, C.POINTER(i64)],
     "srfrd_param_l2": [vp, vp, i32, i64, f32, vp, vp, vp, vp],
-    "srfrd_catalogue_topk_plan": [i64, i64, i64, i32, i32, C.POINTER(i32)],
-    "srfrd_catalogue_topk": [vp, i64, i64, i32, vp, i64, i64, i64, i32, i32, i32, i32, vp, vp, vp, vp],
+    "srfrd_catalogue_topk_plan": [i64, i64, i64, i32, i32, C.POINTER(i32), i32],
+    "srfrd_catalogue_topk_kmax": [i32, i32, C.POINTER(i32)],
+    "srfrd_catalogue_topk": [vp, i64, i64, i32, vp, i64, i64, i64, i32, i32, i32, i32, vp, vp, vp, vp, i32],
     "srfrd_merge_topk_packed": [vp, i64, i32, i32, vp, vp, vp],
     "srfrd_attention_live_items": [vp, i64, i32, i32, vp, vp, vp, vp],
     "srfrd_set_attention_live": [vp, vp, vp, vp],
@@ -131,7 +132,7 @@ def load() -> C.CDLL:
         fn = getattr(lib, name)            # AttributeError if the symbol is not exported
         fn.argtypes = argtypes
         fn.restype = C.c_int
-    if lib.srfrd_abi_version() != 7:
+    if lib.srfrd_abi_version() != 8:
         raise RuntimeError("srfrd_b200: ABI version mismatch between _lib.py and the built library")
     _lib = lib
     return lib

@@ -19,6 +19,9 @@
 //     same bf16 operands, fp32 accumulation, order (score desc, id asc); writes the row's final list (and, for the
 //     row-sharded protocol, the 80-byte wire format of the all-gather).
 // n_split = 2/3 feeds hi/lo bf16 splits of the fp32 user features as extra K (near-fp32 scores).
+// k <= 10 runs these top-10 kernels (a smaller k is the prefix of their lists).  10 < k <= KMAX runs compile-time k-list
+// variants (catalogue_unitmax_kernel<.., KLIST = true>, catalogue_refine_k_kernel, merge_topk_k_kernel) with lists of k
+// entries everywhere; only the unit form serves them, and the host plan refuses a k whose lists do not fit (topk_kmax).
 #include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -29,6 +32,8 @@
 namespace srfrd {
 
 static constexpr int TK = 10;               // list length kept per row
+static constexpr int KMAX = SRFRD_TOPK_KMAX;  // longest list of the k-list kernels (k > TK)
+static constexpr int KL_ROWS = 256;         // rows (epilogue threads) whose lists a unit-form CTA keeps in shared memory
 static constexpr int TILE_U = 128;          // users per MMA (TMEM lanes)
 static constexpr int KB = 64;               // k-block (bf16 elements)
 
@@ -53,6 +58,9 @@ struct TopkShape {
   int* out_ids;           // (U, slots, TK)  phase 1: tile indices (-1 = empty); phase 2: global item ids in slot 0
   float* packed;          // optional (U, 2 * TK): the row's final list as TK fp32 scores followed by TK int32 global ids
                           // -- the send buffer of the row-sharded all-gather (80 B per user), written by phase 2
+  int k;                  // list length of the k-list kernels (11 .. KMAX); the TK kernels never read it.  Every list
+                          // buffer above is then k entries long instead of TK (last field: the TK kernels' parameter
+                          // offsets are unchanged)
 };
 
 // D[tmem] (+)= A[tmem] * B[smem]
@@ -398,7 +406,14 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
                : "memory");
 }
 
-template <int MT, bool TRACE>
+//
+// KLIST: the k-list variant (k = s.k in TK + 1 .. KMAX).  A k-long list per row does not fit in registers next to the MT
+// scores, so the 256 rows' lists live in shared memory after the barriers, entry j of thread x at [j * 256 + x] (bank-
+// conflict free), UNSORTED: an insertion overwrites the current worst entry (lowest maximum; among equal maxima the
+// highest unit, which the order (max desc, unit asc) ranks last) and rescans the k entries for the new worst -- no shifts,
+// no dependent chain.  The strict v > thr test stays: units reach a thread in increasing index order, so an equal maximum
+// never displaces an earlier unit.  The proof above holds with TK replaced by k.  Everything else is the same code.
+template <int MT, bool TRACE, bool KLIST = false>
 __global__ void __launch_bounds__(384, 1)
 catalogue_unitmax_kernel(const __grid_constant__ CUtensorMap tmE, TopkShape s) {
   constexpr int UBS = 2, NEPI = 8, NACC = 4;
@@ -555,21 +570,40 @@ catalogue_unitmax_kernel(const __grid_constant__ CUtensorMap tmE, TopkShape s) {
         __syncwarp();
         if (lane == 0) mbar_arrive(afull);
       }
-      float ts[TK]; int ti[TK];                       // this row's TK best (unit maximum, unit index), sorted
+      constexpr int TKR = KLIST ? 1 : TK;               // register list (unused by the k-list variant)
+      float ts[TKR]; int ti[TKR];                       // this row's TK best (unit maximum, unit index), sorted
 #pragma unroll
-      for (int r = 0; r < TK; ++r) { ts[r] = -INFINITY; ti[r] = -1; }
+      for (int r = 0; r < TKR; ++r) { ts[r] = -INFINITY; ti[r] = -1; }
       float thr = -INFINITY;
+      float* kls = nullptr; int* kli = nullptr;         // k-list variant: this thread's list in shared memory
+      int kworst = 0;                                   //   and the slot of its worst entry
+      if constexpr (KLIST) {
+        kls = reinterpret_cast<float*>(bars + 2 * s.stages + 32) + threadIdx.x;
+        kli = reinterpret_cast<int*>(kls - threadIdx.x + s.k * KL_ROWS) + threadIdx.x;
+        for (int j = 0; j < s.k; ++j) { kls[j * KL_ROWS] = -INFINITY; kli[j * KL_ROWS] = -1; }
+      }
       auto offer = [&](float v, int id) {               // rare after warm-up, thread-divergent
         if (v > thr && s.debug != 1) {
-          ts[TK - 1] = v; ti[TK - 1] = id;
-#pragma unroll
-          for (int r = TK - 1; r > 0; --r) {            // strict: an equal maximum never overtakes an earlier unit
-            if (ts[r] > ts[r - 1]) {
-              const float fs = ts[r]; ts[r] = ts[r - 1]; ts[r - 1] = fs;
-              const int is = ti[r]; ti[r] = ti[r - 1]; ti[r - 1] = is;
+          if constexpr (KLIST) {
+            kls[kworst * KL_ROWS] = v; kli[kworst * KL_ROWS] = id;
+            float wv = kls[0]; int wi = kli[0], wj = 0;
+#pragma unroll 8
+            for (int j = 1; j < s.k; ++j) {
+              const float x = kls[j * KL_ROWS]; const int xi = kli[j * KL_ROWS];
+              if (x < wv || (x == wv && xi > wi)) { wv = x; wi = xi; wj = j; }
             }
+            thr = wv; kworst = wj;
+          } else {
+            ts[TK - 1] = v; ti[TK - 1] = id;
+#pragma unroll
+            for (int r = TK - 1; r > 0; --r) {          // strict: an equal maximum never overtakes an earlier unit
+              if (ts[r] > ts[r - 1]) {
+                const float fs = ts[r]; ts[r] = ts[r - 1]; ts[r - 1] = fs;
+                const int is = ti[r]; ti[r] = ti[r - 1]; ti[r - 1] = is;
+              }
+            }
+            thr = ts[TK - 1];
           }
-          thr = ts[TK - 1];
         }
       };
       auto reduce_half = [&](uint32_t (&r0)[32], uint32_t (&r1)[16], uint32_t (&r2)[8], int limit) {
@@ -647,7 +681,15 @@ catalogue_unitmax_kernel(const __grid_constant__ CUtensorMap tmE, TopkShape s) {
         offer(mB, 2 * t + 1);
         if (tr) trq[8] = clock64();
       }
-      if (urow < s.U) {
+      if constexpr (KLIST) {
+        if (urow < s.U) {
+          const size_t o = ((size_t)urow * s.slots + piece * 2) * s.k;  // unsorted; phase 2 selects from it
+          for (int r = 0; r < s.k; ++r) {
+            s.out_scores[o + r] = kls[r * KL_ROWS];
+            s.out_ids[o + r] = kli[r * KL_ROWS];
+          }
+        }
+      } else if (urow < s.U) {
         const size_t o = ((size_t)urow * s.slots + piece * 2) * TK;     // the piece's second list slot stays empty
 #pragma unroll
         for (int r = 0; r < TK; ++r) {
@@ -947,6 +989,239 @@ __global__ void __launch_bounds__(256, 2) catalogue_refine64_kernel(TopkShape s)
   }
 }
 
+// Phase 2, k-list form (k = s.k in TK + 1 .. KMAX; unit form only, so a ranking unit is s.nt <= 56 rows).  One warp per
+// user row, same contract as the two kernels above:
+//   1. the k best units (max desc, unit asc): k rounds of warp arg-best over the row's (unsorted) per-piece lists;
+//   2. the exact scores of their k x RU rows, same bf16 operands, fp32 accumulation, into this warp's shared memory.
+//      RU = 56: the coalesced D = 64 form of catalogue_refine64_kernel (a unit is RU / 4 512-byte requests, a row's
+//      score an 8-lane butterfly); RU = 0: one row per lane as in catalogue_refine_kernel (other widths and splits);
+//   3. tau = the minimum exact unit maximum (-inf when the row has fewer than k units): the k-th best score is >= tau,
+//      so only scores >= tau survive, typically k .. 2k of k x RU, compacted with (score, row);
+//   4. order by counting: a survivor's rank is the number of survivors ahead of it in (score desc, row asc).  More than
+//      KSCAP survivors (dyadic data with mass ties: every one of the k x RU scores can tie) take k selection rounds over
+//      all k x RU scores instead;
+//   5. slot 0 of the row's lists (and, when requested, the 8k-byte wire row) gets the k best, (-inf, -1) past the end.
+static constexpr int KSCAP = 256;                     // survivors ordered by counting
+static constexpr int KWARPS = 8;                      // warps (user rows) per block
+__host__ __device__ constexpr size_t refine_k_warp_bytes(int k, int ru) {
+  return (size_t)k * ru * 4 + (size_t)k * 4 + (size_t)KSCAP * 8;
+}
+
+template <int RU>
+__global__ void __launch_bounds__(32 * KWARPS) catalogue_refine_k_kernel(TopkShape s) {
+  static_assert(RU == 0 || RU == 56, "refine_k: RU 56 (D = 64) or 0 (general)");
+  extern __shared__ uint8_t smem_raw[];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const int64_t u = (int64_t)blockIdx.x * KWARPS + wib;
+  if (u >= s.U) return;
+  const int k = s.k, ru = RU ? RU : s.nt, ncand = k * ru;
+  uint8_t* wsm = smem_raw + (size_t)wib * refine_k_warp_bytes(k, ru);
+  float* sc = reinterpret_cast<float*>(wsm);                       // [k][ru] exact scores
+  int* units = reinterpret_cast<int*>(sc + ncand);                 // [k] chosen units (-1: the row has fewer)
+  float* sv = reinterpret_cast<float*>(units + k);                 // [KSCAP] survivors
+  int* si = reinterpret_cast<int*>(sv + KSCAP);
+  float* osc = s.out_scores + (size_t)u * s.slots * k;
+  int* oid = s.out_ids + (size_t)u * s.slots * k;
+  const int nent = s.slots * k;
+  // ---- 1. the k best units
+  {
+    float last_v = INFINITY; int last_t = -1;
+#pragma unroll 1
+    for (int r = 0; r < k; ++r) {
+      float bv = -INFINITY; int bt = -1;
+      for (int e = lane; e < nent; e += 32) {
+        const float v = osc[e]; const int t = oid[e];
+        if (t < 0) continue;
+        const bool after_last = (last_t < 0) || v < last_v || (v == last_v && t > last_t);
+        if (after_last && better(v, t, bv, bt)) { bv = v; bt = t; }
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+        const int ot = __shfl_xor_sync(0xffffffffu, bt, o);
+        if (better(ov, ot, bv, bt)) { bv = ov; bt = ot; }
+      }
+      if (lane == 0) units[r] = bt;
+      if (bt >= 0) { last_v = bv; last_t = bt; }
+    }
+  }
+  __syncwarp();
+  for (int e = lane; e < nent; e += 32) oid[e] = -1;    // empty every slot (phase-1 entries are consumed)
+  // ---- 2. exact scores of the k units, tau
+  float tau = INFINITY;
+  if constexpr (RU != 0) {
+    constexpr int NI = RU / 4;
+    float f[8];                                         // this lane's eighth of the user's features
+    {
+      const uint4 fv = __ldg(reinterpret_cast<const uint4*>(s.feats + (size_t)u * s.ld_feats) + (lane & 7));
+      const uint32_t fw[4] = {fv.x, fv.y, fv.z, fv.w};
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        const float2 x = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&fw[q]));
+        f[2 * q] = x.x; f[2 * q + 1] = x.y;
+      }
+    }
+#pragma unroll 1
+    for (int r = 0; r < k; ++r) {
+      const int t = units[r];
+      if (t < 0) { tau = -INFINITY; continue; }         // warp-uniform
+      const int row0 = s.row_lo + t * RU + (lane >> 3);
+      const uint4* e0 = reinterpret_cast<const uint4*>(s.table + (size_t)row0 * 64) + (lane & 7);
+      uint4 ev[NI];
+#pragma unroll
+      for (int i = 0; i < NI; ++i)
+        ev[i] = (row0 + 4 * i < s.row_hi) ? __ldg(e0 + i * 32) : make_uint4(0, 0, 0, 0);
+      float um = -INFINITY;
+#pragma unroll
+      for (int i = 0; i < NI; ++i) {
+        const uint32_t ew[4] = {ev[i].x, ev[i].y, ev[i].z, ev[i].w};
+        float a = 0.f;
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          const float2 y = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&ew[q]));
+          a = fmaf(f[2 * q], y.x, a);
+          a = fmaf(f[2 * q + 1], y.y, a);
+        }
+        a += __shfl_xor_sync(0xffffffffu, a, 1);
+        a += __shfl_xor_sync(0xffffffffu, a, 2);
+        a += __shfl_xor_sync(0xffffffffu, a, 4);
+        if (row0 + 4 * i >= s.row_hi) a = -INFINITY;     // past the table: not an item
+        um = fmaxf(um, a);
+        if ((lane & 7) == 0) sc[r * RU + 4 * i + (lane >> 3)] = a;
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) um = fmaxf(um, __shfl_xor_sync(0xffffffffu, um, o));
+      tau = fminf(tau, um);
+    }
+  } else {
+#pragma unroll 1
+    for (int r = 0; r < k; ++r) {
+      const int t = units[r];
+      if (t < 0) { tau = -INFINITY; continue; }         // warp-uniform
+      float um = -INFINITY;
+      for (int j = lane; j < ru; j += 32) {
+        const int row = s.row_lo + t * ru + j;
+        float acc = -INFINITY;                          // past the table: not an item
+        if (row < s.row_hi) {
+          const uint4* e = reinterpret_cast<const uint4*>(s.table + (size_t)row * s.ld_table);
+          acc = 0.f;
+          for (int sp = 0; sp < s.n_split; ++sp) {
+            const uint4* f = reinterpret_cast<const uint4*>(s.feats + ((size_t)sp * s.u_pad + u) * s.ld_feats);
+            float a = 0.f;
+            for (int c = 0; c < s.D / 8; ++c) {
+              const uint4 fv = __ldg(f + c), ev = __ldg(e + c);
+              const uint32_t fw[4] = {fv.x, fv.y, fv.z, fv.w}, ew[4] = {ev.x, ev.y, ev.z, ev.w};
+#pragma unroll
+              for (int q = 0; q < 4; ++q) {
+                const float2 x = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&fw[q]));
+                const float2 y = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&ew[q]));
+                a = fmaf(x.x, y.x, a);
+                a = fmaf(x.y, y.y, a);
+              }
+            }
+            acc += a;
+          }
+        }
+        sc[r * ru + j] = acc;
+        um = fmaxf(um, acc);
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) um = fmaxf(um, __shfl_xor_sync(0xffffffffu, um, o));
+      tau = fminf(tau, um);
+    }
+  }
+  __syncwarp();
+  // ---- 3. survivors (score >= tau) -> (sv, si), as many as fit; ns counts them all
+  int ns = 0;
+  for (int e0 = 0; e0 < ncand; e0 += 32) {
+    const int e = e0 + lane;
+    const int t = e < ncand ? units[e / ru] : -1;
+    const float a = t >= 0 ? sc[e] : -INFINITY;
+    const bool keep = a >= tau && a > -INFINITY;
+    const uint32_t m = __ballot_sync(0xffffffffu, keep);
+    const int at = ns + __popc(m & ((1u << lane) - 1));
+    if (keep && at < KSCAP) { sv[at] = a; si[at] = s.row_lo + t * ru + e % ru; }
+    ns += __popc(m);
+  }
+  __syncwarp();
+  // ---- 4./5. order and write
+  float* pk = s.packed ? s.packed + (size_t)u * 2 * k : nullptr;
+  auto put = [&](int r, float v, int row) {
+    const int gid = row < 0 ? -1 : (int)(s.id_base + row);
+    osc[r] = v; oid[r] = gid;
+    if (pk) { pk[r] = v; reinterpret_cast<int*>(pk)[k + r] = gid; }
+  };
+  if (ns <= KSCAP) {
+    for (int e = lane; e < ns; e += 32) {
+      const float v = sv[e]; const int row = si[e];
+      int rank = 0;
+      for (int j = 0; j < ns; ++j) rank += (sv[j] > v || (sv[j] == v && si[j] < row)) ? 1 : 0;
+      if (rank < k) put(rank, v, row);
+    }
+    for (int r = ns + lane; r < k; r += 32) put(r, -INFINITY, -1);   // fewer than k items: the tail is empty
+  } else {
+    float last_v = INFINITY; int last_i = -1;
+#pragma unroll 1
+    for (int r = 0; r < k; ++r) {
+      float bv = -INFINITY; int bi = -1;
+      for (int e = lane; e < ncand; e += 32) {
+        const int t = units[e / ru];
+        if (t < 0) continue;
+        const float v = sc[e]; const int id = s.row_lo + t * ru + e % ru;
+        if (v == -INFINITY) continue;                   // past the table
+        const bool after_last = (last_i < 0) || v < last_v || (v == last_v && id > last_i);
+        if (after_last && better(v, id, bv, bi)) { bv = v; bi = id; }
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+        const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+        if (better(ov, oi, bv, bi)) { bv = ov; bi = oi; }
+      }
+      if (lane == 0) put(r, bv, bi);
+      if (bi >= 0) { last_v = bv; last_i = bi; }
+    }
+  }
+}
+
+// K9 for lists of L = k > TK entries, SORTED by (score desc, id asc) with empty entries (id < 0) only at the tail -- what
+// phase 2 writes.  One warp per user.  The first k entries of every list are the only candidates; an entry's rank is its
+// position in its own list plus, for every other list, the count of entries ahead of it (binary search: the lists are
+// sorted).  Equal (score, id) in two lists are ordered by list index, so ranks are distinct and the result is the same
+// on every rank that merges the same buffer.  List l of user u starts at word u * u_stride + l * l_stride of `sc` and
+// of `ids`.
+__global__ void __launch_bounds__(256) merge_topk_k_kernel(const float* sc, const int* ids, int64_t u_stride,
+                                                           int64_t l_stride, int64_t U, int nlists, int k, float* out_sc,
+                                                           int64_t* out_ids) {
+  const int lane = threadIdx.x & 31;
+  const int64_t u = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (u >= U) return;
+  for (int r = lane; r < k; r += 32) { out_sc[u * k + r] = -INFINITY; out_ids[u * k + r] = -1; }
+  __syncwarp();
+  const float* s0 = sc + u * u_stride;
+  const int* i0 = ids + u * u_stride;
+  for (int e = lane; e < nlists * k; e += 32) {
+    const int l = e / k, p = e % k;
+    const float v = s0[l * l_stride + p]; const int id = i0[l * l_stride + p];
+    if (id < 0) continue;
+    int rank = p;
+    for (int m = 0; m < nlists && rank < k; ++m) {
+      if (m == l) continue;
+      const float* sm = s0 + m * l_stride;
+      const int* im = i0 + m * l_stride;
+      int lo = 0, hi = k;                               // first entry of list m that is NOT ahead of (v, id, l)
+      while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        const float y = sm[mid]; const int yi = im[mid];
+        const bool ahead = yi >= 0 && (y > v || (y == v && (yi < id || (yi == id && m < l))));
+        if (ahead) lo = mid + 1; else hi = mid;
+      }
+      rank += lo;
+    }
+    if (rank < k) { out_sc[u * k + rank] = v; out_ids[u * k + rank] = id; }
+  }
+}
+
 // K9: merge `nlists` candidate lists of length TK per user into the best k, order (score desc, id asc).
 __global__ void merge_topk_kernel(const float* sc, const int* ids, int64_t U, int nlists, int k, float* out_sc,
                                   int64_t* out_ids) {
@@ -1071,11 +1346,55 @@ static TopkPlan make_plan(const TopkCfg& c, int64_t U, int64_t n_rows, int64_t r
   return p;
 }
 
-extern "C" int srfrd_catalogue_topk_plan(int64_t U, int64_t n_rows, int64_t row_lo, int D, int n_split, int* chunks_out) {
+// Shared memory of the unit form (bytes, 227 KB a block): ring of `stages` k-blocks of MT item rows, the barrier area
+// (2 * stages + 32 words), the k-list variant's 256 per-row lists of k (score, unit) pairs, alignment slack.
+static constexpr int UNIT_SMEM_MAX = 227 * 1024;
+static size_t unit_smem_bytes(int mt, int stages, int k) {
+  return (size_t)stages * mt * KB * 2 + (size_t)(2 * stages + 32) * 8 + (k > TK ? (size_t)KL_ROWS * k * 8 : 0) + 2048;
+}
+// Ring length (k-blocks) of the unit form.  TK form: what 216 KB holds.  k-list variant: that, shortened to what its lists
+// leave; a multiple of 2 * kblocks (each slot's parity belongs to two issuers) and at least 4 item tiles (tile n - 2's
+// slot is refilled only after tile n's MMAs are issued); 0 = does not fit.
+static int unit_stages(int mt, int kblocks, int k) {
+  const int b_tile = mt * KB * 2, unit = 2 * kblocks;
+  int stages = ((216 * 1024) / b_tile) / unit * unit;
+  if (k <= TK) return stages;
+  while (stages >= 2 * unit && unit_smem_bytes(mt, stages, k) > (size_t)UNIT_SMEM_MAX) stages -= unit;
+  return stages >= 2 * unit ? stages : 0;
+}
+// Largest list length the plan serves for this width: TK for the tile form, else the largest k <= KMAX whose lists fit
+// next to a 4-tile ring (D = 64: 64; D = 128, one split: 64; D = 256: 48).
+static int topk_kmax(const TopkCfg& c, int D) {
+  if (c.ubs == 0 || c.nacc != 4) return c.ubs ? TK : 0;
+  int k = KMAX;
+  while (k > TK && !unit_stages(c.nt, (D + KB - 1) / KB, k)) --k;
+  return k;
+}
+static int check_k(const TopkCfg& c, int D, int n_split, int k) {
+  SRFRD_REQUIRE(c.ubs > 0, "catalogue_topk: D=%d with n_split=%d does not fit tensor memory", D, n_split);
+  SRFRD_REQUIRE(k >= 1 && k <= KMAX, "catalogue_topk: k must be in 1..%d (got %d)", KMAX, k);
+  SRFRD_REQUIRE(k <= TK || c.nacc == 4, "catalogue_topk: k=%d > %d needs the unit form; D=%d with n_split=%d runs the tile "
+                "form (n_split * D > 256), which keeps at most %d", k, TK, D, n_split, TK);
+  const int kmax = topk_kmax(c, D);
+  SRFRD_REQUIRE(k <= kmax, "catalogue_topk: k=%d exceeds the limit %d for D=%d with n_split=%d (the per-row lists must fit "
+                "shared memory next to a 4-tile ring)", k, kmax, D, n_split);
+  return 0;
+}
+
+extern "C" int srfrd_catalogue_topk_plan(int64_t U, int64_t n_rows, int64_t row_lo, int D, int n_split, int* chunks_out,
+                                         int k) {
   SRFRD_REQUIRE(chunks_out, "catalogue_topk_plan: null output");
   const TopkCfg c = pick_cfg(D, n_split);
-  SRFRD_REQUIRE(c.ubs > 0, "catalogue_topk: D=%d with n_split=%d does not fit tensor memory", D, n_split);
+  if (int rc = check_k(c, D, n_split, k)) return rc;
   *chunks_out = make_plan(c, U, n_rows, row_lo, D).slots;
+  return 0;
+}
+
+extern "C" int srfrd_catalogue_topk_kmax(int D, int n_split, int* kmax_out) {
+  SRFRD_REQUIRE(kmax_out, "catalogue_topk_kmax: null output");
+  const TopkCfg c = pick_cfg(D, n_split);
+  SRFRD_REQUIRE(c.ubs > 0, "catalogue_topk: D=%d with n_split=%d does not fit tensor memory", D, n_split);
+  *kmax_out = topk_kmax(c, D);
   return 0;
 }
 
@@ -1101,18 +1420,19 @@ static int launch_tilemax(const CUtensorMap& tmE, TopkShape& s, int grid, cudaSt
 
 template <int MT>
 static int launch_unitmax(const CUtensorMap& tmE, TopkShape& s, int grid, cudaStream_t stream) {
-  const int b_tile = MT * KB * 2;
   const int unit = 2 * s.kblocks;                       // ring length: a multiple of 2 * kblocks (see kernel comment)
-  s.stages = ((216 * 1024) / b_tile) / unit * unit;
+  s.stages = unit_stages(MT, s.kblocks, s.k);
   SRFRD_REQUIRE(s.stages >= unit, "catalogue_topk: item tile ring does not fit shared memory");
-  const size_t smem = (size_t)s.stages * b_tile + (2 * s.stages + 32) * 8 + 1024 + 1024;
+  const size_t smem = unit_smem_bytes(MT, s.stages, s.k);
   static bool attr_set = false;
   if (!attr_set) {
     SRFRD_CUDA(cudaFuncSetAttribute(catalogue_unitmax_kernel<MT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     SRFRD_CUDA(cudaFuncSetAttribute(catalogue_unitmax_kernel<MT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    SRFRD_CUDA(cudaFuncSetAttribute(catalogue_unitmax_kernel<MT, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     attr_set = true;
   }
-  if (s.trace) catalogue_unitmax_kernel<MT, true><<<grid, 384, smem, stream>>>(tmE, s);
+  if (s.k > TK) catalogue_unitmax_kernel<MT, false, true><<<grid, 384, smem, stream>>>(tmE, s);
+  else if (s.trace) catalogue_unitmax_kernel<MT, true><<<grid, 384, smem, stream>>>(tmE, s);
   else catalogue_unitmax_kernel<MT, false><<<grid, 384, smem, stream>>>(tmE, s);
   SRFRD_LAUNCH_CHECK();
   return 0;
@@ -1120,7 +1440,7 @@ static int launch_unitmax(const CUtensorMap& tmE, TopkShape& s, int grid, cudaSt
 
 extern "C" int srfrd_catalogue_topk(const void* feats_bf16, int64_t U, int64_t u_pad, int n_split, const void* table_bf16,
                                     int64_t n_rows, int64_t row_lo, int64_t id_base, int D, int ld_feats, int ld_table,
-                                    int chunks, float* part_scores, int* part_ids, float* packed_out, void* stream_) {
+                                    int chunks, float* part_scores, int* part_ids, float* packed_out, void* stream_, int k) {
   cudaStream_t stream = (cudaStream_t)stream_;
   SRFRD_REQUIRE(feats_bf16 && table_bf16 && part_scores && part_ids, "catalogue_topk: null pointer");
   SRFRD_REQUIRE(n_split >= 1 && n_split <= 3, "catalogue_topk: n_split must be 1..3");
@@ -1129,7 +1449,8 @@ extern "C" int srfrd_catalogue_topk(const void* feats_bf16, int64_t U, int64_t u
   SRFRD_REQUIRE(U > 0 && n_rows > row_lo && row_lo >= 0, "catalogue_topk: empty problem");
   SRFRD_REQUIRE(n_rows < (1ll << 31) && id_base + n_rows < (1ll << 31), "catalogue_topk: ids must fit int32");
   const TopkCfg c = pick_cfg(D, n_split);
-  SRFRD_REQUIRE(c.ubs > 0, "catalogue_topk: D=%d with n_split=%d does not fit tensor memory", D, n_split);
+  if (int rc = check_k(c, D, n_split, k)) return rc;
+  const int L = k > TK ? k : TK;                        // list length of every buffer
   const TopkPlan pl = make_plan(c, U, n_rows, row_lo, D);
   SRFRD_REQUIRE(chunks == pl.slots, "catalogue_topk: chunks must come from srfrd_catalogue_topk_plan");
   SRFRD_REQUIRE(u_pad >= U, "catalogue_topk: u_pad < U");
@@ -1142,6 +1463,7 @@ extern "C" int srfrd_catalogue_topk(const void* feats_bf16, int64_t U, int64_t u
   s.feats = (const bf16*)feats_bf16; s.ld_feats = ld_feats;
   s.table = (const bf16*)table_bf16; s.ld_table = ld_table;
   s.out_scores = part_scores; s.out_ids = part_ids; s.packed = packed_out;
+  s.k = L;
   { const char* dbg = getenv("SRFRD_TOPK_DEBUG"); s.debug = dbg ? atoi(dbg) : 0; }
   s.trace = nullptr;
   const char* trace_path = getenv("SRFRD_TOPK_TRACE");
@@ -1151,7 +1473,7 @@ extern "C" int srfrd_catalogue_topk(const void* feats_bf16, int64_t U, int64_t u
     SRFRD_CUDA(cudaMemsetAsync(s.trace, 0, trace_bytes, stream));
   }
   // list slots a user group does not use stay empty (index -1)
-  SRFRD_CUDA(cudaMemsetAsync(part_ids, 0xFF, (size_t)U * pl.slots * TK * sizeof(int), stream));
+  SRFRD_CUDA(cudaMemsetAsync(part_ids, 0xFF, (size_t)U * pl.slots * L * sizeof(int), stream));
   CUtensorMap tmE;
   if (int rc = make_tmap_bf16_2d(&tmE, table_bf16, n_rows, D, ld_table, c.nt, KB)) return rc;
   int rc;
@@ -1181,7 +1503,18 @@ extern "C" int srfrd_catalogue_topk(const void* feats_bf16, int64_t U, int64_t u
   const char* refine_env = getenv("SRFRD_TOPK_REFINE");
   const bool fast_refine = !(refine_env && refine_env[0] == '0');
   const bool fast = fast_refine && D == 64 && n_split == 1 && ld_table == 64;
-  if (fast && c.ru == 56) catalogue_refine64_kernel<56><<<(unsigned)((U + 7) / 8), 256, 0, stream>>>(s);
+  if (k > TK) {
+    const size_t smem = KWARPS * refine_k_warp_bytes(L, c.ru);
+    static bool attr_set = false;
+    if (!attr_set) {
+      SRFRD_CUDA(cudaFuncSetAttribute(catalogue_refine_k_kernel<56>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+      SRFRD_CUDA(cudaFuncSetAttribute(catalogue_refine_k_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+      attr_set = true;
+    }
+    const unsigned blocks = (unsigned)((U + KWARPS - 1) / KWARPS);
+    if (fast && c.ru == 56) catalogue_refine_k_kernel<56><<<blocks, 32 * KWARPS, smem, stream>>>(s);
+    else catalogue_refine_k_kernel<0><<<blocks, 32 * KWARPS, smem, stream>>>(s);
+  } else if (fast && c.ru == 56) catalogue_refine64_kernel<56><<<(unsigned)((U + 7) / 8), 256, 0, stream>>>(s);
   else if (fast && c.ru == 64) catalogue_refine64_kernel<64><<<(unsigned)((U + 7) / 8), 256, 0, stream>>>(s);
   else catalogue_refine_kernel<<<(unsigned)((U + 7) / 8), 256, 0, stream>>>(s);
   SRFRD_LAUNCH_CHECK();
@@ -1191,9 +1524,13 @@ extern "C" int srfrd_catalogue_topk(const void* feats_bf16, int64_t U, int64_t u
 extern "C" int srfrd_merge_topk(const float* scores, const int* ids, int64_t U, int nlists, int k, float* out_scores,
                                 int64_t* out_ids, void* stream) {
   SRFRD_REQUIRE(scores && ids && out_scores && out_ids, "merge_topk: null pointer");
-  SRFRD_REQUIRE(k >= 1 && k <= TK, "merge_topk: k must be in 1..%d", TK);
+  SRFRD_REQUIRE(k >= 1 && k <= KMAX, "merge_topk: k must be in 1..%d", KMAX);
   if (U == 0) return 0;
-  merge_topk_kernel<<<(unsigned)((U + 127) / 128), 128, 0, (cudaStream_t)stream>>>(scores, ids, U, nlists, k, out_scores, out_ids);
+  if (k > TK)                                           // lists of k entries
+    merge_topk_k_kernel<<<(unsigned)((U + 7) / 8), 256, 0, (cudaStream_t)stream>>>(
+        scores, ids, (int64_t)nlists * k, k, U, nlists, k, out_scores, out_ids);
+  else
+    merge_topk_kernel<<<(unsigned)((U + 127) / 128), 128, 0, (cudaStream_t)stream>>>(scores, ids, U, nlists, k, out_scores, out_ids);
   SRFRD_LAUNCH_CHECK();
   return 0;
 }
@@ -1201,9 +1538,13 @@ extern "C" int srfrd_merge_topk(const float* scores, const int* ids, int64_t U, 
 extern "C" int srfrd_merge_topk_packed(const float* packed, int64_t U, int nlists, int k, float* out_scores,
                                        int64_t* out_ids, void* stream) {
   SRFRD_REQUIRE(packed && out_scores && out_ids, "merge_topk_packed: null pointer");
-  SRFRD_REQUIRE(k >= 1 && k <= TK && nlists >= 1, "merge_topk_packed: k must be in 1..%d", TK);
+  SRFRD_REQUIRE(k >= 1 && k <= KMAX && nlists >= 1, "merge_topk_packed: k must be in 1..%d", KMAX);
   if (U == 0) return 0;
-  merge_topk_packed_kernel<<<(unsigned)((U + 127) / 128), 128, 0, (cudaStream_t)stream>>>(packed, U, nlists, k, out_scores, out_ids);
+  if (k > TK)                                           // wire rows of k scores + k ids
+    merge_topk_k_kernel<<<(unsigned)((U + 7) / 8), 256, 0, (cudaStream_t)stream>>>(
+        packed, reinterpret_cast<const int*>(packed) + k, 2 * k, U * 2 * k, U, nlists, k, out_scores, out_ids);
+  else
+    merge_topk_packed_kernel<<<(unsigned)((U + 127) / 128), 128, 0, (cudaStream_t)stream>>>(packed, U, nlists, k, out_scores, out_ids);
   SRFRD_LAUNCH_CHECK();
   return 0;
 }

@@ -1,4 +1,4 @@
-"""Evaluation on the hot path: full-catalogue top-k (tcgen05 scoring fused with a streaming top-10)
+"""Evaluation on the hot path: full-catalogue top-k, 1 <= k <= 64 (tcgen05 scoring fused with a streaming top-k)
 and the reference's sampled-101 protocol (utils.py:544-602), both batched and both on the library's own kernels.
 
 Full-catalogue scoring is the reference's ``predict(user_ids, seq, rsq, label)`` called with
@@ -15,7 +15,15 @@ import torch
 from . import ops
 
 bf16 = torch.bfloat16
-TK = 10
+TK = 10          # list length of the top-10 kernels; a smaller k is the prefix of their lists
+KMAX = 64        # longest top-k (the per-row lists of the k-list kernels live in shared memory)
+
+
+def list_len(k: int) -> int:
+    """Length of every candidate list for a top-k: max(k, 10).  k outside 1..KMAX is refused before any launch."""
+    if not 1 <= int(k) <= KMAX:
+        raise RuntimeError(f"catalogue_topk: k must be in 1..{KMAX} (got {k})")
+    return max(int(k), TK)
 
 
 class CatalogueIndex:
@@ -61,60 +69,69 @@ def _split_feats(feats_f32: torch.Tensor, Dp: int, n_split: int):
     return fb, u_pad
 
 
-def _local_lists(feats_f32: torch.Tensor, index: CatalogueIndex, n_split: int, packed: Optional[torch.Tensor]):
-    """Run K8 on the local shard; returns the (U, chunks, 10) list buffers whose slot 0 holds each user's exact local
-    top-10 (sorted, global ids) and, when `packed` is given, the same list in the all-gather wire format."""
+def _local_lists(feats_f32: torch.Tensor, index: CatalogueIndex, n_split: int, packed: Optional[torch.Tensor],
+                 k: int = TK):
+    """Run K8 on the local shard; returns the (U, chunks, L) list buffers (L = max(k, 10)) whose slot 0 holds each
+    user's exact local top-L (sorted, global ids) and, when `packed` is given, the same list in the all-gather wire
+    format."""
     U = feats_f32.shape[0]
     dev = feats_f32.device
+    L = list_len(k)
+    chunks = ops.catalogue_topk_plan(U, index.n_rows, index.row_lo, index.Dp, n_split, k)   # refuses k above the limit
     fb, u_pad = _split_feats(feats_f32, index.Dp, n_split)
-    chunks = ops.catalogue_topk_plan(U, index.n_rows, index.row_lo, index.Dp, n_split)
-    ps = torch.empty(U, chunks, TK, dtype=torch.float32, device=dev)
-    pi = torch.empty(U, chunks, TK, dtype=torch.int32, device=dev)
-    ops.catalogue_topk(fb, U, u_pad, n_split, index.table, index.row_lo, index.id_base, chunks, ps, pi, packed)
+    ps = torch.empty(U, chunks, L, dtype=torch.float32, device=dev)
+    pi = torch.empty(U, chunks, L, dtype=torch.int32, device=dev)
+    ops.catalogue_topk(fb, U, u_pad, n_split, index.table, index.row_lo, index.id_base, chunks, ps, pi, packed, k=k)
     return ps, pi, chunks
 
 
-def local_topk(feats_f32: torch.Tensor, index: CatalogueIndex, n_split: int = 1):
-    """Per-user top-10 of feats (U, D) against the local shard -> (scores (U,10) fp32, ids (U,10) int64)."""
+def local_topk(feats_f32: torch.Tensor, index: CatalogueIndex, n_split: int = 1, k: int = TK):
+    """Per-user top-k of feats (U, D) against the local shard -> (scores (U,k) fp32, ids (U,k) int64); (-inf, -1) past
+    the last candidate."""
     U = feats_f32.shape[0]
     dev = feats_f32.device
+    list_len(k)
     if index.n_rows <= index.row_lo:                      # empty shard
-        return (torch.full((U, TK), float("-inf"), device=dev), torch.full((U, TK), -1, dtype=torch.int64, device=dev))
-    ps, pi, chunks = _local_lists(feats_f32, index, n_split, None)
-    out_s = torch.empty(U, TK, dtype=torch.float32, device=dev)
-    out_i = torch.empty(U, TK, dtype=torch.int64, device=dev)
-    ops.merge_topk(ps, pi, U, chunks, TK, out_s, out_i)
+        return (torch.full((U, k), float("-inf"), device=dev), torch.full((U, k), -1, dtype=torch.int64, device=dev))
+    ps, pi, chunks = _local_lists(feats_f32, index, n_split, None, k)
+    out_s = torch.empty(U, k, dtype=torch.float32, device=dev)
+    out_i = torch.empty(U, k, dtype=torch.int64, device=dev)
+    ops.merge_topk(ps, pi, U, chunks, k, out_s, out_i)
     return out_s, out_i
 
 
 def merge_shards(scores: torch.Tensor, ids: torch.Tensor, k: int = TK):
-    """scores/ids: (U, G, 10) candidate lists gathered from G shards -> global (U, k)."""
-    U, G, _ = scores.shape
+    """scores/ids: (U, G, L) candidate lists gathered from G shards, L = max(k, 10), each sorted as local_topk returns
+    them -> global (U, k)."""
+    U, G, W = scores.shape
+    if W != list_len(k):
+        raise ValueError(f"merge_shards: top-{k} needs lists of {list_len(k)} entries, got {W}")
     out_s = torch.empty(U, k, dtype=torch.float32, device=scores.device)
     out_i = torch.empty(U, k, dtype=torch.int64, device=scores.device)
     ops.merge_topk(scores.contiguous(), ids.to(torch.int32).contiguous(), U, G, k, out_s, out_i)
     return out_s, out_i
 
 
-def sharded_topk(feats_f32: torch.Tensor, index: CatalogueIndex, process_group=None, n_split: int = 1):
-    """Row-sharded catalogue scoring: local top-10, ONE all-gather of the packed lists (10 fp32 scores + 10 int32 global
-    ids = 80 B / user / rank, written in wire format by the scoring kernel itself), merge straight out of the gathered
-    buffer -> identical (U, 10) on every rank.  No int64 on the wire, no permute / contiguous copies."""
+def sharded_topk(feats_f32: torch.Tensor, index: CatalogueIndex, process_group=None, n_split: int = 1, k: int = TK):
+    """Row-sharded catalogue scoring: local top-k, ONE all-gather of the packed lists (L fp32 scores + L int32 global
+    ids, L = max(k, 10): 8L B / user / rank, written in wire format by the scoring kernel itself), merge straight out of
+    the gathered buffer -> identical (U, k) on every rank.  No int64 on the wire, no permute / contiguous copies."""
     from . import parallel
     if process_group is None or torch.distributed.get_world_size(process_group) == 1:
-        return local_topk(feats_f32, index, n_split)
+        return local_topk(feats_f32, index, n_split, k)
     G = torch.distributed.get_world_size(process_group)
     U = feats_f32.shape[0]
     dev = feats_f32.device
-    packed = torch.empty(U, 2 * TK, dtype=torch.float32, device=dev)
+    L = list_len(k)
+    packed = torch.empty(U, 2 * L, dtype=torch.float32, device=dev)
     if index.n_rows <= index.row_lo:                      # empty shard: ids -1 (bit pattern of int32 -1 in every id word)
         packed.view(torch.int32).fill_(-1)
     else:
-        _local_lists(feats_f32, index, n_split, packed)
-    gathered = parallel.allgather_packed_topk(packed, process_group)        # (G, U, 20)
-    out_s = torch.empty(U, TK, dtype=torch.float32, device=dev)
-    out_i = torch.empty(U, TK, dtype=torch.int64, device=dev)
-    ops.merge_topk_packed(gathered, U, G, TK, out_s, out_i)
+        _local_lists(feats_f32, index, n_split, packed, k)
+    gathered = parallel.allgather_packed_topk(packed, process_group)        # (G, U, 2L)
+    out_s = torch.empty(U, k, dtype=torch.float32, device=dev)
+    out_i = torch.empty(U, k, dtype=torch.int64, device=dev)
+    ops.merge_topk_packed(gathered, U, G, k, out_s, out_i)
     return out_s, out_i
 
 
@@ -144,7 +161,10 @@ def encode_users(model, seq, rsq, process_group=None) -> torch.Tensor:
 
 def hr_ndcg_from_topk(topk_ids: torch.Tensor, target: torch.Tensor, k: int = 10) -> Tuple[float, float]:
     """(NDCG@k, HR@k) in the reference's return order (utils.py:595-602): a hit at 0-based rank r < k adds
-    1 to HT and 1/log2(r+2) to NDCG; means over users.  Reads k ids per user back to the host."""
+    1 to HT and 1/log2(r+2) to NDCG; means over users.  Reads k ids per user back to the host.  k may not exceed the
+    width of topk_ids (a narrower list cannot tell a miss from a hit at a rank it does not hold)."""
+    if k > topk_ids.shape[1]:
+        raise ValueError(f"hr_ndcg_from_topk: k={k} exceeds the {topk_ids.shape[1]} ids per user given")
     ids = topk_ids[:, :k].cpu().numpy()
     tgt = np.asarray(target.cpu() if torch.is_tensor(target) else target).reshape(-1, 1)
     hit = ids == tgt
@@ -157,18 +177,19 @@ def hr_ndcg_from_topk(topk_ids: torch.Tensor, target: torch.Tensor, k: int = 10)
 
 @torch.no_grad()
 def evaluate_full_catalogue(model, seq, rsq, target, batch_users: int = 16384, n_split: int = 1, process_group=None,
-                            index: Optional[CatalogueIndex] = None):
-    """Encode users, score the whole catalogue, return (NDCG@10, HR@10, topk_ids)."""
+                            index: Optional[CatalogueIndex] = None, k: int = TK):
+    """Encode users, score the whole catalogue, return (NDCG@k, HR@k, topk_ids (U, k)); 1 <= k <= KMAX."""
+    list_len(k)
     eng = model._sync_flat()
     if index is None:
         index = CatalogueIndex(eng.P.view(model.spec.item_key), 0)
     outs = []
     for s in range(0, seq.shape[0], batch_users):
         feats = encode_users(model, seq[s:s + batch_users], None if rsq is None else rsq[s:s + batch_users], process_group)
-        _, ids = sharded_topk(feats[:, :model.spec.D], index, process_group, n_split)
+        _, ids = sharded_topk(feats[:, :model.spec.D], index, process_group, n_split, k)
         outs.append(ids)
     ids = torch.cat(outs)
-    ndcg, hr = hr_ndcg_from_topk(ids, target)
+    ndcg, hr = hr_ndcg_from_topk(ids, target, k)
     return ndcg, hr, ids
 
 

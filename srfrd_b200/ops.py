@@ -252,18 +252,27 @@ def _l2_args(l2: Optional[ParamL2]):
     return (None, 0, None, None) if l2 is None else (_p(l2.seg), l2.n_seg, _p(l2.coef), _p(l2.reg))
 
 
-def catalogue_topk_plan(U, n_rows, row_lo, D, n_split) -> int:
+def catalogue_topk_plan(U, n_rows, row_lo, D, n_split, k=10) -> int:
+    """Chunk count of the (U, chunks, max(k, 10)) list buffers; raises if k is outside 1..catalogue_topk_kmax(D, n_split)."""
     out = C.c_int(0)
-    call("srfrd_catalogue_topk_plan", U, n_rows, row_lo, D, n_split, C.byref(out))
+    call("srfrd_catalogue_topk_plan", U, n_rows, row_lo, D, n_split, C.byref(out), int(k))
     return out.value
 
 
-def catalogue_topk(feats, U, u_pad, n_split, table, row_lo, id_base, chunks, part_scores, part_ids, packed=None):
-    """packed: optional (U, 20) fp32 -- each user's final local list as 10 scores + 10 int32 ids (all-gather send buffer)."""
+def catalogue_topk_kmax(D, n_split) -> int:
+    """Largest k catalogue_topk serves for this table width and split (host arithmetic, no launch)."""
+    out = C.c_int(0)
+    call("srfrd_catalogue_topk_kmax", D, n_split, C.byref(out))
+    return out.value
+
+
+def catalogue_topk(feats, U, u_pad, n_split, table, row_lo, id_base, chunks, part_scores, part_ids, packed=None, k=10):
+    """part_scores / part_ids: (U, chunks, L) with L = max(k, 10).  packed: optional (U, 2L) fp32 -- each user's final
+    local list as L scores + L int32 ids (all-gather send buffer)."""
     _lib.require_device()
     D = table.shape[1]
     call("srfrd_catalogue_topk", _p(feats), U, u_pad, n_split, _p(table), table.shape[0], row_lo, id_base, D,
-         feats.stride(0), table.stride(0), chunks, _p(part_scores), _p(part_ids), _p(packed), _stream())
+         feats.stride(0), table.stride(0), chunks, _p(part_scores), _p(part_ids), _p(packed), _stream(), int(k))
 
 
 def merge_topk_packed(packed, U, nlists, k, out_scores, out_ids):

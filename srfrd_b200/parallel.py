@@ -8,7 +8,7 @@ FusedTrainer implements exactly this on the device (two tiny all-reduces for W a
 gradient buffer).
 
 Catalogue scoring: the (N+1)-row item table is row-sharded, every rank scores all users against its rows, and the
-per-rank top-10 lists (80 B per user) are all-gathered and merged with the tie-break (score desc, id asc).
+per-rank top-k lists (8 max(k, 10) B per user) are all-gathered and merged with the tie-break (score desc, id asc).
 """
 from __future__ import annotations
 
@@ -46,8 +46,8 @@ def broadcast_parameters(flat_params: torch.Tensor, src: int = 0, group=None) ->
 
 
 def allgather_packed_topk(packed: torch.Tensor, group=None) -> torch.Tensor:
-    """(U, 20) per rank (10 fp32 scores + 10 int32 ids per user, the scoring kernel's wire format) -> (G, U, 20) on
-    every rank with ONE all-gather."""
+    """(U, 2L) per rank (L fp32 scores + L int32 ids per user, L = max(k, 10): the scoring kernel's wire format)
+    -> (G, U, 2L) on every rank with ONE all-gather."""
     G = dist.get_world_size(group)
     U, W = packed.shape
     out = torch.empty(G * U, W, dtype=packed.dtype, device=packed.device)      # (G * U, W): rank-major concatenation
@@ -65,7 +65,8 @@ def allgather_rows(rows: torch.Tensor, group=None) -> torch.Tensor:
 
 
 def merge_packed_topk_host(gathered: torch.Tensor, k: int = 10):
-    """Host restatement of srfrd_merge_topk_packed (tie-break: score desc, id asc) for the CPU protocol tests."""
+    """Host restatement of srfrd_merge_topk_packed (tie-break: score desc, id asc) for the CPU protocol tests.
+    gathered: (G, U, 2L) wire rows of any list length L; returns the best k of the G * L entries per user."""
     import numpy as np
     g = gathered.cpu().numpy()
     G, U, W = g.shape

@@ -1,6 +1,7 @@
 """Multi-GPU check (run under torchrun): G-rank data-parallel FusedTrainer == 1-rank on the concatenated batch,
 and row-sharded catalogue top-10 (NCCL all-gather + merge) == unsharded top-10.
-`--l2 X` trains both with l2_emb = X (the regulariser's gradient is added once, after the reduction over ranks)."""
+`--l2 X` trains both with l2_emb = X (the regulariser's gradient is added once, after the reduction over ranks).
+`--topk-k K` checks the sharded top-K (1 <= K <= 64) instead of the top-10."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -31,6 +32,7 @@ m_dp, m_one = make_model(), make_model()
 P.broadcast_parameters(m_dp.flat_parameters().data, 0)
 use_graph = os.environ.get("DP_CHECK_GRAPH", "0") == "1"
 l2_emb = float(sys.argv[sys.argv.index("--l2") + 1]) if "--l2" in sys.argv else 0.0
+topk_k = int(sys.argv[sys.argv.index("--topk-k") + 1]) if "--topk-k" in sys.argv else 10
 tr_dp = FusedTrainer(m_dp, process_group=dist.group.WORLD, use_graph=use_graph, l2_emb=l2_emb)
 if rank == 0:
     print("fused reduce-scatter/Adam/all-gather kernel:", tr_dp._dp is not None, "graph:", use_graph, "l2_emb:", l2_emb)
@@ -61,19 +63,19 @@ if rank == 0:
     print("replicas bit-identical:", bool(torch.equal(mine, other)))
 cos = float(torch.dot(a - 0, b - 0) / (a.norm() * b.norm()))
 ok &= drift < 5e-3
-# sharded catalogue top-10
+# sharded catalogue top-k
 g = torch.Generator().manual_seed(3)
 feats = (torch.randint(-16, 17, (500, 64), generator=g).float() / 8).to(dev)
 table = (torch.randint(-16, 17, (20001, 64), generator=g).float() / 8).to(dev)
-_, ref = EV.local_topk(feats, EV.CatalogueIndex(table, 0), 1)
+ref_s, ref = EV.local_topk(feats, EV.CatalogueIndex(table, 0), 1, topk_k)
 lo, hi = EV.CatalogueIndex.shard_bounds(table.shape[0], rank, world)
-_, ids = EV.sharded_topk(feats, EV.CatalogueIndex(table[lo:hi], lo), dist.group.WORLD, 1)
-same = bool(torch.equal(ids, ref))
+got_s, ids = EV.sharded_topk(feats, EV.CatalogueIndex(table[lo:hi], lo), dist.group.WORLD, 1, topk_k)
+same = bool(torch.equal(ids, ref)) and bool(torch.equal(got_s, ref_s))
 ok &= same
 flag = torch.tensor([1.0 if ok else 0.0], device=dev)
 dist.all_reduce(flag, op=dist.ReduceOp.MIN)
 if rank == 0:
-    print(f"param drift after 6 steps {drift:.2e}; sharded top-10 == unsharded: {same}; ALL OK: {bool(flag.item())}")
+    print(f"param drift after 6 steps {drift:.2e}; sharded top-{topk_k} == unsharded: {same}; ALL OK: {bool(flag.item())}")
 # (no destroy_process_group(): with NCCL work captured in live CUDA graphs the communicator teardown can block for minutes)
 rc = 0 if flag.item() else 1
 torch.cuda.synchronize()
