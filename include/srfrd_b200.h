@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define SRFRD_ABI_VERSION 8
+#define SRFRD_ABI_VERSION 9
 #if defined(__GNUC__)
 #define SRFRD_API __attribute__((visibility("default")))
 #else
@@ -241,6 +241,21 @@ SRFRD_API int srfrd_merge_topk(const float* scores, const int* ids, int64_t U, i
  * global top-k, identical on every rank. */
 SRFRD_API int srfrd_merge_topk_packed(const float* packed, int64_t U, int nlists, int k, float* out_scores,
                             int64_t* out_ids, void* stream);
+/* K8 rank form: exact full-catalogue rank of each user's held-out item (the reference's evaluation protocol,
+ * utils.py:589-591, with every item as a candidate).  rank_out[u] (int32, zeroed by the call) receives the number of
+ * local rows r in [row_lo, n_rows), global id i = id_base + r, i != target_ids[u], with score(u, i) > score(u, t) or
+ * score(u, i) == score(u, t) and i < t.  Item scores are the streaming kernel's tensor-core scores (same operands and
+ * splits as srfrd_catalogue_topk); score(u, t) is computed with SIMT fmaf from target_rows_bf16 (U rows of D bf16,
+ * leading dimension ld_target: the target's row, passed in because under row sharding it usually lives on another
+ * rank) in the order of the top-k re-scoring, and written to target_scores (nullable, fp32 (U,)).  The target is
+ * excluded by id, never by score.  Row shards' counts add up to the global rank (one integer all-reduce).  Only the unit
+ * form serves ranks (n_split * D <= 256); the tile form is refused before any launch.  Shape, alignment and null checks
+ * as srfrd_catalogue_topk. */
+SRFRD_API int srfrd_catalogue_rank(const void* feats_bf16, int64_t U, int64_t u_pad, int n_split,
+                                   const void* table_bf16, int64_t n_rows, int64_t row_lo, int64_t id_base,
+                                   int D, int ld_feats, int ld_table,
+                                   const void* target_rows_bf16, int ld_target, const int64_t* target_ids,
+                                   float* target_scores, int* rank_out, void* stream);
 
 /* ---- on-device batch sampler (next row 8f #1) ----
  * replaces: WarpSampler_fr / sample_function_fr (utils.py:14-90) and the seven LongTensor.to(device) copies per

@@ -22,6 +22,8 @@
 // k <= 10 runs these top-10 kernels (a smaller k is the prefix of their lists).  10 < k <= KMAX runs compile-time k-list
 // variants (catalogue_unitmax_kernel<.., KLIST = true>, catalogue_refine_k_kernel, merge_topk_k_kernel) with lists of k
 // entries everywhere; only the unit form serves them, and the host plan refuses a k whose lists do not fit (topk_kmax).
+// srfrd_catalogue_rank runs the unit form's rank variant (catalogue_unitmax_kernel<.., RANK = true>): no lists, each row
+// counts the items ahead of its held-out item, one phase.
 #include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -61,6 +63,11 @@ struct TopkShape {
   int k;                  // list length of the k-list kernels (11 .. KMAX); the TK kernels never read it.  Every list
                           // buffer above is then k entries long instead of TK (last field: the TK kernels' parameter
                           // offsets are unchanged)
+  // rank variant (catalogue_unitmax_kernel<.., RANK = true>) only; the list kernels never read these
+  const bf16* target_rows; int ld_target;   // (U, D) bf16 row of each user's held-out item
+  const int64_t* target_ids;                // (U,) global id of that item
+  float* target_scores;                     // optional (U,): its SIMT score, written by the piece that holds tile 0
+  int* rank_out;                            // (U,) items ahead of the target, summed over pieces with atomicAdd
 };
 
 // D[tmem] (+)= A[tmem] * B[smem]
@@ -413,7 +420,43 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
 // highest unit, which the order (max desc, unit asc) ranks last) and rescans the k entries for the new worst -- no shifts,
 // no dependent chain.  The strict v > thr test stays: units reach a thread in increasing index order, so an equal maximum
 // never displaces an earlier unit.  The proof above holds with TK replaced by k.  Everything else is the same code.
-template <int MT, bool TRACE, bool KLIST = false>
+//
+// RANK: the rank variant (srfrd_catalogue_rank).  No list: each row counts the items ahead of its held-out item t,
+// score > score(t) or score == score(t) at a lower id, t itself excluded BY ID.  At the start of a piece a thread computes
+// score(t) with SIMT arithmetic (target_score: catalogue_refine_kernel's loop) next to staging its user row; per unit,
+// after the accumulator has been handed back, the unit's maximum decides: below score(t), nothing in the unit counts;
+// otherwise the unit's columns are counted against one threshold (a unit entirely below t's id counts x >= score(t),
+// i.e. x > the next float down; one entirely above counts x > score(t)) and the unit that holds t's id is corrected
+// column by column.  At the end of the piece the row's count goes into rank_out with one integer atomicAdd (pieces of
+// the same user group, and row shards launched one after another, add up exactly in any order).  The ring, barriers,
+// refill and plan are those of the top-10 form.
+//
+// SIMT score of a (user row, item row) pair in catalogue_refine_kernel's order: per split, fmaf over the features in
+// order, then the splits summed.
+__device__ __forceinline__ float target_score(const bf16* feats, size_t split_stride, const bf16* item, int D,
+                                              int n_split) {
+  const uint4* e = reinterpret_cast<const uint4*>(item);
+  float acc = 0.f;
+  for (int sp = 0; sp < n_split; ++sp) {
+    const uint4* f = reinterpret_cast<const uint4*>(feats + sp * split_stride);
+    float a = 0.f;
+    for (int c = 0; c < D / 8; ++c) {
+      const uint4 fv = __ldg(f + c), ev = __ldg(e + c);
+      const uint32_t fw[4] = {fv.x, fv.y, fv.z, fv.w}, ew[4] = {ev.x, ev.y, ev.z, ev.w};
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        const float2 x = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&fw[q]));
+        const float2 y = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&ew[q]));
+        a = fmaf(x.x, y.x, a);
+        a = fmaf(x.y, y.y, a);
+      }
+    }
+    acc += a;
+  }
+  return acc;
+}
+
+template <int MT, bool TRACE, bool KLIST = false, bool RANK = false>
 __global__ void __launch_bounds__(384, 1)
 catalogue_unitmax_kernel(const __grid_constant__ CUtensorMap tmE, TopkShape s) {
   constexpr int UBS = 2, NEPI = 8, NACC = 4;
@@ -570,7 +613,18 @@ catalogue_unitmax_kernel(const __grid_constant__ CUtensorMap tmE, TopkShape s) {
         __syncwarp();
         if (lane == 0) mbar_arrive(afull);
       }
-      constexpr int TKR = KLIST ? 1 : TK;               // register list (unused by the k-list variant)
+      float tsc = INFINITY, tsc_dn = INFINITY;          // rank variant: the target's score and the next float below it
+      int tid = -1, rcount = 0;                         //   (+inf for rows past U: nothing counts), its id, the count
+      if constexpr (RANK) {
+        if (urow < s.U) {                               // the MMAs of the piece are already running
+          tid = (int)s.target_ids[urow];
+          tsc = target_score(s.feats + (size_t)urow * s.ld_feats, (size_t)s.u_pad * s.ld_feats,
+                             s.target_rows + (size_t)urow * s.ld_target, s.D, s.n_split);
+          tsc_dn = nextafterf(tsc, -INFINITY);
+          if (t0 == 0 && s.target_scores) s.target_scores[urow] = tsc;   // one piece per user group holds tile 0
+        }
+      }
+      constexpr int TKR = (KLIST || RANK) ? 1 : TK;     // register list (unused by the k-list and rank variants)
       float ts[TKR]; int ti[TKR];                       // this row's TK best (unit maximum, unit index), sorted
 #pragma unroll
       for (int r = 0; r < TKR; ++r) { ts[r] = -INFINITY; ti[r] = -1; }
@@ -640,6 +694,31 @@ catalogue_unitmax_kernel(const __grid_constant__ CUtensorMap tmE, TopkShape s) {
         }
         return fmaxf(fmaxf(m[0], m[1]), fmaxf(m[2], m[3]));
       };
+      // rank variant: items of one unit (columns already masked by reduce_half) ahead of the target; g0 = id of column 0
+      auto count_half = [&](const uint32_t (&r0)[32], const uint32_t (&r1)[16], const uint32_t (&r2)[8], float m,
+                            int g0) {
+        auto col = [&](int j) {                         // j is a compile-time constant in the unrolled loops below
+          return __uint_as_float(j < 32 ? r0[j] : (j < 32 + ((HALF - 32) & 16) ? r1[j - 32] : r2[j - 32 - ((HALF - 32) & 16)]));
+        };
+        int n = 0;
+        if (m >= tsc) {                                 // else no item of the unit reaches the target's score
+          const int p = tid - g0;                       // the target's column (outside 0 .. HALF - 1: another unit)
+          const float thr = p >= HALF ? tsc_dn : tsc;   // all ids below the target's: ties count too
+          int c[4] = {0, 0, 0, 0};
+#pragma unroll
+          for (int j = 0; j < HALF; ++j) c[j & 3] += col(j) > thr ? 1 : 0;
+          n = (c[0] + c[1]) + (c[2] + c[3]);
+          if (p >= 0 && p < HALF) {                     // the target's own unit: ties below its id count, it does not
+#pragma unroll
+            for (int j = 0; j < HALF; ++j) {
+              const float x = col(j);
+              n += (j < p && x == tsc) ? 1 : 0;
+              n -= (j == p && x > tsc) ? 1 : 0;
+            }
+          }
+        }
+        return n;
+      };
       bool ready = false;                               // this unit's tfull was already seen complete (tested a unit ahead)
       for (int t = t0; t < t1; ++t, ++n) {
         const int odd = n & 1, w = ub + 2 * odd;
@@ -675,13 +754,21 @@ catalogue_unitmax_kernel(const __grid_constant__ CUtensorMap tmE, TopkShape s) {
           ready = t + 1 < t1 && mbar_try_wait(&tfull[ub + 2 * (odd ^ 1)], odd ? tph0 : tph1);
           mA = reduce_half(a0, a1, a2, valid);
           mB = reduce_half(b0, b1, b2, valid - HALF);
+          if constexpr (RANK) {
+            const int g0 = (int)(s.id_base + s.row_lo + t * MT);
+            rcount += count_half(a0, a1, a2, mA, g0) + count_half(b0, b1, b2, mB, g0 + HALF);
+          }
         }
         if (tr) trq[7] = clock64();
-        offer(mA, 2 * t);
-        offer(mB, 2 * t + 1);
+        if constexpr (!RANK) {
+          offer(mA, 2 * t);
+          offer(mB, 2 * t + 1);
+        }
         if (tr) trq[8] = clock64();
       }
-      if constexpr (KLIST) {
+      if constexpr (RANK) {
+        if (urow < s.U && rcount) atomicAdd(&s.rank_out[urow], rcount);
+      } else if constexpr (KLIST) {
         if (urow < s.U) {
           const size_t o = ((size_t)urow * s.slots + piece * 2) * s.k;  // unsorted; phase 2 selects from it
           for (int r = 0; r < s.k; ++r) {
@@ -1519,6 +1606,60 @@ extern "C" int srfrd_catalogue_topk(const void* feats_bf16, int64_t U, int64_t u
   else catalogue_refine_kernel<<<(unsigned)((U + 7) / 8), 256, 0, stream>>>(s);
   SRFRD_LAUNCH_CHECK();
   return 0;
+}
+
+template <int MT>
+static int launch_unitrank(const CUtensorMap& tmE, TopkShape& s, int grid, cudaStream_t stream) {
+  s.stages = unit_stages(MT, s.kblocks, TK);            // no lists: the top-10 form's full ring
+  SRFRD_REQUIRE(s.stages >= 2 * s.kblocks, "catalogue_rank: item tile ring does not fit shared memory");
+  const size_t smem = unit_smem_bytes(MT, s.stages, TK);
+  static bool attr_set = false;
+  if (!attr_set) {
+    SRFRD_CUDA(cudaFuncSetAttribute(catalogue_unitmax_kernel<MT, false, false, true>,
+                                    cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    attr_set = true;
+  }
+  catalogue_unitmax_kernel<MT, false, false, true><<<grid, 384, smem, stream>>>(tmE, s);
+  SRFRD_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int srfrd_catalogue_rank(const void* feats_bf16, int64_t U, int64_t u_pad, int n_split, const void* table_bf16,
+                                    int64_t n_rows, int64_t row_lo, int64_t id_base, int D, int ld_feats, int ld_table,
+                                    const void* target_rows_bf16, int ld_target, const int64_t* target_ids,
+                                    float* target_scores, int* rank_out, void* stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  SRFRD_REQUIRE(feats_bf16 && table_bf16 && target_rows_bf16 && target_ids && rank_out, "catalogue_rank: null pointer");
+  SRFRD_REQUIRE(n_split >= 1 && n_split <= 3, "catalogue_rank: n_split must be 1..3");
+  SRFRD_REQUIRE(D % 16 == 0 && ld_feats % 8 == 0 && ld_table % 8 == 0 && ld_target % 8 == 0 && ld_target >= D,
+                "catalogue_rank: D %% 16 and ld %% 8 required (D=%d)", D);
+  SRFRD_REQUIRE(((uintptr_t)feats_bf16 & 15) == 0 && ((uintptr_t)table_bf16 & 15) == 0 &&
+                ((uintptr_t)target_rows_bf16 & 15) == 0, "catalogue_rank: operands must be 16-byte aligned");
+  SRFRD_REQUIRE(U > 0 && n_rows > row_lo && row_lo >= 0, "catalogue_rank: empty problem");
+  SRFRD_REQUIRE(n_rows < (1ll << 31) && id_base + n_rows < (1ll << 31), "catalogue_rank: ids must fit int32");
+  SRFRD_REQUIRE(u_pad >= U, "catalogue_rank: u_pad < U");
+  const TopkCfg c = pick_cfg(D, n_split);
+  SRFRD_REQUIRE(c.ubs > 0 && c.nacc == 4, "catalogue_rank: needs the unit form (n_split * D <= 256); D=%d with n_split=%d "
+                "runs the tile form", D, n_split);
+  const TopkPlan pl = make_plan(c, U, n_rows, row_lo, D);
+  TopkShape s = {};
+  s.U = (int)U; s.D = D; s.n_split = n_split; s.u_pad = (int)u_pad;
+  s.row_lo = (int)row_lo; s.row_hi = (int)n_rows; s.id_base = id_base;
+  s.kblocks = (D + KB - 1) / KB;
+  s.nt = c.ru;
+  s.tiles_total = pl.tiles_total; s.ugroups = pl.ugroups; s.share = pl.share; s.slots = pl.slots;
+  s.feats = (const bf16*)feats_bf16; s.ld_feats = ld_feats;
+  s.table = (const bf16*)table_bf16; s.ld_table = ld_table;
+  s.k = TK;
+  s.target_rows = (const bf16*)target_rows_bf16; s.ld_target = ld_target;
+  s.target_ids = target_ids; s.target_scores = target_scores; s.rank_out = rank_out;
+  SRFRD_CUDA(cudaMemsetAsync(rank_out, 0, (size_t)U * sizeof(int), stream));
+  CUtensorMap tmE;
+  if (int rc = make_tmap_bf16_2d(&tmE, table_bf16, n_rows, D, ld_table, c.nt, KB)) return rc;
+  if (c.nt == 112) return launch_unitrank<112>(tmE, s, pl.grid, stream);
+  if (c.nt == 96) return launch_unitrank<96>(tmE, s, pl.grid, stream);
+  if (c.nt == 80) return launch_unitrank<80>(tmE, s, pl.grid, stream);
+  return launch_unitrank<64>(tmE, s, pl.grid, stream);
 }
 
 extern "C" int srfrd_merge_topk(const float* scores, const int* ids, int64_t U, int nlists, int k, float* out_scores,

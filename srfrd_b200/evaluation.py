@@ -1,5 +1,6 @@
-"""Evaluation on the hot path: full-catalogue top-k, 1 <= k <= 64 (tcgen05 scoring fused with a streaming top-k)
-and the reference's sampled-101 protocol (utils.py:544-602), both batched and both on the library's own kernels.
+"""Evaluation on the hot path: full-catalogue top-k, 1 <= k <= 64 (tcgen05 scoring fused with a streaming top-k), the
+exact full-catalogue rank of each user's held-out item (HR@k / NDCG@k at any cutoff, MRR) and the reference's sampled-101
+protocol (utils.py:544-602), all batched and all on the library's own kernels.
 
 Full-catalogue scoring is the reference's ``predict(user_ids, seq, rsq, label)`` called with
 ``label = arange(1, itemnum + 1)`` followed by ``(-logits).argsort().argsort()`` (utils.py:589-591),
@@ -135,6 +136,63 @@ def sharded_topk(feats_f32: torch.Tensor, index: CatalogueIndex, process_group=N
     return out_s, out_i
 
 
+UNIT_FORM_MAX = 256   # largest n_split * D the unit-form scoring kernel serves; only that form computes ranks
+
+
+def _targets(target, U: int, N: int, device) -> torch.Tensor:
+    """(U,) int64 item ids on `device`; ValueError unless there are U of them, each in 1..N."""
+    t = torch.as_tensor(target).reshape(-1)
+    if t.numel() != U:
+        raise ValueError(f"catalogue_ranks: {t.numel()} targets for {U} users")
+    t = t.to(device=device, dtype=torch.int64)
+    if U and (int(t.min()) < 1 or int(t.max()) > N):
+        raise ValueError(f"catalogue_ranks: targets must be item ids in 1..{N} (got {int(t.min())}..{int(t.max())})")
+    return t
+
+
+def catalogue_ranks(feats_f32: torch.Tensor, index: CatalogueIndex, table_f32: torch.Tensor, target,
+                    process_group=None, n_split: int = 1) -> torch.Tensor:
+    """Exact full-catalogue rank of each user's held-out item -> int64 (U,): the number of items 1..N ahead of target[u]
+    under (score desc, id asc), i.e. the reference's (-logits).argsort().argsort()[0] (utils.py:589-591) with every item
+    a candidate.  Scores as local_topk ranks them (bf16 operands, fp32 accumulation, n_split feature splits).
+
+    index     : the local (shard of the) table the count runs over; an empty shard contributes 0 without a launch
+    table_f32 : the full (N+1, D) fp32 item table, replicated like the model parameters: the targets' rows are gathered
+                from it with the conversion CatalogueIndex uses, so every rank scores the target with the same bits
+    With a process group the per-shard counts are summed by ONE int32 all-reduce (4 B per user)."""
+    from . import parallel
+    U = feats_f32.shape[0]
+    dev = feats_f32.device
+    if table_f32.shape[1] != index.D:
+        raise ValueError(f"catalogue_ranks: table width {table_f32.shape[1]} != index width {index.D}")
+    tgt = _targets(target, U, table_f32.shape[0] - 1, dev)
+    if n_split * index.Dp > UNIT_FORM_MAX:
+        raise RuntimeError(f"catalogue_rank: needs the unit form (n_split * D <= {UNIT_FORM_MAX}); D={index.Dp} with "
+                           f"n_split={n_split} runs the tile form")
+    rank = torch.zeros(U, dtype=torch.int32, device=dev)
+    if U and index.n_rows > index.row_lo:
+        rows = torch.zeros(U, index.Dp, dtype=bf16, device=dev)
+        ops.f32_to_bf16_split(table_f32.contiguous(), rows[:, :index.D], None, row_index=tgt)
+        fb, u_pad = _split_feats(feats_f32, index.Dp, n_split)
+        ops.catalogue_rank(fb, U, u_pad, n_split, index.table, index.row_lo, index.id_base, rows, tgt, rank)
+    parallel.allreduce_sum_(rank, process_group)
+    return rank.to(torch.int64)
+
+
+def metrics_from_ranks(ranks, ks=(10,)) -> dict:
+    """HR@k = mean(rank < k), NDCG@k = mean(1 / log2(rank + 2) where rank < k) for every k in ks, and MRR =
+    mean(1 / (rank + 1)), from 0-based ranks (utils.py:595-597 generalised to any cutoff)."""
+    r = np.asarray(ranks.cpu() if torch.is_tensor(ranks) else ranks, dtype=np.int64).reshape(-1)
+    n = max(len(r), 1)
+    out = {}
+    for k in ks:
+        hit = r < k
+        out[f"HR@{k}"] = float(hit.sum() / n)
+        out[f"NDCG@{k}"] = float(np.where(hit, 1.0 / np.log2(r + 2.0), 0.0).sum() / n)
+    out["MRR"] = float((1.0 / (r + 1.0)).sum() / n)
+    return out
+
+
 @torch.no_grad()
 def encode_users(model, seq, rsq, process_group=None) -> torch.Tensor:
     """hidden[:, -1, :] for every user (U, Dout) fp32.  With a process group the USERS are split over the ranks (a sequence's
@@ -191,6 +249,28 @@ def evaluate_full_catalogue(model, seq, rsq, target, batch_users: int = 16384, n
     ids = torch.cat(outs)
     ndcg, hr = hr_ndcg_from_topk(ids, target, k)
     return ndcg, hr, ids
+
+
+@torch.no_grad()
+def evaluate_full_catalogue_ranks(model, seq, rsq, target, ks=(10,), batch_users: int = 16384, n_split: int = 1,
+                                  process_group=None, index: Optional[CatalogueIndex] = None):
+    """Encode users, rank each held-out item among the whole catalogue -> (metrics_from_ranks(ranks, ks), ranks int64
+    (U,)).  Any cutoff and MRR.  Without `index`, the rank's row shard of the item table (the whole table on one GPU)."""
+    eng = model._sync_flat()
+    table = eng.P.view(model.spec.item_key)
+    U = seq.shape[0]
+    tgt = _targets(target, U, table.shape[0] - 1, "cpu")
+    if index is None:
+        G = 1 if process_group is None else torch.distributed.get_world_size(process_group)
+        r = 0 if G == 1 else torch.distributed.get_rank(process_group)
+        lo, hi = CatalogueIndex.shard_bounds(table.shape[0], r, G)
+        index = CatalogueIndex(table[lo:hi], lo)
+    outs = []
+    for s in range(0, U, batch_users):
+        feats = encode_users(model, seq[s:s + batch_users], None if rsq is None else rsq[s:s + batch_users], process_group)
+        outs.append(catalogue_ranks(feats[:, :model.spec.D], index, table, tgt[s:s + batch_users], process_group, n_split))
+    ranks = torch.cat(outs) if outs else torch.zeros(0, dtype=torch.int64)
+    return metrics_from_ranks(ranks, ks), ranks
 
 
 def dataset_to_csr(dataset):

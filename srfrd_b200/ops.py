@@ -275,6 +275,18 @@ def catalogue_topk(feats, U, u_pad, n_split, table, row_lo, id_base, chunks, par
          feats.stride(0), table.stride(0), chunks, _p(part_scores), _p(part_ids), _p(packed), _stream(), int(k))
 
 
+def catalogue_rank(feats, U, u_pad, n_split, table, row_lo, id_base, target_rows, target_ids, rank_out,
+                   target_scores=None):
+    """rank_out (U,) int32 <- items of table rows [row_lo, n_rows) (global id id_base + row) ahead of each user's target
+    under (score desc, id asc).  target_rows: (U, D) bf16 rows of the targets; target_ids: (U,) int64 global ids;
+    target_scores: optional (U,) fp32 output of the targets' own scores."""
+    _lib.require_device()
+    D = table.shape[1]
+    call("srfrd_catalogue_rank", _p(feats), U, u_pad, n_split, _p(table), table.shape[0], row_lo, id_base, D,
+         feats.stride(0), table.stride(0), _p(target_rows), target_rows.stride(0), _p(target_ids), _p(target_scores),
+         _p(rank_out), _stream())
+
+
 def merge_topk_packed(packed, U, nlists, k, out_scores, out_ids):
     _lib.require_device()
     call("srfrd_merge_topk_packed", _p(packed), U, nlists, k, _p(out_scores), _p(out_ids), _stream())
