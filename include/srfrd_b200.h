@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define SRFRD_ABI_VERSION 9
+#define SRFRD_ABI_VERSION 10
 #if defined(__GNUC__)
 #define SRFRD_API __attribute__((visibility("default")))
 #else
@@ -256,6 +256,33 @@ SRFRD_API int srfrd_catalogue_rank(const void* feats_bf16, int64_t U, int64_t u_
                                    int D, int ld_feats, int ld_table,
                                    const void* target_rows_bf16, int ld_target, const int64_t* target_ids,
                                    float* target_scores, int* rank_out, void* stream);
+
+/* ---- full-catalogue softmax cross-entropy (opt-in training objective; no reference counterpart) ----
+ * The logits are predict()'s (SRFR_model.py:144-152 with label = arange(1, N+1)) at every h row with a loss term:
+ * z_rj = <h_r, E_j>, j = 1..N (row 0, the pad item, is never a candidate); loss = sum_r w_r (LSE_j z_rj - z_r,pos) / norm[0],
+ * dh_r = (w_r / norm[0]) (sum_j p_rj E_j - E_pos),  dE_j = sum_r (w_r / norm[0]) (p_rj - 1[j = pos_r]) h_r,  dE_0 = 0.
+ * The (rows, N) logits never reach memory.  Operands: h_bf16 (cap_rows, ldh) and table_bf16 ((n_items + 1), ldt) bf16
+ * K-major rows padded with zeros to Dp columns (a multiple of 16, at most 256), 16-byte aligned with ld % 8 == 0;
+ * fp32 accumulation and LSE; probabilities enter the second tcgen05 product as bf16.
+ * Rows: rows = cap_rows, or min(cap_rows, rows_dev[0]) read on the device (packed token layout).  h row r belongs to
+ * dense token row_tok[r] (-1: none; NULL: identity); pos / w_pos are indexed by the dense token.  A row carries a loss
+ * term when its token exists, 1 <= pos <= n_items and its weight (w_pos, or 1 when w_pos is NULL) is non-zero.
+ * srfrd_catalogue_ce_plan: host only; the shared-memory bytes, ring stages and TMEM columns of the kernels (any pointer
+ * may be NULL); refuses a Dp the kernels cannot serve. */
+SRFRD_API int srfrd_catalogue_ce_plan(int Dp, int64_t* smem_bytes, int* ring_stages, int* tmem_cols);
+/* Pass 1: lse[r] (fp32, natural log) for r < rows, and loss_acc[0] += sum_r w_r (lse_r - z_r,pos) -- the unnormalised
+ * loss; the read-out of srfrd_adam_step_fused / srfrd_dp_adam_step / srfrd_loss_finalize divides it by norm[0]. */
+SRFRD_API int srfrd_catalogue_ce_fwd(const void* h_bf16, int ldh, const void* table_bf16, int ldt, int64_t n_items, int Dp,
+                                     const int64_t* pos, const float* w_pos, const int* row_tok, const int* rows_dev,
+                                     int64_t cap_rows, float* lse, float* loss_acc, void* stream);
+/* Passes 2 and 3 from pass 1's lse; norm[0] is read on the device (0 -> every gradient is 0).  dh (nullable): rows
+ * r < rows, first D columns, written (zero rows for rows without a loss term).  d_item (nullable, (n_items + 1, ldd)
+ * fp32): dE added to the first D columns of rows 1..n_items; each item tile is owned by one CTA, so the result is
+ * deterministic and needs no atomics. */
+SRFRD_API int srfrd_catalogue_ce_bwd(const void* h_bf16, int ldh, const void* table_bf16, int ldt, int64_t n_items, int Dp,
+                                     int D, const int64_t* pos, const float* w_pos, const float* norm, const int* row_tok,
+                                     const int* rows_dev, int64_t cap_rows, const float* lse, float* dh, int lddh,
+                                     float* d_item, int ldd, void* stream);
 
 /* ---- on-device batch sampler (next row 8f #1) ----
  * replaces: WarpSampler_fr / sample_function_fr (utils.py:14-90) and the seven LongTensor.to(device) copies per

@@ -86,6 +86,9 @@ SIGNATURES = {
     "srfrd_catalogue_topk": [vp, i64, i64, i32, vp, i64, i64, i64, i32, i32, i32, i32, vp, vp, vp, vp, i32],
     "srfrd_merge_topk_packed": [vp, i64, i32, i32, vp, vp, vp],
     "srfrd_catalogue_rank": [vp, i64, i64, i32, vp, i64, i64, i64, i32, i32, i32, vp, i32, vp, vp, vp, vp],
+    "srfrd_catalogue_ce_plan": [i32, C.POINTER(i64), C.POINTER(i32), C.POINTER(i32)],
+    "srfrd_catalogue_ce_fwd": [vp, i32, vp, i32, i64, i32, vp, vp, vp, vp, i64, vp, vp, vp],
+    "srfrd_catalogue_ce_bwd": [vp, i32, vp, i32, i64, i32, i32, vp, vp, vp, vp, vp, i64, vp, vp, i32, vp, i32, vp],
     "srfrd_attention_live_items": [vp, i64, i32, i32, vp, vp, vp, vp],
     "srfrd_set_attention_live": [vp, vp, vp, vp],
     "srfrd_merge_topk": [vp, vp, i64, i32, i32, vp, vp, vp],
@@ -133,7 +136,7 @@ def load() -> C.CDLL:
         fn = getattr(lib, name)            # AttributeError if the symbol is not exported
         fn.argtypes = argtypes
         fn.restype = C.c_int
-    if lib.srfrd_abi_version() != 9:
+    if lib.srfrd_abi_version() != 10:
         raise RuntimeError("srfrd_b200: ABI version mismatch between _lib.py and the built library")
     _lib = lib
     return lib

@@ -235,8 +235,23 @@ class HotPath:
             self.sh["wcT"] = zb(Hp, Dp)
             entries.append((P.mat("last_conv.weight"), self.sh["wc"][:D, :H], self.sh["wcT"][:H, :D]))
             vec("bc", P.view("last_conv.bias"), Dp)
+        self._cast_entries = entries
         self._cast_table, self._cast_n = ops.make_cast_table(entries, dev)
         self.shadows_version = -1
+
+    def enable_ce_table(self) -> torch.Tensor:
+        """The bf16 K-major copy of the item table the catalogue cross-entropy kernels read, (N + 1, Dp) with zero
+        padding columns, refreshed by the same cast launch as every other shadow from then on.  The table is cast in
+        blocks of rows so that a large catalogue spreads over many CTAs of that launch."""
+        if "ce_table" not in self.sh:
+            s = self.spec
+            E = self.P.view(s.item_key)
+            self.sh["ce_table"] = torch.zeros(E.shape[0], s.Dp, dtype=bf16, device=self.device)
+            for r0 in range(0, E.shape[0], 4096):
+                self._cast_entries.append((E[r0:r0 + 4096], self.sh["ce_table"][r0:r0 + 4096, :s.D], None))
+            self._cast_table, self._cast_n = ops.make_cast_table(self._cast_entries, self.device)
+            self.refresh_shadows()
+        return self.sh["ce_table"]
 
     def bias(self, tag: str, i: Optional[int] = None) -> torch.Tensor:
         """Bias vector a GEMM epilogue reads (length = the GEMM's padded N)."""

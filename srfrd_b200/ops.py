@@ -499,3 +499,36 @@ def mlp2_tn(A, W1, W2, mid_out, out, bias1=None, bias2=None, gate=None, relu1=Fa
                       mid_out.stride(0), _p(out), out.stride(0), _p(ln_out), 0 if ln_out is None else ln_out.stride(0),
                       _p(ln_w), _p(ln_b), _p(ln_stats), float(ln_eps))
     call("srfrd_mlp2_tn", _p(A), A.stride(0), _p(W1), W1.stride(0), _p(W2), W2.stride(0), M, N, C.byref(ep), _stream())
+
+
+def catalogue_ce_plan(Dp: int):
+    """(shared-memory bytes, ring stages, TMEM columns) of the cross-entropy kernels for padded width Dp (host only);
+    raises for a Dp they cannot serve (not a multiple of 16, or above 256)."""
+    smem, stages, tmem = C.c_int64(0), C.c_int(0), C.c_int(0)
+    call("srfrd_catalogue_ce_plan", int(Dp), C.byref(smem), C.byref(stages), C.byref(tmem))
+    return int(smem.value), int(stages.value), int(tmem.value)
+
+
+def _ce_rows(h, plan):
+    return (None, None, h.shape[0]) if plan is None else (plan.row_tok, plan.rows, plan.cap)
+
+
+def catalogue_ce_fwd(h, table, pos, w_pos, lse, loss_acc, plan: Optional[PackedPlan] = None):
+    """Pass 1 of the full-catalogue cross-entropy: lse (fp32, one per h row) and loss_acc[0] += sum w (lse - z_pos).
+    h: (rows, Dp) bf16; table: (N + 1, Dp) bf16; pos / w_pos indexed by dense token (plan: packed h rows)."""
+    _lib.require_device()
+    _chk(h, bf16, "h"); _chk(table, bf16, "table"); _chk(pos, torch.int64, "pos")
+    row_tok, rows, cap = _ce_rows(h, plan)
+    call("srfrd_catalogue_ce_fwd", _p(h), h.stride(0), _p(table), table.stride(0), table.shape[0] - 1, table.shape[1],
+         _p(pos), _p(w_pos), _p(row_tok), _p(rows), cap, _p(lse), _p(loss_acc), _stream())
+
+
+def catalogue_ce_bwd(h, table, pos, w_pos, norm, lse, dh, d_item, D, plan: Optional[PackedPlan] = None):
+    """Passes 2 and 3: dh (fp32 rows, first D columns written) and d_item ((N + 1, D) fp32, added to); either may be
+    None.  norm[0] is the loss normaliser (sum of the weights), read on the device."""
+    _lib.require_device()
+    _chk(h, bf16, "h"); _chk(table, bf16, "table"); _chk(pos, torch.int64, "pos")
+    row_tok, rows, cap = _ce_rows(h, plan)
+    call("srfrd_catalogue_ce_bwd", _p(h), h.stride(0), _p(table), table.stride(0), table.shape[0] - 1, table.shape[1],
+         int(D), _p(pos), _p(w_pos), _p(norm), _p(row_tok), _p(rows), cap, _p(lse), _p(dh),
+         0 if dh is None else dh.stride(0), _p(d_item), 0 if d_item is None else d_item.stride(0), _stream())

@@ -19,6 +19,7 @@ import torch
 
 from . import ops, parallel
 from .engine import HotPath
+from .losses import check_ce_width
 
 __all__ = ["simulate", "FusedTrainer", "DeviceSampler", "discriminator_weights"]
 
@@ -97,10 +98,24 @@ class FusedTrainer:
                    tensor), both from the parameters before the step's update.  The norm gradient reaches every row of the
                    embedding tables, the pad row included, so rows no batch touches drift under Adam as in the reference.
                    Fixed for the trainer's lifetime (a captured graph holds it).
+    loss         : "bce" -- the reference's objective (one sampled negative per position, trainer.py:31-38);
+                   "ce" -- full-catalogue softmax cross-entropy over predict's logits (every item 1..N a candidate, the
+                   positive the target; losses.catalogue_cross_entropy) with the same discriminator weights and normaliser,
+                   computed by the tcgen05 kernels of csrc/catalogue_ce.cu without materialising the logits.  The sampled
+                   negatives are unused and w_neg is refused; SRFRN is refused (its logits need a fake label per candidate,
+                   SRFR_model.py:225-233, which unobserved items do not have).
     """
 
     def __init__(self, model, lr: float = 1e-3, betas=(0.9, 0.98), eps: float = 1e-8, process_group=None,
-                 use_graph: bool = True, l2_emb: float = 0.0, packed: Optional[bool] = None):
+                 use_graph: bool = True, l2_emb: float = 0.0, packed: Optional[bool] = None, loss: str = "bce"):
+        if loss not in ("bce", "ce"):
+            raise ValueError(f"unknown loss {loss!r} (expected 'bce' or 'ce')")
+        if loss == "ce":
+            if model.spec.kind == "SRFRN":
+                raise ValueError("loss='ce' does not support SRFRN: its logits need each candidate's fake label "
+                                 "(SRFR_model.py:225-233), which unobserved items do not have")
+            check_ce_width(model.spec.D)
+        self.loss_kind = loss
         self.model = model
         self._dp = None
         if process_group is not None and torch.distributed.get_world_size(process_group) > 1:
@@ -126,9 +141,26 @@ class FusedTrainer:
         self._has_w = (False, False)
         self.l2_emb = float(l2_emb)
         self._l2 = self._setup_l2(model) if self.l2_emb != 0.0 else None
+        self._ce_ws: Optional[Dict[str, torch.Tensor]] = None
+        if loss == "ce":
+            self.eng.enable_ce_table()
         self.P.grad_bucket.zero_()
         self.eng.refresh_shadows()
         self.steps = 0
+
+    def _ce_buffers(self, rows: int) -> Dict[str, torch.Tensor]:
+        """bf16 copy of the final hidden rows and their log-sum-exp (loss="ce"); a larger batch re-allocates, which the
+        graph key's workspace generation covers."""
+        if self._ce_ws is None or self._ce_ws["lse"].numel() < rows:
+            dev = self.eng.device
+            self._ce_ws = dict(h=torch.zeros(rows, self.spec.Dp, dtype=torch.bfloat16, device=dev),
+                               lse=torch.zeros(rows, dtype=torch.float32, device=dev))
+            self.eng.ws_generation += 1
+        return self._ce_ws
+
+    def _refuse_w_neg(self, w_neg):
+        if w_neg is not None and self.loss_kind == "ce":
+            raise ValueError("w_neg weights the sampled negatives of the BCE; loss='ce' has no negatives")
 
     def _setup_l2(self, model) -> ops.ParamL2:
         """The regulariser's segment table: every tensor of model.parameters() is one segment of the flat buffer."""
@@ -231,7 +263,16 @@ class FusedTrainer:
         torch.cuda.current_stream().wait_stream(self.comm)
         prs_ = st["prs"].view(-1) if ft is not None else None
         nrs_ = st["nrs"].view(-1) if ft is not None else None
-        if packed:
+        if self.loss_kind == "ce":
+            plan = eng.saved["plan"] if packed else None
+            rows = plan.cap if packed else T
+            ce = self._ce_buffers(rows)
+            hb, lse, table = ce["h"][:rows], ce["lse"][:rows], eng.sh["ce_table"]
+            ops.f32_to_bf16_split(ws["hfin"][:rows], hb)
+            ops.catalogue_ce_fwd(hb, table, pos, w_pos, lse, acc, plan)
+            ops.catalogue_ce_bwd(hb, table, pos, w_pos, norm, lse, ws["dh"][:rows], P.view(s.item_key, grad=True), s.D, plan)
+            eng.backward(ws["dh"][:rows])
+        elif packed:
             plan = eng.saved["plan"]
             Tp = plan.cap
             ops.score_loss_fused_packed(ws["hfin"][:Tp], P.view(s.item_key), ft, pos, neg, prs_, nrs_, w_pos, w_neg, norm, acc,
@@ -258,6 +299,7 @@ class FusedTrainer:
     # ------------------------------------------------------------------
     def load_batch(self, batch: Dict[str, torch.Tensor], w_pos=None, w_neg=None, non_blocking: bool = True):
         """Copy one batch (host pinned or device tensors, int64 (B, L)) into the static buffers."""
+        self._refuse_w_neg(w_neg)
         B, L = batch["seq"].shape
         if self._static is None or self._static["seq"].shape != (B, L):
             self._alloc_static(B, L)
@@ -277,6 +319,7 @@ class FusedTrainer:
     def pack_batch(self, batch: Dict[str, torch.Tensor], w_pos=None, w_neg=None) -> torch.Tensor:
         """One flat device buffer holding a whole batch in the layout of the step's static inputs (six int64 (B, L) id
         arrays + two fp32 (B, L) weight arrays): ``step_packed`` then needs ONE device-to-device copy per step."""
+        self._refuse_w_neg(w_neg)
         B, L = batch["seq"].shape
         flat = torch.zeros(7 * B * L, dtype=torch.int64, device=self.eng.device)
         v = self._carve(flat, B, L)
@@ -304,6 +347,7 @@ class FusedTrainer:
         """Start copying a (pinned) host batch into a device staging buffer on a separate copy stream.  The next
         ``step_prefetched()`` waits for it, moves it into the step's static buffers with ONE device-to-device copy and
         runs the step, so the PCIe transfer of the next batch hides behind the current step."""
+        self._refuse_w_neg(w_neg)
         B, L = batch["seq"].shape
         if self._static is None or self._static["seq"].shape != (B, L):
             self._alloc_static(B, L)

@@ -1,7 +1,8 @@
 """Multi-GPU check (run under torchrun): G-rank data-parallel FusedTrainer == 1-rank on the concatenated batch,
 and row-sharded catalogue top-10 (NCCL all-gather + merge) == unsharded top-10.
 `--l2 X` trains both with l2_emb = X (the regulariser's gradient is added once, after the reduction over ranks).
-`--topk-k K` checks the sharded top-K (1 <= K <= 64) instead of the top-10."""
+`--topk-k K` checks the sharded top-K (1 <= K <= 64) instead of the top-10.
+`--loss ce` trains both with the full-catalogue cross-entropy (FusedTrainer(loss="ce")) instead of the BCE."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -33,10 +34,12 @@ P.broadcast_parameters(m_dp.flat_parameters().data, 0)
 use_graph = os.environ.get("DP_CHECK_GRAPH", "0") == "1"
 l2_emb = float(sys.argv[sys.argv.index("--l2") + 1]) if "--l2" in sys.argv else 0.0
 topk_k = int(sys.argv[sys.argv.index("--topk-k") + 1]) if "--topk-k" in sys.argv else 10
-tr_dp = FusedTrainer(m_dp, process_group=dist.group.WORLD, use_graph=use_graph, l2_emb=l2_emb)
+loss = sys.argv[sys.argv.index("--loss") + 1] if "--loss" in sys.argv else "bce"
+tr_dp = FusedTrainer(m_dp, process_group=dist.group.WORLD, use_graph=use_graph, l2_emb=l2_emb, loss=loss)
 if rank == 0:
-    print("fused reduce-scatter/Adam/all-gather kernel:", tr_dp._dp is not None, "graph:", use_graph, "l2_emb:", l2_emb)
-tr_one = FusedTrainer(m_one, use_graph=False, l2_emb=l2_emb)
+    print("fused reduce-scatter/Adam/all-gather kernel:", tr_dp._dp is not None, "graph:", use_graph, "l2_emb:", l2_emb,
+          "loss:", loss)
+tr_one = FusedTrainer(m_one, use_graph=False, l2_emb=l2_emb, loss=loss)
 ok = True
 for i, nb in enumerate(batches):
     full = {k: torch.from_numpy(v).to(dev) for k, v in nb.items()}
