@@ -79,10 +79,7 @@ class _EncodeAndScore(torch.autograd.Function):
         seq, rsq, pos, prs, neg, nrs = ctx.ids
         B, L = seq.shape
         T = B * L
-        if eng.saved is None or eng.saved.get("version") != ctx.version or eng.fwd_version != ctx.version:
-            raise RuntimeError("srfrd_b200: backward() of a stale forward -- another forward() (training, validation or "
-                               "predict) ran on this model after the one being back-propagated and overwrote the shared "
-                               "activation workspace; run backward() before the next forward()")
+        eng.check_saved(ctx.version)                # raises before score_bwd writes anything
         ws = eng._ws
         dh = ws["dh"][:T]
         eng.P.grad.zero_()

@@ -167,8 +167,33 @@ class FlatParams:
         return v.view(v.shape[0], -1)
 
 
+@dataclass
+class _Saved:
+    """What a saving forward used; backward() takes every input and layout decision from here."""
+    seq: torch.Tensor
+    aux_ids: Optional[torch.Tensor]
+    B: int
+    L: int
+    T: int                                # activation rows: B * L dense, plan.cap packed
+    row_ids: torch.Tensor                 # item id of every row (0: a pad row, zeroed by the row_ids epilogues)
+    plan: Optional[ops.PackedPlan]        # None: dense layout
+    hyb: Optional[Dict[str, torch.Tensor]]    # hybrid mode's dense attention operands (None: dense or tile layout)
+    live: Optional[ops.LiveTiles]         # hybrid mode's live query tiles (None: every tile walked)
+    p_drop: float
+    seed: int
+    step: Optional[torch.Tensor]
+    fuse_ln: bool
+    oproj: int                            # bit 0 / 1: the packed attention forward / backward takes the out-projection
+    mlp2: bool                            # FFN1 + FFN2 (and their backward pair) as one mlp2_tn launch
+    version: int
+
+    def __getitem__(self, key: str):
+        """saved["plan"] etc.: callers that read the forward's record as the dict it used to be keep working."""
+        return getattr(self, key)
+
+
 class HotPath:
-    """Forward / backward kernel sequences over a FlatParams store."""
+    """Forward / backward kernel sequences over a FlatParams store, one sequence for the dense and the packed layout."""
 
     def __init__(self, spec: ModelSpec, params: FlatParams):
         self.spec, self.P = spec, params
@@ -189,10 +214,15 @@ class HotPath:
         self.side2 = torch.cuda.Stream(device=self.device)     # a second independent branch (backward: dx through k | v)
         self.overlap = os.environ.get("SRFRD_OVERLAP", "1") != "0"
         self.drop_seed = 0x5EED5EED
-        self.saved: Optional[dict] = None
+        self.saved: Optional[_Saved] = None
         self._plans: Dict[Tuple[int, int], ops.PackedPlan] = {}
+        self._lives: Dict[Tuple[int, int], ops.LiveTiles] = {}
+        # experiment switches (DESIGN.md section 8), fixed for the engine's lifetime
         self.packed_default = os.environ.get("SRFRD_PACKED", "1") != "0"
         self.fuse_ffn = os.environ.get("SRFRD_FUSE_FFN", "1") != "0"    # FFN1 + FFN2 (and their backward pair) in one launch
+        self.fuse_ln = os.environ.get("SRFRD_FUSE_LN", "1") != "0"      # LayerNorms in the epilogues of the GEMMs before them
+        self.hybrid = os.environ.get("SRFRD_HYBRID", "1") != "0"        # packed layout for maxlen > 127 (packed_mode)
+        self.live_tiles = os.environ.get("SRFRD_LIVE_TILES", "1") != "0"  # hybrid attention skips all-pad query tiles
 
     # ------------------------------------------------------------------ bf16 operand shadows
     def _build_shadows(self):
@@ -350,7 +380,7 @@ class HotPath:
             return None
         if ops.attention_packed_supported(L, s.H, s.num_heads):
             return "tile"
-        if os.environ.get("SRFRD_HYBRID", "1") != "0" and L <= 4096:
+        if self.hybrid and L <= 4096:
             return "hybrid"
         return None
 
@@ -370,28 +400,36 @@ class HotPath:
         self.ws_generation += 1
         return hw
 
-    def _live_tiles(self, B: int, L: int) -> "ops.LiveTiles":
-        key = (B, L)
-        lt = getattr(self, "_lives", None)
-        if lt is None:
-            lt = self._lives = {}
-        if key not in lt:
-            if len(lt) >= 4:                          # a captured graph may hold pointers into these: bump the generation
-                lt.clear()
+    def _cached(self, cache: dict, key, make):
+        """cache[key], made on a miss.  A captured graph may hold pointers into the entries, so when a fifth key arrives the
+        cache is cleared and ws_generation bumped (FusedTrainer then re-captures)."""
+        if key not in cache:
+            if len(cache) >= 4:
+                cache.clear()
                 self.ws_generation += 1
-            lt[key] = ops.LiveTiles(B, L, self.spec.num_heads, self.device)
-        return lt[key]
-
-    def _plan(self, B: int, L: int) -> "ops.PackedPlan":
-        key = (B, L)
-        if key not in self._plans:
-            if len(self._plans) >= 4:                 # a captured graph may hold pointers into a plan: bump the generation
-                self._plans.clear()
-                self.ws_generation += 1
-            self._plans[key] = ops.PackedPlan(B, L, self.device)
-        return self._plans[key]
+            cache[key] = make()
+        return cache[key]
 
     # ------------------------------------------------------------------ forward
+    def _aux_ids(self, fake_ids: Optional[torch.Tensor], B: int, L: int) -> Optional[torch.Tensor]:
+        """The embedding's aux ids: the per-token fake labels (SRFR / SRFRN) or the per-user labels (SRFU_*)."""
+        s = self.spec
+        if s.mode == 1:
+            return None if fake_ids is None else fake_ids.contiguous()
+        if s.mode != 2:
+            return None
+        aux_ids = torch.empty(B, dtype=torch.int64, device=self.device)
+        ops.srfu_labels(fake_ids.contiguous(), {"SRFU_B": 0, "SRFU_F": 1, "SRFU_R": 2}[s.kind], aux_ids)
+        # label ranges are static per kind: B {1, 2}, F [0, L], R [0, 10] (SRFR_model.py:546-570; the reference's own
+        # zoo passes 3 / maxlen + 1 / 11 rows, trainer.py:173-205).  A smaller table (e.g. the constructor default
+        # number_of_labels = 2) makes the reference raise IndexError when such a label occurs; only in that
+        # under-provisioned case the labels are checked here (one D2H sync) instead of reading past the table.
+        need = {"SRFU_B": 3, "SRFU_F": L + 1, "SRFU_R": 11}[s.kind]
+        if s.n_labels < need and B > 0 and int(aux_ids.max()) >= s.n_labels:
+            raise IndexError(f"index out of range in self: {s.kind} user label {int(aux_ids.max())} needs "
+                             f"number_of_labels >= {need}, got {s.n_labels}")
+        return aux_ids
+
     def forward(self, seq: torch.Tensor, fake_ids: Optional[torch.Tensor], training: bool,
                 last_only: bool = False, save: Optional[bool] = None, packed: bool = False,
                 keep: Optional[torch.Tensor] = None) -> torch.Tensor:
@@ -399,14 +437,16 @@ class HotPath:
         hidden[:, -1, :] only, SRFR_model.py:147).  Saves what backward needs when training.
         packed=True runs on the packed token layout (pad slots are not computed; `keep` (B, L) marks pad slots that must
         still get a row because they carry a loss term): the full hidden state is then left in PACKED rows in the
-        workspace (ws["hfin"], row maps in the plan) and only last_only returns a dense result."""
+        workspace (ws["hfin"], row maps in the plan) and only last_only returns a dense result.  The packed row count M is
+        data dependent and lives on the device: every row-wise kernel reads it through ops.row_limit, the packed kernels
+        take the plan."""
         s, P = self.spec, self.P
         B, L = seq.shape
         if L > s.max_len:
             raise RuntimeError(f"sequence length {L} exceeds max_len {s.max_len} (pos_embed rows, SRFR_model.py:12)")
-        if packed:
-            return self._forward_packed(seq, fake_ids, training, last_only, save, keep)
-        T, H, Hp, nb = B * L, s.H, s.Hp, s.num_blocks
+        H, Hp, nb = s.H, s.Hp, s.num_blocks
+        plan = self._cached(self._plans, (B, L), lambda: ops.PackedPlan(B, L, self.device)) if packed else None
+        T = plan.cap if packed else B * L
         ws = self._workspace(T, L)
         self.fwd_version += 1                   # EVERY forward overwrites the shared activations (saving or not)
         p_drop = s.dropout if training else 0.0
@@ -416,213 +456,36 @@ class HotPath:
         # _EncodeAndScore bumps host_drop_counter per training forward and it is folded into the seed here
         seed = (self.drop_seed + self.host_drop_counter * 0x9E3779B97F4A7C15) & 0xFFFFFFFFFFFFFFFF
         seq = seq.contiguous()
-        aux_ids = None
-        if s.mode == 1:
-            aux_ids = None if fake_ids is None else fake_ids.contiguous()
-        elif s.mode == 2:
-            aux_ids = torch.empty(B, dtype=torch.int64, device=self.device)
-            ops.srfu_labels(fake_ids.contiguous(), {"SRFU_B": 0, "SRFU_F": 1, "SRFU_R": 2}[s.kind], aux_ids)
-            # label ranges are static per kind: B {1, 2}, F [0, L], R [0, 10] (SRFR_model.py:546-570; the reference's own
-            # zoo passes 3 / maxlen + 1 / 11 rows, trainer.py:173-205).  A smaller table (e.g. the constructor default
-            # number_of_labels = 2) makes the reference raise IndexError when such a label occurs; only in that
-            # under-provisioned case the labels are checked here (one D2H sync) instead of reading past the table.
-            need = {"SRFU_B": 3, "SRFU_F": L + 1, "SRFU_R": 11}[s.kind]
-            if s.n_labels < need and B > 0 and int(aux_ids.max()) >= s.n_labels:
-                raise IndexError(f"index out of range in self: {s.kind} user label {int(aux_ids.max())} needs "
-                                 f"number_of_labels >= {need}, got {s.n_labels}")
-        aux_table = P.view(s.aux_key) if s.aux_key else None
-        x = [ws[f"x{i}"][:T] for i in range(nb + 1)]
-        ops.embed_ln_fwd(P.view(s.item_key), P.view(s.pos_key), aux_table, s.mode, seq, aux_ids, s.item_scale,
-                         P.view("attention_layernorms.0.weight"), P.view("attention_layernorms.0.bias"), LN_EPS,
-                         x0_bf16=x[0], q_bf16=ws["Q0"][:T], stats=ws["st1_0"][:T],
-                         drop_p=p_drop if s.kind == "SASRec" else 0.0, drop_seed=seed, drop_stream=1, drop_step=step)
-        seq_flat = seq.view(-1)
+        aux_ids = self._aux_ids(fake_ids, B, L)
+        hyb = live = None
+        if packed:
+            plan.build(seq, None if keep is None else keep.contiguous())
+            if self.packed_mode(B, L) == "hybrid":
+                hyb = self._hybrid_ws(B * L)
+                if self.live_tiles:
+                    # query tiles whose 128 positions are all dropped padding (C4: the first tile of 58 % of the sequences):
+                    # the dense-layout attention kernels skip them -- nothing reads a pad query's o / dq and its dO is zero
+                    live = self._cached(self._lives, (B, L), lambda: ops.LiveTiles(B, L, s.num_heads, self.device))
+                    live.build(plan)
         # rows wider than the true width (ragged H, zero padded) keep the separate LayerNorm with true-width statistics
-        fuse_ln = (H == Hp) and Hp <= 128 and os.environ.get("SRFRD_FUSE_LN", "1") != "0"
-        for i in range(nb):
-            Q, q, kv, o, r, y, h1 = (ws[f"{n}{i}"][:T] for n in ("Q", "q", "kv", "o", "r", "y", "h1"))
-            with self._branch():                                   # k | v need the un-normalised x only
-                ops.gemm_tn(x[i], self.sh[f"wkv{i}"], out_bf16=kv, bias=self.bias("bkv", i))
-            if i > 0 and not fuse_ln:
-                ops.layernorm_fwd(x[i], P.view(f"attention_layernorms.{i}.weight"), P.view(f"attention_layernorms.{i}.bias"),
-                                  LN_EPS, y_bf16=Q, stats=ws[f"st1_{i}"][:T], H=H)
-            ops.gemm_tn(Q, self.sh[f"wq{i}"], out_bf16=q, bias=self.bias("bq", i))
-            self._join()                                           # k | v (side stream) are ready
-            ops.attention_fwd(q, kv[:, :Hp], kv[:, Hp:], o, B, L, H, s.num_heads, p_drop, seed, 10 + 4 * i, step,
-                              stats=ws.get(f"ast{i}"))
-            if fuse_ln:                                            # LayerNorm computed in the GEMM's epilogue
-                ops.gemm_tn(o, self.sh[f"wo{i}"], out_bf16=r, bias=self.bias("bo", i), residual=Q, ln_out=y,
-                            ln_w=P.view(f"forward_layernorms.{i}.weight"), ln_b=P.view(f"forward_layernorms.{i}.bias"),
-                            ln_eps=LN_EPS, ln_stats=ws[f"st2_{i}"][:T])
+        fuse_ln = H == Hp and Hp <= 128 and self.fuse_ln
+        # the packed tile attention takes the out-projection (bit 0 forward, bit 1 backward) with one head at the
+        # fused-LayerNorm width when the kernel's shared-memory plan fits; otherwise the separate gemm_tn launches
+        oproj = 0
+        if packed and hyb is None and s.num_heads == 1 and fuse_ln:
+            oproj = ops.attention_packed_oproj_supported(L, H, s.num_heads)
+        sv = _Saved(seq=seq, aux_ids=aux_ids, B=B, L=L, T=T, row_ids=plan.row_ids if packed else seq.view(-1), plan=plan,
+                    hyb=hyb, live=live, p_drop=p_drop, seed=seed, step=step, fuse_ln=fuse_ln, oproj=oproj,
+                    mlp2=packed and self.fuse_ffn and Hp <= 128, version=self.fwd_version)
+        x = [ws[f"x{i}"][:T] for i in range(nb + 1)]
+        with ops.row_limit(plan.rows) if packed else nullcontext():
+            emb = (P.view(s.item_key), P.view(s.pos_key), P.view(s.aux_key) if s.aux_key else None, s.mode, seq, aux_ids,
+                   s.item_scale, P.view("attention_layernorms.0.weight"), P.view("attention_layernorms.0.bias"), LN_EPS)
+            emb_drop = dict(drop_p=p_drop if s.kind == "SASRec" else 0.0, drop_seed=seed, drop_stream=1, drop_step=step)
+            if packed:
+                ops.embed_ln_fwd_packed(*emb, x[0], ws["Q0"][:T], ws["st1_0"][:T], plan, **emb_drop)
             else:
-                ops.gemm_tn(o, self.sh[f"wo{i}"], out_bf16=r, bias=self.bias("bo", i), residual=Q)
-                ops.layernorm_fwd(r, P.view(f"forward_layernorms.{i}.weight"), P.view(f"forward_layernorms.{i}.bias"), LN_EPS,
-                                  y_bf16=y, stats=ws[f"st2_{i}"][:T], H=H)
-            ops.gemm_tn(y, self.sh[f"w1{i}"], out_bf16=h1, bias=self.bias("b1", i), relu=True,
-                        drop_p=p_drop, drop_seed=seed, drop_stream=11 + 4 * i, drop_step=step)
-            nxt = {}
-            if fuse_ln and i + 1 < nb:                             # the next block's attention LayerNorm rides along
-                nxt = dict(ln_out=ws[f"Q{i + 1}"][:T], ln_w=P.view(f"attention_layernorms.{i + 1}.weight"),
-                           ln_b=P.view(f"attention_layernorms.{i + 1}.bias"), ln_eps=LN_EPS, ln_stats=ws[f"st1_{i + 1}"][:T])
-            ops.gemm_tn(h1, self.sh[f"w2{i}"], out_bf16=x[i + 1], bias=self.bias("b2", i),
-                        residual=y, row_ids=seq_flat, drop_p=p_drop, drop_seed=seed, drop_stream=12 + 4 * i, drop_step=step,
-                        **nxt)
-        fin_in = x[nb]
-        if s.kind == "SRFR":      # last_conv H -> D (SRFR_model.py:123)
-            ops.gemm_tn(x[nb], self.sh["wc"], out_bf16=ws["c"][:T], bias=self.bias("bc"))
-            fin_in = ws["c"][:T]
-        hfin = ws["hfin"][:T]
-        if last_only:
-            out = ws["hfin"][:B]
-            ops.layernorm_fwd(fin_in, P.view("last_layernorm.weight"), P.view("last_layernorm.bias"), LN_EPS, y_f32=out,
-                              T=B, H=s.Dout, row_stride=L, row_offset=L - 1)
-            return out[:, :s.Dout]
-        ops.layernorm_fwd(fin_in, P.view("last_layernorm.weight"), P.view("last_layernorm.bias"), LN_EPS, y_f32=hfin,
-                          stats=ws["stF"][:T], H=s.Dout)
-        if training if save is None else save:
-            self.saved = dict(seq=seq, aux_ids=aux_ids, B=B, L=L, p_drop=p_drop, seed=seed, step=step,
-                              version=self.fwd_version)
-        return hfin.view(B, L, s.Doutp)[..., :s.Dout]
-
-    # ------------------------------------------------------------------ backward
-    def backward(self, dh: torch.Tensor, version: Optional[int] = None) -> None:
-        """Given dL/dhidden (T, Dout) fp32, accumulate every parameter gradient into P.grad
-        (the score kernels have already added the pos/neg rows of the item table).  The activations live in the
-        engine's shared workspace, so only the LATEST saving forward can be back-propagated: `version` (the stamp the
-        autograd node took at forward time) is checked against it."""
-        s, P, sv = self.spec, self.P, self.saved
-        if sv is None:
-            raise RuntimeError("backward() without a training forward()")
-        if sv["version"] != self.fwd_version or (version is not None and version != sv["version"]):
-            raise RuntimeError("srfrd_b200: backward() of a stale forward -- another forward() (training, validation or "
-                               "predict) ran on this model after the one being back-propagated and overwrote the shared "
-                               "activation workspace; run backward() before the next forward()")
-        if sv.get("plan") is not None:
-            return self._backward_packed(dh)
-        B, L = sv["B"], sv["L"]
-        T, H, Hp, nb = B * L, s.H, s.Hp, s.num_blocks
-        ws = self._ws
-        seq_flat = sv["seq"].view(-1)
-        p_drop, seed, step = sv["p_drop"], sv["seed"], sv["step"]
-        gA, gC, gD, gX = (ws[n][:T] for n in ("gA", "gC", "gD", "gX"))
-        G = lambda name: P.view(name, grad=True)
-        GM = lambda name: P.mat(name, grad=True)
-        x = [ws[f"x{i}"][:T] for i in range(nb + 1)]
-        dz_top = ws[f"gdz_{nb - 1}"][:T]
-
-        # final LayerNorm (+ last_conv) -> dz = dL/dx[nb], pad rows zeroed
-        if s.kind == "SRFR":
-            gc = ws["gc"][:T]
-            ops.layernorm_bwd(dh, ws["c"][:T], ws["stF"][:T], P.view("last_layernorm.weight"), gc,
-                              G("last_layernorm.weight"), G("last_layernorm.bias"), H=s.D)
-            with self._branch():
-                ops.gemm_wgrad(gc, x[nb], GM("last_conv.weight"), G("last_conv.bias"), Mo=s.D, No=H)
-            ops.gemm_tn(gc, self.sh["wcT"], out_bf16=dz_top, row_ids=seq_flat)
-        else:
-            ops.layernorm_bwd(dh, x[nb], ws["stF"][:T], P.view("last_layernorm.weight"), dz_top,
-                              G("last_layernorm.weight"), G("last_layernorm.bias"), row_ids=seq_flat, H=s.Dout)
-
-        for i in reversed(range(nb)):
-            Q, q, kv, o, r, y, h1 = (ws[f"{n}{i}"][:T] for n in ("Q", "q", "kv", "o", "r", "y", "h1"))
-            dz, da1, dr, dq, dkv = (ws[f"{n}{i}"][:T] for n in ("gdz_", "gda1_", "gdr_", "gdq_", "gdkv_"))
-            dx_out = ws[f"gdz_{i - 1}"][:T] if i > 0 else gA          # dL/dx[i]: the next (earlier) block's dz
-            dz2 = dz
-            if p_drop > 0:      # da2 = dz * mask2 (dropout2 sits between conv2 and the residual add)
-                dz2 = ws[f"gE_{i}"][:T]
-                ops.dropout_apply(dz, dz2, Hp, p_drop, seed, 12 + 4 * i, step)
-            # FFN: z = drop2(h1 W2^T + b2) + y ; h1 = relu(drop1(y W1^T + b1))
-            with self._branch():
-                ops.gemm_wgrad(dz2, h1, GM(f"forward_layers.{i}.conv2.weight"), G(f"forward_layers.{i}.conv2.bias"), Mo=H, No=H)
-            ops.gemm_tn(dz2, self.sh[f"w2T{i}"], out_bf16=da1, gate=h1, drop_p=p_drop, drop_seed=seed,
-                        drop_stream=11 + 4 * i, drop_step=step)                                   # da1
-            with self._branch():
-                ops.gemm_wgrad(da1, y, GM(f"forward_layers.{i}.conv1.weight"), G(f"forward_layers.{i}.conv1.bias"), Mo=H, No=H)
-            ops.gemm_tn(da1, self.sh[f"w1T{i}"], out_bf16=gC, residual=dz)                         # dy
-            # LN2
-            ops.layernorm_bwd(gC, r, ws[f"st2_{i}"][:T], P.view(f"forward_layernorms.{i}.weight"), dr,
-                              G(f"forward_layernorms.{i}.weight"), G(f"forward_layernorms.{i}.bias"), H=H)   # dr
-            # r = Q + o Wo^T + bo
-            with self._branch():
-                ops.gemm_wgrad(dr, o, GM(f"attention_layers.{i}.out_proj.weight"), G(f"attention_layers.{i}.out_proj.bias"),
-                               Mo=H, No=H)
-            ops.gemm_tn(dr, self.sh[f"woT{i}"], out_bf16=gC)                                       # do
-            ops.attention_bwd(gC, q, kv[:, :Hp], kv[:, Hp:], dq, dkv[:, :Hp], dkv[:, Hp:], B, L, H, s.num_heads, p_drop,
-                              seed, 10 + 4 * i, step, o=o, stats=ws.get(f"ast{i}"))               # dq, dk|dv
-            gin = GM(f"attention_layers.{i}.in_proj_weight")
-            gbin = G(f"attention_layers.{i}.in_proj_bias")
-            with self._branch():
-                ops.gemm_wgrad(dq, Q, gin[:H], gbin[:H], Mo=H, No=H)
-                if Hp == H:
-                    ops.gemm_wgrad(dkv, x[i], gin[H:], gbin[H:], Mo=2 * H, No=H)
-                else:   # k and v gradients sit at column offsets 0 and Hp: two row blocks of in_proj_weight
-                    ops.gemm_wgrad(dkv[:, :Hp], x[i], gin[H:2 * H], gbin[H:2 * H], Mo=H, No=H)
-                    ops.gemm_wgrad(dkv[:, Hp:], x[i], gin[2 * H:], gbin[2 * H:], Mo=H, No=H)
-            with self._branch(second=True):                                                        # independent of dQ
-                ops.gemm_tn(dkv, self.sh[f"wkvT{i}"], out_bf16=gX)                                 # dx via k, v
-            ops.gemm_tn(dq, self.sh[f"wqT{i}"], out_bf16=gD, residual=dr)                          # dQ = dr + dq Wq
-            self._join(second=True)
-            # LN1 + the un-normalised k/v path; pad rows zeroed (x_i was masked, SRFR_model.py:99,121)
-            ops.layernorm_bwd(gD, x[i], ws[f"st1_{i}"][:T], P.view(f"attention_layernorms.{i}.weight"), dx_out,
-                              G(f"attention_layernorms.{i}.weight"), G(f"attention_layernorms.{i}.bias"),
-                              add=gX, row_ids=seq_flat, H=H)
-
-        # embedding tables
-        dx0 = gA
-        if s.kind == "SASRec" and p_drop > 0:
-            ops.dropout_apply(gA, gC, H, p_drop, seed, 1, step)
-            dx0 = gC
-        aux_grad = G(s.aux_key) if s.aux_key else None
-        ops.embed_bwd(dx0, sv["seq"], sv["aux_ids"], s.D, s.F if s.mode == 1 else 0, s.mode, s.item_scale,
-                      G(s.item_key), aux_grad)
-        pos_tmp = ws["pos_tmp"][:L * Hp]          # zero on entry: allocated zeroed, and add_segments consumes (re-zeroes) it
-        ops.colsum(dx0, pos_tmp, M=B, N=L * Hp, ld=L * Hp)
-        ops.add_segments(pos_tmp, L * Hp, Hp, s.D, G(s.pos_key))
-        self._join()                                # every weight gradient has landed in P.grad
-        self.saved = None
-
-    # ------------------------------------------------------------------ packed forward / backward
-    def _forward_packed(self, seq, fake_ids, training, last_only, save, keep):
-        """The same kernel sequence as forward() over M packed rows (M is data dependent and lives on the device:
-        every row-wise kernel reads it through ops.row_limit, the packed kernels take the plan)."""
-        s, P = self.spec, self.P
-        B, L = seq.shape
-        H, Hp, nb = s.H, s.Hp, s.num_blocks
-        plan = self._plan(B, L)
-        T = plan.cap
-        ws = self._workspace(T, L)
-        self.fwd_version += 1
-        p_drop = s.dropout if training else 0.0
-        step = self.step_state[3:4] if p_drop > 0 else None
-        seed = (self.drop_seed + self.host_drop_counter * 0x9E3779B97F4A7C15) & 0xFFFFFFFFFFFFFFFF
-        seq = seq.contiguous()
-        aux_ids = None
-        if s.mode == 1:
-            aux_ids = None if fake_ids is None else fake_ids.contiguous()
-        elif s.mode == 2:
-            aux_ids = torch.empty(B, dtype=torch.int64, device=self.device)
-            ops.srfu_labels(fake_ids.contiguous(), {"SRFU_B": 0, "SRFU_F": 1, "SRFU_R": 2}[s.kind], aux_ids)
-            need = {"SRFU_B": 3, "SRFU_F": L + 1, "SRFU_R": 11}[s.kind]
-            if s.n_labels < need and int(aux_ids.max()) >= s.n_labels:
-                raise IndexError(f"index out of range in self: {s.kind} user label {int(aux_ids.max())} needs "
-                                 f"number_of_labels >= {need}, got {s.n_labels}")
-        aux_table = P.view(s.aux_key) if s.aux_key else None
-        plan.build(seq, None if keep is None else keep.contiguous())
-        hyb = self._hybrid_ws(B * L) if self.packed_mode(B, L) == "hybrid" else None
-        live = None
-        if hyb is not None and os.environ.get("SRFRD_LIVE_TILES", "1") != "0":
-            # query tiles whose 128 positions are all dropped padding (C4: the first tile of 58 % of the sequences): the
-            # dense-layout attention kernels skip them -- nothing reads a pad query's o / dq and its dO is zero
-            live = self._live_tiles(B, L)
-            live.build(plan)
-        x = [ws[f"x{i}"][:T] for i in range(nb + 1)]
-        row_ids = plan.row_ids
-        fuse_ln = Hp <= 128 and os.environ.get("SRFRD_FUSE_LN", "1") != "0"
-        fuse_oproj = self._fuse_oproj(hyb, L, fuse_ln) & 1
-        with ops.row_limit(plan.rows):
-            ops.embed_ln_fwd_packed(P.view(s.item_key), P.view(s.pos_key), aux_table, s.mode, seq, aux_ids, s.item_scale,
-                                    P.view("attention_layernorms.0.weight"), P.view("attention_layernorms.0.bias"), LN_EPS,
-                                    x[0], ws["Q0"][:T], ws["st1_0"][:T], plan,
-                                    drop_p=p_drop if s.kind == "SASRec" else 0.0, drop_seed=seed, drop_stream=1, drop_step=step)
+                ops.embed_ln_fwd(*emb, x0_bf16=x[0], q_bf16=ws["Q0"][:T], stats=ws["st1_0"][:T], **emb_drop)
             for i in range(nb):
                 Q, q, kv, o, r, y, h1 = (ws[f"{n}{i}"][:T] for n in ("Q", "q", "kv", "o", "r", "y", "h1"))
                 with self._branch():                                   # k | v need the un-normalised x only
@@ -631,87 +494,104 @@ class HotPath:
                     ops.layernorm_fwd(x[i], P.view(f"attention_layernorms.{i}.weight"), P.view(f"attention_layernorms.{i}.bias"),
                                       LN_EPS, y_bf16=Q, stats=ws[f"st1_{i}"][:T], H=H)
                 ops.gemm_tn(Q, self.sh[f"wq{i}"], out_bf16=q, bias=self.bias("bq", i))
-                self._join()
-                if fuse_oproj:              # out-projection, residual and LayerNorm in the attention kernel's epilogue
-                    ops.attention_fwd_packed(q, kv[:, :Hp], kv[:, Hp:], o, plan, L, H, s.num_heads, p_drop, seed, 10 + 4 * i, step,
-                                             wo=self.sh[f"wo{i}"], bias=self.bias("bo", i), residual=Q, r=r, y=y,
-                                             ln_w=P.view(f"forward_layernorms.{i}.weight"),
-                                             ln_b=P.view(f"forward_layernorms.{i}.bias"), ln_eps=LN_EPS,
-                                             ln_stats=ws[f"st2_{i}"][:T])
-                elif hyb is None:
-                    ops.attention_fwd_packed(q, kv[:, :Hp], kv[:, Hp:], o, plan, L, H, s.num_heads, p_drop, seed, 10 + 4 * i, step)
-                else:       # dense-layout attention between an unpack and a pack copy
-                    qd, kvd, od = hyb[f"qd{i}"][:B * L], hyb[f"kvd{i}"][:B * L], hyb[f"od{i}"][:B * L]
-                    ops.unpack_rows([(q, qd, Hp, 0), (kv, kvd, 2 * Hp, 0)], plan)
-                    with (live.active() if live is not None else nullcontext()):
-                        ops.attention_fwd(qd, kvd[:, :Hp], kvd[:, Hp:], od, B, L, H, s.num_heads, p_drop, seed, 10 + 4 * i, step,
-                                          stats=ws.get(f"ast{i}"))
-                    ops.pack_rows([(od, o, Hp, 0)], plan)
-                if fuse_oproj:
+                self._join()                                           # k | v (side stream) are ready
+                ln2 = dict(ln_w=P.view(f"forward_layernorms.{i}.weight"), ln_b=P.view(f"forward_layernorms.{i}.bias"),
+                           ln_eps=LN_EPS, ln_stats=ws[f"st2_{i}"][:T])
+                fold = dict(wo=self.sh[f"wo{i}"], bias=self.bias("bo", i), residual=Q, r=r, y=y, **ln2) if oproj & 1 else {}
+                self._attention_fwd(sv, i, q, kv, o, ws.get(f"ast{i}"), fold)
+                if oproj & 1:
                     pass                    # r, y and their statistics came out of the attention kernel
-                elif fuse_ln:
-                    ops.gemm_tn(o, self.sh[f"wo{i}"], out_bf16=r, bias=self.bias("bo", i), residual=Q, ln_out=y,
-                                ln_w=P.view(f"forward_layernorms.{i}.weight"), ln_b=P.view(f"forward_layernorms.{i}.bias"),
-                                ln_eps=LN_EPS, ln_stats=ws[f"st2_{i}"][:T])
+                elif fuse_ln:                                          # LayerNorm computed in the GEMM's epilogue
+                    ops.gemm_tn(o, self.sh[f"wo{i}"], out_bf16=r, bias=self.bias("bo", i), residual=Q, ln_out=y, **ln2)
                 else:
                     ops.gemm_tn(o, self.sh[f"wo{i}"], out_bf16=r, bias=self.bias("bo", i), residual=Q)
-                    ops.layernorm_fwd(r, P.view(f"forward_layernorms.{i}.weight"), P.view(f"forward_layernorms.{i}.bias"),
-                                      LN_EPS, y_bf16=y, stats=ws[f"st2_{i}"][:T], H=H)
+                    ops.layernorm_fwd(r, ln2["ln_w"], ln2["ln_b"], LN_EPS, y_bf16=y, stats=ln2["ln_stats"], H=H)
                 nxt = {}
-                if fuse_ln and i + 1 < nb:
+                if fuse_ln and i + 1 < nb:                             # the next block's attention LayerNorm rides along
                     nxt = dict(ln_out=ws[f"Q{i + 1}"][:T], ln_w=P.view(f"attention_layernorms.{i + 1}.weight"),
                                ln_b=P.view(f"attention_layernorms.{i + 1}.bias"), ln_eps=LN_EPS,
                                ln_stats=ws[f"st1_{i + 1}"][:T])
-                if self.fuse_ffn and Hp <= 128:            # FFN1 + FFN2 (+ the next LayerNorm) in one launch, h1 through smem
+                if sv.mlp2:                 # FFN1 + FFN2 (+ the next LayerNorm) in one launch, h1 through smem (packed only)
                     ops.mlp2_tn(y, self.sh[f"w1{i}"], self.sh[f"w2{i}"], h1, x[i + 1], bias1=self.bias("b1", i),
                                 bias2=self.bias("b2", i), relu1=True, drop1_p=p_drop, drop2_p=p_drop, drop1_stream=11 + 4 * i,
-                                drop2_stream=12 + 4 * i, drop_seed=seed, drop_step=step, residual_is_a=True, row_ids=row_ids,
-                                **nxt)
+                                drop2_stream=12 + 4 * i, drop_seed=seed, drop_step=step, residual_is_a=True,
+                                row_ids=sv.row_ids, **nxt)
                 else:
                     ops.gemm_tn(y, self.sh[f"w1{i}"], out_bf16=h1, bias=self.bias("b1", i), relu=True,
                                 drop_p=p_drop, drop_seed=seed, drop_stream=11 + 4 * i, drop_step=step)
-                    ops.gemm_tn(h1, self.sh[f"w2{i}"], out_bf16=x[i + 1], bias=self.bias("b2", i), residual=y, row_ids=row_ids,
-                                drop_p=p_drop, drop_seed=seed, drop_stream=12 + 4 * i, drop_step=step, **nxt)
+                    ops.gemm_tn(h1, self.sh[f"w2{i}"], out_bf16=x[i + 1], bias=self.bias("b2", i), residual=y,
+                                row_ids=sv.row_ids, drop_p=p_drop, drop_seed=seed, drop_stream=12 + 4 * i, drop_step=step,
+                                **nxt)
             fin_in = x[nb]
-            if s.kind == "SRFR":
+            if s.kind == "SRFR":      # last_conv H -> D (SRFR_model.py:123)
                 ops.gemm_tn(x[nb], self.sh["wc"], out_bf16=ws["c"][:T], bias=self.bias("bc"))
                 fin_in = ws["c"][:T]
             if not last_only:
                 ops.layernorm_fwd(fin_in, P.view("last_layernorm.weight"), P.view("last_layernorm.bias"), LN_EPS,
                                   y_f32=ws["hfin"][:T], stats=ws["stF"][:T], H=s.Dout)
-        if last_only:
+        if last_only:               # the final LayerNorm of each sequence's last position only
             out = ws["hfin"][:B]
-            ops.layernorm_fwd_rows(fin_in, P.view("last_layernorm.weight"), P.view("last_layernorm.bias"), LN_EPS, out,
-                                   plan.last_row, B, s.Dout)
+            if packed:
+                ops.layernorm_fwd_rows(fin_in, P.view("last_layernorm.weight"), P.view("last_layernorm.bias"), LN_EPS, out,
+                                       plan.last_row, B, s.Dout)
+            else:                   # row L - 1 of every sequence: a strided row walk
+                ops.layernorm_fwd(fin_in, P.view("last_layernorm.weight"), P.view("last_layernorm.bias"), LN_EPS, y_f32=out,
+                                  T=B, H=s.Dout, row_stride=L, row_offset=L - 1)
             return out[:, :s.Dout]
         if training if save is None else save:
-            self.saved = dict(seq=seq, aux_ids=aux_ids, B=B, L=L, p_drop=p_drop, seed=seed, step=step,
-                              version=self.fwd_version, plan=plan, hyb=hyb, live=live)
-        return ws["hfin"][:T]
+            self.saved = sv
+        return ws["hfin"][:T] if packed else ws["hfin"][:T].view(B, L, s.Doutp)[..., :s.Dout]
 
-    def _fuse_oproj(self, hyb, L, fuse_ln) -> int:
-        """Bit 0 / 1: the packed attention forward / backward takes the out-projection (tile layout, one head, the
-        fused-LayerNorm width, and the kernel's shared-memory plan fits); otherwise the separate gemm_tn launches."""
-        s = self.spec
-        if hyb is not None or s.num_heads != 1 or not fuse_ln or s.Hp != s.H:
-            return 0
-        return ops.attention_packed_oproj_supported(L, s.H, s.num_heads)
+    def _attention_fwd(self, sv: "_Saved", i: int, q, kv, o, stats, fold: dict) -> None:
+        """o = attention(q, k | v) of block i.  Packed tile layout: the packed kernel, which with `fold` (oproj bit 0) also
+        writes r, y and y's statistics.  Dense layout: the dense kernel.  Hybrid: the dense kernel on dense copies of the
+        packed rows, under the live-tile list when there is one."""
+        s, Hp = self.spec, self.spec.Hp
+        drop = (sv.p_drop, sv.seed, 10 + 4 * i, sv.step)
+        if sv.plan is not None and sv.hyb is None:
+            ops.attention_fwd_packed(q, kv[:, :Hp], kv[:, Hp:], o, sv.plan, sv.L, s.H, s.num_heads, *drop, **fold)
+            return
+        qd, kvd, od = q, kv, o
+        if sv.hyb is not None:
+            Td = sv.B * sv.L
+            qd, kvd, od = sv.hyb[f"qd{i}"][:Td], sv.hyb[f"kvd{i}"][:Td], sv.hyb[f"od{i}"][:Td]
+            ops.unpack_rows([(q, qd, Hp, 0), (kv, kvd, 2 * Hp, 0)], sv.plan)
+        with sv.live.active() if sv.live is not None else nullcontext():
+            ops.attention_fwd(qd, kvd[:, :Hp], kvd[:, Hp:], od, sv.B, sv.L, s.H, s.num_heads, *drop, stats=stats)
+        if sv.hyb is not None:
+            ops.pack_rows([(od, o, Hp, 0)], sv.plan)
 
-    def _backward_packed(self, dh: torch.Tensor) -> None:
-        s, P, sv = self.spec, self.P, self.saved
-        plan, hyb, live = sv["plan"], sv.get("hyb"), sv.get("live")
-        B, L = sv["B"], sv["L"]
-        T, H, Hp, nb = plan.cap, s.H, s.Hp, s.num_blocks
+    # ------------------------------------------------------------------ backward
+    def check_saved(self, version: Optional[int] = None) -> "_Saved":
+        """The record of the forward being back-propagated.  The activations live in the engine's shared workspace, so
+        only the LATEST saving forward can be back-propagated: `version` (the stamp an autograd node took at forward
+        time) is checked against it."""
+        sv = self.saved
+        if sv is None and version is None:
+            raise RuntimeError("backward() without a training forward()")
+        if sv is None or sv.version != self.fwd_version or (version is not None and version != sv.version):
+            raise RuntimeError("srfrd_b200: backward() of a stale forward -- another forward() (training, validation or "
+                               "predict) ran on this model after the one being back-propagated and overwrote the shared "
+                               "activation workspace; run backward() before the next forward()")
+        return sv
+
+    def backward(self, dh: torch.Tensor, version: Optional[int] = None) -> None:
+        """Given dL/dhidden (T, Dout) fp32 -- T rows of the forward's layout -- accumulate every parameter gradient into
+        P.grad (the score kernels have already added the pos/neg rows of the item table).  Every layout decision is the
+        saving forward's (check_saved)."""
+        s, P = self.spec, self.P
+        sv = self.check_saved(version)
+        T, H, Hp, nb = sv.T, s.H, s.Hp, s.num_blocks
         ws = self._ws
-        row_ids = plan.row_ids
-        p_drop, seed, step = sv["p_drop"], sv["seed"], sv["step"]
+        row_ids = sv.row_ids
+        p_drop, seed, step = sv.p_drop, sv.seed, sv.step
         gA, gC, gD, gX = (ws[n][:T] for n in ("gA", "gC", "gD", "gX"))
         G = lambda name: P.view(name, grad=True)
         GM = lambda name: P.mat(name, grad=True)
         x = [ws[f"x{i}"][:T] for i in range(nb + 1)]
         dz_top = ws[f"gdz_{nb - 1}"][:T]
-        fuse_oproj = self._fuse_oproj(hyb, L, Hp <= 128 and os.environ.get("SRFRD_FUSE_LN", "1") != "0") & 2
-        with ops.row_limit(plan.rows):
+        with ops.row_limit(sv.plan.rows) if sv.plan is not None else nullcontext():
+            # final LayerNorm (+ last_conv) -> dz = dL/dx[nb], pad rows zeroed
             if s.kind == "SRFR":
                 gc = ws["gc"][:T]
                 ops.layernorm_bwd(dh, ws["c"][:T], ws["stF"][:T], P.view("last_layernorm.weight"), gc,
@@ -722,61 +602,54 @@ class HotPath:
             else:
                 ops.layernorm_bwd(dh, x[nb], ws["stF"][:T], P.view("last_layernorm.weight"), dz_top,
                                   G("last_layernorm.weight"), G("last_layernorm.bias"), row_ids=row_ids, H=s.Dout)
+
             for i in reversed(range(nb)):
                 Q, q, kv, o, r, y, h1 = (ws[f"{n}{i}"][:T] for n in ("Q", "q", "kv", "o", "r", "y", "h1"))
                 dz, da1, dr, dq, dkv = (ws[f"{n}{i}"][:T] for n in ("gdz_", "gda1_", "gdr_", "gdq_", "gdkv_"))
-                dx_out = ws[f"gdz_{i - 1}"][:T] if i > 0 else gA
+                dx_out = ws[f"gdz_{i - 1}"][:T] if i > 0 else gA          # dL/dx[i]: the next (earlier) block's dz
                 dz2 = dz
-                if p_drop > 0:
+                if p_drop > 0:      # da2 = dz * mask2 (dropout2 sits between conv2 and the residual add)
                     dz2 = ws[f"gE_{i}"][:T]
                     ops.dropout_apply(dz, dz2, Hp, p_drop, seed, 12 + 4 * i, step)
+                # FFN: z = drop2(h1 W2^T + b2) + y ; h1 = relu(drop1(y W1^T + b1))
                 with self._branch():
-                    ops.gemm_wgrad(dz2, h1, GM(f"forward_layers.{i}.conv2.weight"), G(f"forward_layers.{i}.conv2.bias"), Mo=H, No=H)
-                if self.fuse_ffn and Hp <= 128:            # da1 = (dz2 W2) * drop1 * (h1 > 0);  dy = da1 W1 + dz: one launch
+                    ops.gemm_wgrad(dz2, h1, GM(f"forward_layers.{i}.conv2.weight"), G(f"forward_layers.{i}.conv2.bias"),
+                                   Mo=H, No=H)
+                if sv.mlp2:                 # da1 = (dz2 W2) * drop1 * (h1 > 0);  dy = da1 W1 + dz: one launch
                     ops.mlp2_tn(dz2, self.sh[f"w2T{i}"], self.sh[f"w1T{i}"], da1, gC, gate=h1, drop1_p=p_drop,
                                 drop1_stream=11 + 4 * i, drop_seed=seed, drop_step=step, residual=dz)
-                    with self._branch():
-                        ops.gemm_wgrad(da1, y, GM(f"forward_layers.{i}.conv1.weight"), G(f"forward_layers.{i}.conv1.bias"),
-                                       Mo=H, No=H)
                 else:
                     ops.gemm_tn(dz2, self.sh[f"w2T{i}"], out_bf16=da1, gate=h1, drop_p=p_drop, drop_seed=seed,
-                                drop_stream=11 + 4 * i, drop_step=step)
-                    with self._branch():
-                        ops.gemm_wgrad(da1, y, GM(f"forward_layers.{i}.conv1.weight"), G(f"forward_layers.{i}.conv1.bias"),
-                                       Mo=H, No=H)
-                    ops.gemm_tn(da1, self.sh[f"w1T{i}"], out_bf16=gC, residual=dz)
+                                drop_stream=11 + 4 * i, drop_step=step)                               # da1
+                with self._branch():
+                    ops.gemm_wgrad(da1, y, GM(f"forward_layers.{i}.conv1.weight"), G(f"forward_layers.{i}.conv1.bias"),
+                                   Mo=H, No=H)
+                if not sv.mlp2:
+                    ops.gemm_tn(da1, self.sh[f"w1T{i}"], out_bf16=gC, residual=dz)                     # dy
+                # LN2
                 ops.layernorm_bwd(gC, r, ws[f"st2_{i}"][:T], P.view(f"forward_layernorms.{i}.weight"), dr,
-                                  G(f"forward_layernorms.{i}.weight"), G(f"forward_layernorms.{i}.bias"), H=H)
+                                  G(f"forward_layernorms.{i}.weight"), G(f"forward_layernorms.{i}.bias"), H=H)   # dr
+                # r = Q + o Wo^T + bo
                 with self._branch():
                     ops.gemm_wgrad(dr, o, GM(f"attention_layers.{i}.out_proj.weight"),
                                    G(f"attention_layers.{i}.out_proj.bias"), Mo=H, No=H)
-                if not fuse_oproj:
-                    ops.gemm_tn(dr, self.sh[f"woT{i}"], out_bf16=gC)
-                if fuse_oproj:              # dO = dr Wo inside the attention kernel
-                    ops.attention_bwd_packed(None, q, kv[:, :Hp], kv[:, Hp:], dq, dkv[:, :Hp], dkv[:, Hp:], plan, L, H,
-                                             s.num_heads, p_drop, seed, 10 + 4 * i, step, dr=dr, woT=self.sh[f"woT{i}"])
-                elif hyb is None:
-                    ops.attention_bwd_packed(gC, q, kv[:, :Hp], kv[:, Hp:], dq, dkv[:, :Hp], dkv[:, Hp:], plan, L, H,
-                                             s.num_heads, p_drop, seed, 10 + 4 * i, step)
-                else:
-                    Td = B * L
-                    qd, kvd, od = hyb[f"qd{i}"][:Td], hyb[f"kvd{i}"][:Td], hyb[f"od{i}"][:Td]
-                    dod, dqd, dkvd = hyb["dod"][:Td], hyb["dqd"][:Td], hyb["dkvd"][:Td]
-                    ops.unpack_rows([(gC, dod, Hp, 1)], plan)                  # a pad query's output is dead: dO = 0
-                    with (live.active() if live is not None else nullcontext()):
-                        ops.attention_bwd(dod, qd, kvd[:, :Hp], kvd[:, Hp:], dqd, dkvd[:, :Hp], dkvd[:, Hp:], B, L, H,
-                                          s.num_heads, p_drop, seed, 10 + 4 * i, step, o=od, stats=ws.get(f"ast{i}"))
-                    # dk, dv of the pad representative = the sum over its sequence's pad slots (every copy of the pad key)
-                    ops.pack_rows([(dqd, dq, Hp, 0), (dkvd, dkv, 2 * Hp, 1)], plan)
+                if not sv.oproj & 2:        # otherwise dO = dr Wo inside the attention kernel
+                    ops.gemm_tn(dr, self.sh[f"woT{i}"], out_bf16=gC)                                   # do
+                self._attention_bwd(sv, i, gC, q, kv, o, dq, dkv, dr, ws.get(f"ast{i}"))               # dq, dk|dv
                 gin = GM(f"attention_layers.{i}.in_proj_weight")
                 gbin = G(f"attention_layers.{i}.in_proj_bias")
                 with self._branch():
                     ops.gemm_wgrad(dq, Q, gin[:H], gbin[:H], Mo=H, No=H)
-                    ops.gemm_wgrad(dkv, x[i], gin[H:], gbin[H:], Mo=2 * H, No=H)
-                with self._branch(second=True):                        # dx through k | v: independent of dQ
-                    ops.gemm_tn(dkv, self.sh[f"wkvT{i}"], out_bf16=gX)
-                ops.gemm_tn(dq, self.sh[f"wqT{i}"], out_bf16=gD, residual=dr)
+                    if Hp == H:
+                        ops.gemm_wgrad(dkv, x[i], gin[H:], gbin[H:], Mo=2 * H, No=H)
+                    else:   # k and v gradients sit at column offsets 0 and Hp: two row blocks of in_proj_weight
+                        ops.gemm_wgrad(dkv[:, :Hp], x[i], gin[H:2 * H], gbin[H:2 * H], Mo=H, No=H)
+                        ops.gemm_wgrad(dkv[:, Hp:], x[i], gin[2 * H:], gbin[2 * H:], Mo=H, No=H)
+                with self._branch(second=True):                                                        # independent of dQ
+                    ops.gemm_tn(dkv, self.sh[f"wkvT{i}"], out_bf16=gX)                                 # dx via k, v
+                ops.gemm_tn(dq, self.sh[f"wqT{i}"], out_bf16=gD, residual=dr)                          # dQ = dr + dq Wq
                 self._join(second=True)
+                # LN1 + the un-normalised k/v path; pad rows zeroed (x_i was masked, SRFR_model.py:99,121)
                 ops.layernorm_bwd(gD, x[i], ws[f"st1_{i}"][:T], P.view(f"attention_layernorms.{i}.weight"), dx_out,
                                   G(f"attention_layernorms.{i}.weight"), G(f"attention_layernorms.{i}.bias"),
                                   add=gX, row_ids=row_ids, H=H)
@@ -784,11 +657,46 @@ class HotPath:
             if s.kind == "SASRec" and p_drop > 0:
                 ops.dropout_apply(gA, gC, H, p_drop, seed, 1, step)
                 dx0 = gC
+
+        # embedding tables
         aux_grad = G(s.aux_key) if s.aux_key else None
-        ops.embed_bwd_packed(dx0, sv["seq"], sv["aux_ids"], plan, s.D, s.F if s.mode == 1 else 0, s.mode, s.item_scale,
-                             G(s.item_key), aux_grad, G(s.pos_key))
-        self._join()
+        F = s.F if s.mode == 1 else 0
+        if sv.plan is not None:
+            ops.embed_bwd_packed(dx0, sv.seq, sv.aux_ids, sv.plan, s.D, F, s.mode, s.item_scale, G(s.item_key), aux_grad,
+                                 G(s.pos_key))
+        else:
+            ops.embed_bwd(dx0, sv.seq, sv.aux_ids, s.D, F, s.mode, s.item_scale, G(s.item_key), aux_grad)
+            LH = sv.L * Hp
+            pos_tmp = ws["pos_tmp"][:LH]      # zero on entry: allocated zeroed, and add_segments consumes (re-zeroes) it
+            ops.colsum(dx0, pos_tmp, M=sv.B, N=LH, ld=LH)
+            ops.add_segments(pos_tmp, LH, Hp, s.D, G(s.pos_key))
+        self._join()                                # every weight gradient has landed in P.grad
         self.saved = None
+
+    def _attention_bwd(self, sv: "_Saved", i: int, do, q, kv, o, dq, dkv, dr, stats) -> None:
+        """dq, dk | dv of block i's attention from dO = `do`.  Packed tile layout: the packed kernel, which with oproj
+        bit 1 computes dO = dr Wo itself.  Dense layout: the dense kernel.  Hybrid: the dense kernel on dense copies,
+        under the live-tile list when there is one."""
+        s, Hp = self.spec, self.spec.Hp
+        drop = (sv.p_drop, sv.seed, 10 + 4 * i, sv.step)
+        if sv.plan is not None and sv.hyb is None:
+            fold = dict(dr=dr, woT=self.sh[f"woT{i}"]) if sv.oproj & 2 else {}
+            ops.attention_bwd_packed(None if fold else do, q, kv[:, :Hp], kv[:, Hp:], dq, dkv[:, :Hp], dkv[:, Hp:], sv.plan,
+                                     sv.L, s.H, s.num_heads, *drop, **fold)
+            return
+        dqd, dkvd = dq, dkv
+        if sv.hyb is not None:
+            Td, hyb = sv.B * sv.L, sv.hyb
+            q, kv, o = hyb[f"qd{i}"][:Td], hyb[f"kvd{i}"][:Td], hyb[f"od{i}"][:Td]
+            dod, dqd, dkvd = hyb["dod"][:Td], hyb["dqd"][:Td], hyb["dkvd"][:Td]
+            ops.unpack_rows([(do, dod, Hp, 1)], sv.plan)                   # a pad query's output is dead: dO = 0
+            do = dod
+        with sv.live.active() if sv.live is not None else nullcontext():
+            ops.attention_bwd(do, q, kv[:, :Hp], kv[:, Hp:], dqd, dkvd[:, :Hp], dkvd[:, Hp:], sv.B, sv.L, s.H, s.num_heads,
+                              *drop, o=o, stats=stats)
+        if sv.hyb is not None:
+            # dk, dv of the pad representative = the sum over its sequence's pad slots (every copy of the pad key)
+            ops.pack_rows([(dqd, dq, Hp, 0), (dkvd, dkv, 2 * Hp, 1)], sv.plan)
 
     # ------------------------------------------------------------------ scoring helpers
     def fake_table(self) -> Optional[torch.Tensor]:

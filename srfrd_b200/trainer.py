@@ -233,7 +233,6 @@ class FusedTrainer:
         """The kernel sequence of one step, on static buffers (captured once, replayed forever)."""
         st, eng, P, s = self._static, self.eng, self.P, self.spec
         B, L = st["seq"].shape
-        T = B * L
         pos, neg = st["pos"].view(-1), st["neg"].view(-1)
         w_pos = st["w_pos"].view(-1) if has_wp else None
         w_neg = st["w_neg"].view(-1) if has_wn else None
@@ -263,25 +262,20 @@ class FusedTrainer:
         torch.cuda.current_stream().wait_stream(self.comm)
         prs_ = st["prs"].view(-1) if ft is not None else None
         nrs_ = st["nrs"].view(-1) if ft is not None else None
+        rows, plan = eng.saved.T, eng.saved.plan          # the forward's activation rows (B * L, or packed) and plan
         if self.loss_kind == "ce":
-            plan = eng.saved["plan"] if packed else None
-            rows = plan.cap if packed else T
             ce = self._ce_buffers(rows)
             hb, lse, table = ce["h"][:rows], ce["lse"][:rows], eng.sh["ce_table"]
             ops.f32_to_bf16_split(ws["hfin"][:rows], hb)
             ops.catalogue_ce_fwd(hb, table, pos, w_pos, lse, acc, plan)
             ops.catalogue_ce_bwd(hb, table, pos, w_pos, norm, lse, ws["dh"][:rows], P.view(s.item_key, grad=True), s.D, plan)
-            eng.backward(ws["dh"][:rows])
-        elif packed:
-            plan = eng.saved["plan"]
-            Tp = plan.cap
-            ops.score_loss_fused_packed(ws["hfin"][:Tp], P.view(s.item_key), ft, pos, neg, prs_, nrs_, w_pos, w_neg, norm, acc,
-                                        ws["dh"][:Tp], P.view(s.item_key, grad=True), eng.fake_table_grad(), plan)
-            eng.backward(ws["dh"][:Tp])
+        elif plan is not None:
+            ops.score_loss_fused_packed(ws["hfin"][:rows], P.view(s.item_key), ft, pos, neg, prs_, nrs_, w_pos, w_neg, norm,
+                                        acc, ws["dh"][:rows], P.view(s.item_key, grad=True), eng.fake_table_grad(), plan)
         else:
-            ops.score_loss_fused(ws["hfin"][:T], P.view(s.item_key), ft, pos, neg, prs_, nrs_, w_pos, w_neg, norm, acc,
-                                 ws["dh"][:T], P.view(s.item_key, grad=True), eng.fake_table_grad())
-            eng.backward(ws["dh"][:T])
+            ops.score_loss_fused(ws["hfin"][:rows], P.view(s.item_key), ft, pos, neg, prs_, nrs_, w_pos, w_neg, norm, acc,
+                                 ws["dh"][:rows], P.view(s.item_key, grad=True), eng.fake_table_grad())
+        eng.backward(ws["dh"][:rows])
         if self._dp is not None:
             # reduce-scatter -> Adam on this rank's slice -> all-gather of the new parameters + loss, one kernel over NVLink
             # peer memory (csrc/dp_adam.cu) instead of an NCCL all-reduce followed by the same Adam on every rank
