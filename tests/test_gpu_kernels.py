@@ -250,34 +250,59 @@ def _attn_ref(q, k, v, heads):
     return O.attention(q, k, v, heads)
 
 
-@pytest.mark.parametrize("B,L,H,heads", [(3, 12, 32, 1), (5, 50, 80, 1), (2, 50, 80, 2), (2, 200, 272, 1), (4, 7, 16, 4),
-                                         (64, 50, 64, 1), (7, 50, 64, 2), (3, 128, 64, 1), (5, 100, 128, 1),
-                                         (300, 50, 80, 1), (9, 33, 96, 3), (2, 240, 32, 1),
-                                         # 128 < maxlen <= 256: two query tiles per sequence, FlashAttention-2 style backward
-                                         (3, 129, 64, 1), (2, 256, 128, 2), (5, 200, 80, 1), (160, 200, 272, 1), (3, 150, 96, 2)])
-def test_attention_fwd_bwd(ops, B, L, H, heads):
+def _attn_ref_dropout(q, k, v, heads, factor):
+    """fp64 causal attention whose probabilities are multiplied by the dropout factors (B, heads, L, L) after the
+    softmax, as every attention kernel does (F.dropout on the attention weights, SRFR_model.py:112)."""
+    B, L, H = q.shape
+    hd = H // heads
+    split = lambda x: x.view(B, L, heads, hd).transpose(1, 2)
+    s = split(q) @ split(k).transpose(-1, -2) / math.sqrt(hd)
+    s = s.masked_fill(~torch.ones(L, L, dtype=torch.bool).tril(), float("-inf"))
+    return ((torch.softmax(s, -1) * factor) @ split(v)).transpose(1, 2).reshape(B, L, H)
+
+
+_ATTN_CASES = [(3, 12, 32, 1), (5, 50, 80, 1), (2, 50, 80, 2), (2, 200, 272, 1), (4, 7, 16, 4), (64, 50, 64, 1), (7, 50, 64, 2),
+               (3, 128, 64, 1), (5, 100, 128, 1), (300, 50, 80, 1), (9, 33, 96, 3), (2, 240, 32, 1),
+               # 128 < maxlen <= 256: two query tiles per sequence, FlashAttention-2 style backward
+               (3, 129, 64, 1), (2, 256, 128, 2), (5, 200, 80, 1), (160, 200, 272, 1), (3, 150, 96, 2)]
+# dropout p = 0.3 with two heads on each kernel: SIMT (head width 20), the tile kernel (L <= 128), the long kernel (L > 128)
+_ATTN_DROP = [(6, 20, 40, 2), (7, 50, 128, 2), (3, 150, 128, 2)]
+
+
+@pytest.mark.parametrize("B,L,H,heads,drop", [c + (0.0,) for c in _ATTN_CASES] + [c + (0.3,) for c in _ATTN_DROP],
+                         ids=["-".join(map(str, c)) for c in _ATTN_CASES] + ["-".join(map(str, c)) + "-drop0.3" for c in _ATTN_DROP])
+def test_attention_fwd_bwd(ops, B, L, H, heads, drop):
+    from tests.test_dropout_mask import keep_mask, masked
     T = B * L
     q, kv = rnd((T, H), 30, 0.7, bf16), rnd((T, 2 * H), 31, 0.7, bf16)
     o = torch.empty(T, H, dtype=bf16, device="cuda")
     stats = torch.zeros(T * heads, 4, device="cuda") if L > 128 else None
-    ops.attention_fwd(q, kv[:, :H], kv[:, H:], o, B, L, H, heads, stats=stats)
-    qr = q.float().cpu().view(B, L, H).requires_grad_(True)
-    kr = kv[:, :H].float().cpu().view(B, L, H).requires_grad_(True)
-    vr = kv[:, H:].float().cpu().view(B, L, H).requires_grad_(True)
-    ref = _attn_ref(qr, kr, vr, heads)
-    torch.testing.assert_close(o.float().cpu().view(B, L, H), ref.detach(), rtol=2e-2, atol=1e-2)   # bf16 output
+    seed, stream, step = 2024, 6, 3.0
+    dkw = dict(drop_p=drop, seed=seed, stream_id=stream, drop_step=torch.tensor([step], device="cuda")) if drop else {}
+    ops.attention_fwd(q, kv[:, :H], kv[:, H:], o, B, L, H, heads, stats=stats, **dkw)
+    dt = torch.float64 if drop else torch.float32
+    qr = q.to(dt).cpu().view(B, L, H).requires_grad_(True)
+    kr = kv[:, :H].to(dt).cpu().view(B, L, H).requires_grad_(True)
+    vr = kv[:, H:].to(dt).cpu().view(B, L, H).requires_grad_(True)
+    if drop:
+        # dense kernels hash element ((b * heads + h) * L + query) * L + key
+        keep = keep_mask(seed, stream, np.arange(B * heads * L * L).reshape(B, heads, L, L), drop, step)
+        ref = _attn_ref_dropout(qr, kr, vr, heads, masked(torch.ones(keep.shape), keep, drop).double())
+    else:
+        ref = _attn_ref(qr, kr, vr, heads)
+    torch.testing.assert_close(o.to(dt).cpu().view(B, L, H), ref.detach(), rtol=2e-2, atol=1e-2)   # bf16 output
     ntri = (L * (L + 1) // 2 + 3) // 4 * 4      # SIMT path (no stats given): packed causal triangles of P and dS in smem
     if L > 128 and 2 * ntri * 4 + 4 * L * 34 > 227 * 1024:
         with pytest.raises(RuntimeError, match="shared memory"):
             ops.attention_bwd(o, q, kv[:, :H], kv[:, H:], o, kv[:, :H], kv[:, H:], B, L, H, heads)
     do = rnd((T, H), 32, dtype=bf16)
-    ref.backward(do.float().cpu().view(B, L, H))
+    ref.backward(do.to(dt).cpu().view(B, L, H))
     dq = torch.empty(T, H, dtype=bf16, device="cuda")
     dkv = torch.empty(T, 2 * H, dtype=bf16, device="cuda")
-    ops.attention_bwd(do, q, kv[:, :H], kv[:, H:], dq, dkv[:, :H], dkv[:, H:], B, L, H, heads, o=o, stats=stats)
+    ops.attention_bwd(do, q, kv[:, :H], kv[:, H:], dq, dkv[:, :H], dkv[:, H:], B, L, H, heads, o=o, stats=stats, **dkw)
     for got, want in ((dq, qr.grad), (dkv[:, :H], kr.grad), (dkv[:, H:], vr.grad)):
         w = want.view(T, H)
-        torch.testing.assert_close(got.float().cpu(), w, rtol=3e-2, atol=2e-2 * float(w.abs().max()))
+        torch.testing.assert_close(got.to(dt).cpu(), w, rtol=3e-2, atol=2e-2 * float(w.abs().max()))
 
 
 def test_attention_dropout_is_consistent(ops):
