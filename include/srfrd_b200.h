@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define SRFRD_ABI_VERSION 10
+#define SRFRD_ABI_VERSION 11
 #if defined(__GNUC__)
 #define SRFRD_API __attribute__((visibility("default")))
 #else
@@ -283,6 +283,36 @@ SRFRD_API int srfrd_catalogue_ce_bwd(const void* h_bf16, int ldh, const void* ta
                                      int D, const int64_t* pos, const float* w_pos, const float* norm, const int* row_tok,
                                      const int* rows_dev, int64_t cap_rows, const float* lse, float* dh, int lddh,
                                      float* d_item, int ldd, void* stream);
+
+/* ---- gSASRec's gBCE over k negatives shared by every row of a step (opt-in training objective) ----
+ * alpha = k / (N - 1), beta = 1 - t (1 - alpha) (the caller passes beta); z_r = <h_r, E[pos_r]>, s_rj = <h_r, E[n_j]>;
+ * m_rj = 0 when n_j occurs in row r's sequence, else 1; W = norm[0] = sum_r w_r;
+ * loss = (sum_r w_r beta softplus(-z_r) + sum_r w_r sum_j m_rj softplus(s_rj)) / W -- gSASRec's loss times (k + 1).
+ * Operands bf16, accumulation fp32.  Rows, weights and row maps as for srfrd_catalogue_ce_fwd.
+ * srfrd_gbce_plan: host only; the padded negative rows Kp (k rounded up to 128), the row splits of the dN pass (its
+ * workspace is n_split x Kp x Dp fp32), the shared-memory bytes and ring stages; refuses k outside 1..256 and a Dp the
+ * kernels cannot serve (any output pointer may be NULL). */
+SRFRD_API int srfrd_gbce_plan(int k, int Dp, int64_t cap_rows, int* neg_rows, int* n_split, int64_t* smem_bytes,
+                              int* ring_stages);
+/* draw = 1: neg_ids[j] = 1 + hash(seed, step[0], j) mod n_items for j < k (step: the device step counter, or NULL), so a
+ * captured graph draws new negatives on every replay; draw = 0: neg_ids is read (ids in 1..n_items).  Writes neg_bf16
+ * (Kp, Dp) bf16 = the fp32 item rows of the negatives, zero past k and past D, and, for each of n_seq sequences, the
+ * exclusion words excl (n_seq, ceil(k / 32)) uint32: bit j % 32 of word j / 32 is set when n_j is one of the sequence's
+ * len_a ids in ex_a (n_seq, len_a) or len_b ids in ex_b (n_seq, len_b) (either may be empty). */
+SRFRD_API int srfrd_gbce_draw(const float* item, int ldi, int64_t n_items, int D, int Dp, int k, uint64_t seed,
+                              const float* step, int draw, int64_t* neg_ids, void* neg_bf16, const int64_t* ex_a, int len_a,
+                              const int64_t* ex_b, int len_b, int64_t n_seq, uint32_t* excl, void* stream);
+/* The loss and both gradients in one call.  loss_acc[0] += the positive terms, loss_acc[1] += the negative terms
+ * (unnormalised: the Adam read-out divides by norm[0] and norm[1]); dh (rows r < rows, first D columns) is written (zero
+ * rows for rows without a loss term).  d_item (nullable, (n_items + 1, ldd) fp32) gains dz_r h_r at each positive
+ * (red.add) and the negatives' gradient sum_r ds_rj h_r at each n_j: per-split partials in `part` summed in a fixed order,
+ * duplicates summed, d_item[0] untouched.  excl (nullable = no exclusion) is srfrd_gbce_draw's, with row r's sequence
+ * = its dense token / L. */
+SRFRD_API int srfrd_gbce_loss(const void* h_bf16, int ldh, const void* neg_bf16, const int64_t* neg_ids, int k, int Dp,
+                              int D, const float* item, int ldi, int64_t n_items, const int64_t* pos, const float* w_pos,
+                              const float* norm, const uint32_t* excl, int L, const int* row_tok, const int* rows_dev,
+                              int64_t cap_rows, float beta, float* loss_acc, float* dh, int lddh, float* d_item, int ldd,
+                              float* part, void* stream);
 
 /* ---- on-device batch sampler (next row 8f #1) ----
  * replaces: WarpSampler_fr / sample_function_fr (utils.py:14-90) and the seven LongTensor.to(device) copies per

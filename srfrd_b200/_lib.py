@@ -89,6 +89,10 @@ SIGNATURES = {
     "srfrd_catalogue_ce_plan": [i32, C.POINTER(i64), C.POINTER(i32), C.POINTER(i32)],
     "srfrd_catalogue_ce_fwd": [vp, i32, vp, i32, i64, i32, vp, vp, vp, vp, i64, vp, vp, vp],
     "srfrd_catalogue_ce_bwd": [vp, i32, vp, i32, i64, i32, i32, vp, vp, vp, vp, vp, i64, vp, vp, i32, vp, i32, vp],
+    "srfrd_gbce_plan": [i32, i32, i64, C.POINTER(i32), C.POINTER(i32), C.POINTER(i64), C.POINTER(i32)],
+    "srfrd_gbce_draw": [vp, i32, i64, i32, i32, i32, u64, vp, i32, vp, vp, vp, i32, vp, i32, i64, vp, vp],
+    "srfrd_gbce_loss": [vp, i32, vp, vp, i32, i32, i32, vp, i32, i64, vp, vp, vp, vp, i32, vp, vp, i64, f32, vp, vp, i32, vp,
+                        i32, vp, vp],
     "srfrd_attention_live_items": [vp, i64, i32, i32, vp, vp, vp, vp],
     "srfrd_set_attention_live": [vp, vp, vp, vp],
     "srfrd_merge_topk": [vp, vp, i64, i32, i32, vp, vp, vp],
@@ -136,7 +140,7 @@ def load() -> C.CDLL:
         fn = getattr(lib, name)            # AttributeError if the symbol is not exported
         fn.argtypes = argtypes
         fn.restype = C.c_int
-    if lib.srfrd_abi_version() != 10:
+    if lib.srfrd_abi_version() != 11:
         raise RuntimeError("srfrd_b200: ABI version mismatch between _lib.py and the built library")
     _lib = lib
     return lib

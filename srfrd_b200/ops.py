@@ -532,3 +532,42 @@ def catalogue_ce_bwd(h, table, pos, w_pos, norm, lse, dh, d_item, D, plan: Optio
     call("srfrd_catalogue_ce_bwd", _p(h), h.stride(0), _p(table), table.stride(0), table.shape[0] - 1, table.shape[1],
          int(D), _p(pos), _p(w_pos), _p(norm), _p(row_tok), _p(rows), cap, _p(lse), _p(dh),
          0 if dh is None else dh.stride(0), _p(d_item), 0 if d_item is None else d_item.stride(0), _stream())
+
+
+def gbce_plan(k: int, Dp: int, cap_rows: int):
+    """(Kp, n_split, shared-memory bytes, ring stages) of the gBCE kernels for k negatives, padded width Dp and an h
+    buffer of cap_rows rows (host only); the dN workspace is (n_split, Kp, Dp) fp32.  Raises for k outside 1..256 or a
+    Dp they cannot serve."""
+    kp, ns, stages, smem = C.c_int(0), C.c_int(0), C.c_int(0), C.c_int64(0)
+    call("srfrd_gbce_plan", int(k), int(Dp), int(cap_rows), C.byref(kp), C.byref(ns), C.byref(smem), C.byref(stages))
+    return int(kp.value), int(ns.value), int(smem.value), int(stages.value)
+
+
+def gbce_draw(item_table, neg_ids, neg_bf16, excl, ex_a=None, ex_b=None, seed: int = 0, step=None, draw: bool = True):
+    """Draw (draw=True; step = device counter mixed into the seed) or take (draw=False) the k = neg_ids.numel()
+    negatives, gather their fp32 rows into neg_bf16 (Kp, Dp) and build the exclusion words excl (n_seq, ceil(k / 32))
+    of the (n_seq, *) int64 id arrays ex_a / ex_b."""
+    _lib.require_device()
+    _chk(item_table, torch.float32, "item_table"); _chk(neg_ids, torch.int64, "neg_ids"); _chk(neg_bf16, bf16, "neg_bf16")
+    ex = ex_a if ex_a is not None else ex_b
+    n_seq = 0 if ex is None else ex.shape[0]
+    la = 0 if ex_a is None else ex_a.shape[1]
+    lb = 0 if ex_b is None else ex_b.shape[1]
+    call("srfrd_gbce_draw", _p(item_table), item_table.stride(0), item_table.shape[0] - 1, item_table.shape[1],
+         neg_bf16.shape[1], neg_ids.numel(), int(seed) & 0xFFFFFFFFFFFFFFFF, _p(step), int(draw), _p(neg_ids), _p(neg_bf16),
+         _p(ex_a), la, _p(ex_b), lb, n_seq, _p(excl), _stream())
+
+
+def gbce_loss(h, neg_bf16, neg_ids, item_table, pos, w_pos, norm, excl, L, beta, loss_acc, dh, d_item, part,
+              plan: Optional[PackedPlan] = None):
+    """The gBCE loss and both gradients: loss_acc[0] / [1] += the positive / negative terms, dh written (first D columns
+    of the rows), d_item ((N + 1, D) fp32, or None) added to.  h (rows, Dp) bf16; pos / w_pos indexed by dense token,
+    whose sequence is token // L; part: the (n_split, Kp, Dp) fp32 workspace of gbce_plan."""
+    _lib.require_device()
+    _chk(h, bf16, "h"); _chk(neg_bf16, bf16, "neg_bf16"); _chk(pos, torch.int64, "pos")
+    _chk(item_table, torch.float32, "item_table")
+    row_tok, rows, cap = _ce_rows(h, plan)
+    call("srfrd_gbce_loss", _p(h), h.stride(0), _p(neg_bf16), _p(neg_ids), neg_ids.numel(), neg_bf16.shape[1],
+         item_table.shape[1], _p(item_table), item_table.stride(0), item_table.shape[0] - 1, _p(pos), _p(w_pos), _p(norm),
+         _p(excl), int(L), _p(row_tok), _p(rows), cap, float(beta), _p(loss_acc), _p(dh), dh.stride(0), _p(d_item),
+         0 if d_item is None else d_item.stride(0), _p(part), _stream())

@@ -19,7 +19,7 @@ import torch
 
 from . import ops, parallel
 from .engine import HotPath
-from .losses import check_ce_width
+from .losses import check_ce_width, check_gbce, gbce_beta
 
 __all__ = ["simulate", "FusedTrainer", "DeviceSampler", "discriminator_weights"]
 
@@ -104,17 +104,31 @@ class FusedTrainer:
                    computed by the tcgen05 kernels of csrc/catalogue_ce.cu without materialising the logits.  The sampled
                    negatives are unused and w_neg is refused; SRFRN is refused (its logits need a fake label per candidate,
                    SRFR_model.py:225-233, which unobserved items do not have).
+                   "gbce" -- gSASRec's gBCE (losses.sampled_gbce) over num_negatives (k, default 256) item ids drawn
+                   uniformly on the device each step from (the engine's seed, the device step counter) and shared by
+                   every position of the batch, with calibration gbce_t (t, default 0.75; t = 0 is BCE with k negatives).
+                   A negative that occurs in a position's sequence (its seq or pos ids) is left out of that position's
+                   loss.  Same discriminator weights and normaliser as the BCE; the kernels are csrc/gbce.cu.  Every
+                   data-parallel rank draws the same negatives.  w_neg and SRFRN are refused as for "ce".
     """
 
     def __init__(self, model, lr: float = 1e-3, betas=(0.9, 0.98), eps: float = 1e-8, process_group=None,
-                 use_graph: bool = True, l2_emb: float = 0.0, packed: Optional[bool] = None, loss: str = "bce"):
-        if loss not in ("bce", "ce"):
-            raise ValueError(f"unknown loss {loss!r} (expected 'bce' or 'ce')")
+                 use_graph: bool = True, l2_emb: float = 0.0, packed: Optional[bool] = None, loss: str = "bce",
+                 num_negatives: Optional[int] = None, gbce_t: Optional[float] = None):
+        if loss not in ("bce", "ce", "gbce"):
+            raise ValueError(f"unknown loss {loss!r} (expected 'bce', 'ce' or 'gbce')")
+        if loss != "gbce" and (num_negatives is not None or gbce_t is not None):
+            raise ValueError(f"num_negatives / gbce_t configure loss='gbce', not loss={loss!r}")
+        if loss in ("ce", "gbce") and model.spec.kind == "SRFRN":
+            raise ValueError(f"loss={loss!r} does not support SRFRN: its logits need each candidate's fake label "
+                             "(SRFR_model.py:225-233), which unobserved items do not have")
         if loss == "ce":
-            if model.spec.kind == "SRFRN":
-                raise ValueError("loss='ce' does not support SRFRN: its logits need each candidate's fake label "
-                                 "(SRFR_model.py:225-233), which unobserved items do not have")
             check_ce_width(model.spec.D)
+        if loss == "gbce":
+            self.num_negatives = 256 if num_negatives is None else num_negatives
+            self.gbce_t = 0.75 if gbce_t is None else gbce_t
+            n_items = dict(model.named_parameters())[model.spec.item_key].shape[0] - 1
+            check_gbce(self.num_negatives, self.gbce_t, n_items, model.spec.D)
         self.loss_kind = loss
         self.model = model
         self._dp = None
@@ -142,6 +156,7 @@ class FusedTrainer:
         self.l2_emb = float(l2_emb)
         self._l2 = self._setup_l2(model) if self.l2_emb != 0.0 else None
         self._ce_ws: Optional[Dict[str, torch.Tensor]] = None
+        self._gbce_ws: Optional[Dict[str, torch.Tensor]] = None
         if loss == "ce":
             self.eng.enable_ce_table()
         self.P.grad_bucket.zero_()
@@ -158,9 +173,27 @@ class FusedTrainer:
             self.eng.ws_generation += 1
         return self._ce_ws
 
+    def _gbce_buffers(self, rows: int, B: int) -> Dict[str, torch.Tensor]:
+        """loss="gbce": the bf16 final hidden rows, the drawn ids, their bf16 rows, the exclusion words of the batch's
+        sequences and the dN pass's partials; re-allocated (bumping the workspace generation) when a batch needs more."""
+        ws = self._gbce_ws
+        if ws is None or ws["h"].shape[0] < rows or ws["excl"].shape[0] < B:
+            dev, Dp, k = self.eng.device, self.spec.Dp, self.num_negatives
+            rows = max(rows, 0 if ws is None else ws["h"].shape[0])
+            B = max(B, 0 if ws is None else ws["excl"].shape[0])
+            Kp, n_split, _, _ = ops.gbce_plan(k, Dp, rows)
+            self._gbce_ws = ws = dict(
+                h=torch.zeros(rows, Dp, dtype=torch.bfloat16, device=dev),
+                ids=torch.zeros(k, dtype=torch.int64, device=dev),
+                nb=torch.zeros(Kp, Dp, dtype=torch.bfloat16, device=dev),
+                excl=torch.zeros(B, (k + 31) // 32, dtype=torch.int32, device=dev),
+                part=torch.zeros(n_split * Kp * Dp, dtype=torch.float32, device=dev))
+            self.eng.ws_generation += 1
+        return ws
+
     def _refuse_w_neg(self, w_neg):
-        if w_neg is not None and self.loss_kind == "ce":
-            raise ValueError("w_neg weights the sampled negatives of the BCE; loss='ce' has no negatives")
+        if w_neg is not None and self.loss_kind in ("ce", "gbce"):
+            raise ValueError(f"w_neg weights the sampled negative of the BCE; loss={self.loss_kind!r} does not take it")
 
     def _setup_l2(self, model) -> ops.ParamL2:
         """The regulariser's segment table: every tensor of model.parameters() is one segment of the flat buffer."""
@@ -269,6 +302,16 @@ class FusedTrainer:
             ops.f32_to_bf16_split(ws["hfin"][:rows], hb)
             ops.catalogue_ce_fwd(hb, table, pos, w_pos, lse, acc, plan)
             ops.catalogue_ce_bwd(hb, table, pos, w_pos, norm, lse, ws["dh"][:rows], P.view(s.item_key, grad=True), s.D, plan)
+        elif self.loss_kind == "gbce":
+            gb = self._gbce_buffers(rows, B)
+            hb, E = gb["h"][:rows], P.view(s.item_key)
+            ops.f32_to_bf16_split(ws["hfin"][:rows], hb)
+            # the same (seed, step) on every data-parallel rank: every rank draws the same negatives
+            ops.gbce_draw(E, gb["ids"], gb["nb"], gb["excl"][:B], st["seq"], st["pos"], seed=eng.drop_seed,
+                          step=eng.step_state[3:4])
+            ops.gbce_loss(hb, gb["nb"], gb["ids"], E, pos, w_pos, norm, gb["excl"], L,
+                          gbce_beta(self.num_negatives, E.shape[0] - 1, self.gbce_t), acc, ws["dh"][:rows],
+                          P.view(s.item_key, grad=True), gb["part"], plan)
         elif plan is not None:
             ops.score_loss_fused_packed(ws["hfin"][:rows], P.view(s.item_key), ft, pos, neg, prs_, nrs_, w_pos, w_neg, norm,
                                         acc, ws["dh"][:rows], P.view(s.item_key, grad=True), eng.fake_table_grad(), plan)

@@ -2,7 +2,9 @@
 and row-sharded catalogue top-10 (NCCL all-gather + merge) == unsharded top-10.
 `--l2 X` trains both with l2_emb = X (the regulariser's gradient is added once, after the reduction over ranks).
 `--topk-k K` checks the sharded top-K (1 <= K <= 64) instead of the top-10.
-`--loss ce` trains both with the full-catalogue cross-entropy (FusedTrainer(loss="ce")) instead of the BCE."""
+`--loss ce` trains both with the full-catalogue cross-entropy (FusedTrainer(loss="ce")) instead of the BCE.
+`--loss gbce [--negatives K] [--t T]` trains both with gSASRec's gBCE (FusedTrainer(loss="gbce")); every rank draws the
+same K negatives per step, so the check is the same.  Its loss is about K times the BCE's, so its bound is relative."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -35,11 +37,15 @@ use_graph = os.environ.get("DP_CHECK_GRAPH", "0") == "1"
 l2_emb = float(sys.argv[sys.argv.index("--l2") + 1]) if "--l2" in sys.argv else 0.0
 topk_k = int(sys.argv[sys.argv.index("--topk-k") + 1]) if "--topk-k" in sys.argv else 10
 loss = sys.argv[sys.argv.index("--loss") + 1] if "--loss" in sys.argv else "bce"
-tr_dp = FusedTrainer(m_dp, process_group=dist.group.WORLD, use_graph=use_graph, l2_emb=l2_emb, loss=loss)
+gb = {}
+if loss == "gbce":
+    gb = dict(num_negatives=int(sys.argv[sys.argv.index("--negatives") + 1]) if "--negatives" in sys.argv else 256,
+              gbce_t=float(sys.argv[sys.argv.index("--t") + 1]) if "--t" in sys.argv else 0.75)
+tr_dp = FusedTrainer(m_dp, process_group=dist.group.WORLD, use_graph=use_graph, l2_emb=l2_emb, loss=loss, **gb)
 if rank == 0:
     print("fused reduce-scatter/Adam/all-gather kernel:", tr_dp._dp is not None, "graph:", use_graph, "l2_emb:", l2_emb,
-          "loss:", loss)
-tr_one = FusedTrainer(m_one, use_graph=False, l2_emb=l2_emb, loss=loss)
+          "loss:", loss, gb)
+tr_one = FusedTrainer(m_one, use_graph=False, l2_emb=l2_emb, loss=loss, **gb)
 ok = True
 for i, nb in enumerate(batches):
     full = {k: torch.from_numpy(v).to(dev) for k, v in nb.items()}
@@ -49,7 +55,7 @@ for i, nb in enumerate(batches):
     l2 = float(tr_dp.step(sh, w_pos=sh["w"]))
     if rank == 0:
         print(f"loss single {l1:.6f}  dp{world} {l2:.6f}")
-    ok &= abs(l1 - l2) < 2e-3
+    ok &= abs(l1 - l2) < 2e-3 * (max(1.0, abs(l1)) if loss == "gbce" else 1.0)
     if i == 0:                      # the first step's parameters, before Adam amplifies bf16 noise into sign flips
         d0 = float((m_one.flat_parameters().data - m_dp.flat_parameters().data).abs().max())
         if rank == 0:

@@ -1,8 +1,8 @@
 """Host-order trace of every library call the encoder makes, in a form that does not depend on addresses.
 
 For each configuration of a fixed matrix (model kind and widths, heads, maxlen, dropout, the SRFRD_* switches) and each
-entry path (the autograd model call + backward, an eval forward, encode_last, eager FusedTrainer steps with loss "bce"
-and "ce", each on the dense and the packed token layout where it has one), every call into libsrfrd_b200.so is written
+entry path (the autograd model call + backward, an eval forward, encode_last, eager FusedTrainer steps with loss "bce",
+"ce" and "gbce", each on the dense and the packed token layout where it has one), every call into libsrfrd_b200.so is written
 as one line:
   - the entry point's name;
   - the stream it was enqueued on: "main", "side", "side2" (HotPath's branch streams) or "comm" (FusedTrainer's);
@@ -181,8 +181,8 @@ def run_config(make, L, seed):
     trace("eval forward", eval_fwd)
     trace("encode_last dense", lambda: encode_last(False))
     trace("encode_last packed", lambda: encode_last(True))
-    for loss in ("bce", "ce"):
-        if loss == "ce" and s.kind == "SRFRN":
+    for loss in ("bce", "ce", "gbce"):
+        if loss != "bce" and s.kind == "SRFRN":
             continue
         for packed in (False, True):
             tr = FusedTrainer(m, use_graph=False, packed=packed, loss=loss)
