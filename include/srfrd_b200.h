@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define SRFRD_ABI_VERSION 11
+#define SRFRD_ABI_VERSION 12
 #if defined(__GNUC__)
 #define SRFRD_API __attribute__((visibility("default")))
 #else
@@ -201,6 +201,20 @@ SRFRD_API int srfrd_adam_step(float* p, float* g, float* m, float* v, int64_t n,
 SRFRD_API int srfrd_adam_step_fused(float* p, float* g, float* m, float* v, int64_t n, float lr, float beta1, float beta2,
                           float eps, float* state8, int zero_grad, float* acc2, const float* norm2, float* loss,
                           void* stream, const int64_t* l2_seg, int l2_n_seg, const float* l2_coef, const float* l2_reg);
+
+/* ---- lazy Adam for the item table (FusedTrainer(lazy_item_adam=True)) ----
+ * srfrd_touch_rows: stamp[id] = epoch for every id of the int64 arrays a, b, c (n_tok ids each) and list (n_list ids)
+ * with 1 <= id <= n_items; other ids and null arrays are skipped.  epoch = the uint32 step bits of state8[3] + 1, i.e. the
+ * epoch of the Adam launch that ends this step; stamps start at 0 and are never cleared.  stamp holds n_items + 1 words.
+ * srfrd_adam_step_fused_rows: srfrd_adam_step_fused (no l2 term) with the item table -- table_rows x D floats at float
+ * table_off of the flat buffer (4-aligned; n a multiple of 4) -- updated only on rows with stamp[row] == epoch: those get
+ * exactly the dense arithmetic (bias corrections of the global step) and a zeroed gradient, every other table row keeps
+ * p, m and v bit for bit and is not read.  The rest of the buffer, the tick and the loss read-out are as in the dense call. */
+SRFRD_API int srfrd_touch_rows(const int64_t* a, const int64_t* b, const int64_t* c, int64_t n_tok, const int64_t* list,
+                     int64_t n_list, int64_t n_items, uint32_t* stamp, const float* state8, void* stream);
+SRFRD_API int srfrd_adam_step_fused_rows(float* p, float* g, float* m, float* v, int64_t n, float lr, float beta1, float beta2,
+                               float eps, float* state8, int zero_grad, float* acc2, const float* norm2, float* loss,
+                               int64_t table_off, int64_t table_rows, int D, const uint32_t* stamp, void* stream);
 
 /* ---- l2_emb regulariser: per-tensor L2 norms of the flat parameter buffer (replaces: trainer.py:37-39) ----
  * seg = {offset, numel} per parameter tensor (int64 pairs, offsets 4-aligned and increasing, the gaps between tensors
@@ -482,6 +496,14 @@ SRFRD_API int srfrd_dp_adam_step(float* const* grad_ptrs_dev, float* const* para
                        int rank, int world, int64_t n, float* m, float* v, float lr, float beta1, float beta2, float eps,
                        float* state8, const float* norm2, uint32_t* local4, void* stream, const int64_t* l2_seg,
                        int l2_n_seg, const float* l2_coef, const float* l2_reg);
+/* srfrd_dp_adam_step (no l2 term) with the lazy item table of srfrd_adam_step_fused_rows: a table row of the owned slice
+ * is reduced, updated, broadcast and zeroed only when some rank stamped it this step (stamp_ptrs_dev: device array of
+ * `world` peer-mapped stamp arrays); the other rows move no data.  D must be a multiple of 4 (rows are whole float4s).
+ * With world == 1 it is the same arithmetic as srfrd_adam_step_fused_rows. */
+SRFRD_API int srfrd_dp_adam_step_rows(float* const* grad_ptrs_dev, float* const* param_ptrs_dev,
+                            uint32_t* const* signal_ptrs_dev, int rank, int world, int64_t n, float* m, float* v, float lr,
+                            float beta1, float beta2, float eps, float* state8, const float* norm2, uint32_t* local4,
+                            int64_t table_off, int64_t table_rows, int D, uint32_t* const* stamp_ptrs_dev, void* stream);
 
 #ifdef __cplusplus
 }

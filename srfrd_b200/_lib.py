@@ -79,6 +79,8 @@ SIGNATURES = {
     "srfrd_adam_tick": [vp, f32, f32, vp],
     "srfrd_adam_step": [vp, vp, vp, vp, i64, f32, f32, f32, f32, vp, i32, vp],
     "srfrd_adam_step_fused": [vp, vp, vp, vp, i64, f32, f32, f32, f32, vp, i32, vp, vp, vp, vp, vp, i32, vp, vp],
+    "srfrd_touch_rows": [vp, vp, vp, i64, vp, i64, i64, vp, vp, vp],
+    "srfrd_adam_step_fused_rows": [vp, vp, vp, vp, i64, f32, f32, f32, f32, vp, i32, vp, vp, vp, i64, i64, i32, vp, vp],
     "srfrd_param_l2_plan": [C.POINTER(i64), i32, C.POINTER(i64)],
     "srfrd_param_l2": [vp, vp, i32, i64, f32, vp, vp, vp, vp],
     "srfrd_catalogue_topk_plan": [i64, i64, i64, i32, i32, C.POINTER(i32), i32],
@@ -99,6 +101,7 @@ SIGNATURES = {
     "srfrd_unpack_rows": [C.POINTER(RepackPart), i32, C.POINTER(PackDesc), i64, i32, vp],
     "srfrd_pack_rows": [C.POINTER(RepackPart), i32, C.POINTER(PackDesc), i64, i32, vp],
     "srfrd_dp_adam_step": [vp, vp, vp, i32, i32, i64, vp, vp, f32, f32, f32, f32, vp, vp, vp, vp, vp, i32, vp, vp],
+    "srfrd_dp_adam_step_rows": [vp, vp, vp, i32, i32, i64, vp, vp, f32, f32, f32, f32, vp, vp, vp, i64, i64, i32, vp, vp],
     "srfrd_pack_plan": [vp, vp, i64, i32, C.POINTER(PackDesc), vp],
     "srfrd_set_row_limit": [vp],
     "srfrd_embed_ln_fwd_packed": [vp, i64, i32, vp, vp, i64, i32, i32, vp, vp, i64, i32, f32, vp, vp, f32, vp, vp, vp, i32,
@@ -140,7 +143,7 @@ def load() -> C.CDLL:
         fn = getattr(lib, name)            # AttributeError if the symbol is not exported
         fn.argtypes = argtypes
         fn.restype = C.c_int
-    if lib.srfrd_abi_version() != 11:
+    if lib.srfrd_abi_version() != 12:
         raise RuntimeError("srfrd_b200: ABI version mismatch between _lib.py and the built library")
     _lib = lib
     return lib

@@ -403,4 +403,15 @@ __device__ __forceinline__ int l2_advance(const int64_t* s_off, int n_seg, int t
   return t;
 }
 
+// Lazy Adam over the item table (srfrd_adam_step_fused_rows, srfrd_dp_adam_step_rows): the table is rows x D floats
+// starting at float `off` (4-aligned) of the flat buffer, and only its rows whose epoch stamp (srfrd_touch_rows) equals
+// the step's epoch = uint32 step bits + 1 are read, updated and have their gradient zeroed.  Everything outside the
+// table is dense Adam.
+struct RowGate {
+  int64_t off;
+  int64_t rows;
+  int D;
+  const uint32_t* stamp;     // single GPU: this rank's stamps (the data-parallel kernel takes peer pointers instead)
+};
+
 }  // namespace srfrd

@@ -65,11 +65,66 @@ struct DpAdam {
   L2Segments l2s;            // l2_emb regulariser (L2 instantiation only)
 };
 
+// The ROWS part of dp_adam_kernel on the slice of float4s [lo, hi): the table rows overlapping the slice, 32 stamps per
+// warp, each row stamped by any rank updated by the whole warp.  D % 4 == 0 (srfrd_dp_adam_step_rows checks it): rows are
+// whole float4s, so the row walk runs the dense loop's float4 body and gives its bits.
+__device__ void dp_rows(const DpAdam& p, const RowGate& rg, uint32_t* const* stamp, int64_t lo, int64_t hi, uint32_t epoch,
+                        float step_size, float inv_sqrt_bc2) {
+  const int64_t tend = rg.off + rg.rows * rg.D;
+  const int64_t e_lo = max(4 * lo, rg.off), e_hi = min(4 * hi, tend);   // table floats of this slice
+  if (e_lo >= e_hi) return;
+  const int64_t r_lo = (e_lo - rg.off) / rg.D, r_hi = (e_hi - rg.off + rg.D - 1) / rg.D;
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t r0 = r_lo + warp * 32; r0 < r_hi; r0 += n_warps * 32) {
+    const int64_t r = r0 + lane;
+    bool mine = false;
+    if (r < r_hi)
+      for (int q = 0; q < p.world; ++q) mine |= __ldcg(stamp[q] + r) == epoch;
+    unsigned hit = __ballot_sync(0xffffffffu, mine);
+    while (hit) {
+      const int64_t e0 = rg.off + (r0 + __ffs(hit) - 1) * rg.D;
+      hit &= hit - 1;
+      const int64_t a = max(e0, e_lo), b = min(e0 + rg.D, e_hi);
+      for (int64_t i = (a >> 2) + lane; i < (b >> 2); i += 32) {
+        float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
+        for (int q = 0; q < p.world; ++q) {
+          const float4 t = __ldcg(reinterpret_cast<const float4*>(p.grad[q]) + i);
+          g.x += t.x; g.y += t.y; g.z += t.z; g.w += t.w;
+        }
+        float4 w = reinterpret_cast<const float4*>(p.param[p.rank])[i];
+        float4 mm = reinterpret_cast<float4*>(p.m)[i], vv = reinterpret_cast<float4*>(p.v)[i];
+        float* wa = &w.x; float* ga = &g.x; float* ma = &mm.x; float* va = &vv.x;
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+          ma[k] = p.beta1 * ma[k] + (1.f - p.beta1) * ga[k];
+          va[k] = p.beta2 * va[k] + (1.f - p.beta2) * ga[k] * ga[k];
+          wa[k] -= step_size * ma[k] / (sqrtf(va[k]) * inv_sqrt_bc2 + p.eps);
+        }
+        reinterpret_cast<float4*>(p.m)[i] = mm;
+        reinterpret_cast<float4*>(p.v)[i] = vv;
+        const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+        for (int q = 0; q < p.world; ++q) {
+          reinterpret_cast<float4*>(p.param[q])[i] = w;
+          reinterpret_cast<float4*>(p.grad[q])[i] = z;
+        }
+      }
+    }
+  }
+}
+
 // L2: g += coef[tensor] * p on the reduced gradient (added once, after the sum over ranks) and rank 0 adds reg to the loss.
-template <bool L2>
-__global__ void __launch_bounds__(DP_THREADS, 1) dp_adam_kernel(DpAdam p) {
+// ROWS (lazy item table, RowGate): in its slice, a rank skips the table's float4s in the dense loop and walks the table
+// rows that overlap the slice instead; a row is reduced, updated, broadcast and zeroed only when SOME rank stamped it in
+// this step (stamp[r][row] == epoch for any r), so the peer traffic of rows no rank looked up disappears.  Every float is
+// still computed by exactly one rank (the owner of its float4).  rg and stamp (a device array of every rank's stamp
+// pointers) are kernel arguments of their own: inside DpAdam they cost the dense instantiations registers.
+template <bool L2, bool ROWS>
+__global__ void __launch_bounds__(DP_THREADS, 1) dp_adam_kernel(DpAdam p, RowGate rg, uint32_t* const* stamp) {
   __shared__ float s_bc[2];
   __shared__ uint32_t s_epoch;
+  __shared__ uint32_t s_row_epoch;
   pdl_prologue_done();
   const int tid = threadIdx.x;
   int64_t* s_off = nullptr;
@@ -81,6 +136,7 @@ __global__ void __launch_bounds__(DP_THREADS, 1) dp_adam_kernel(DpAdam p) {
   }
   if (tid == 0) {
     s_epoch = p.local[0];
+    if constexpr (ROWS) s_row_epoch = __float_as_uint(p.state[3]) + 1u;
     const float step = p.state[0] + 1.f;
     s_bc[0] = (float)(1.0 - pow((double)p.beta1, (double)step));
     s_bc[1] = (float)(1.0 - pow((double)p.beta2, (double)step));
@@ -114,7 +170,14 @@ __global__ void __launch_bounds__(DP_THREADS, 1) dp_adam_kernel(DpAdam p) {
   }
   int sg = 0;
   if constexpr (L2) sg = l2_find(s_off, p.l2s.n_seg, lo + (int64_t)blockIdx.x * blockDim.x + tid);
-  for (int64_t i = lo + (int64_t)blockIdx.x * blockDim.x + tid; i < hi; i += (int64_t)gridDim.x * blockDim.x) {
+  // ROWS: the table's float4s [x0, x0 + skip) of this slice are left to the row walk below; j counts the others
+  int64_t x0 = hi, skip = 0;
+  if constexpr (ROWS) {
+    x0 = max(lo, rg.off >> 2);
+    skip = max((int64_t)0, min(hi, (rg.off + rg.rows * rg.D + 3) >> 2) - x0);
+  }
+  for (int64_t j = lo + (int64_t)blockIdx.x * blockDim.x + tid; j < hi - skip; j += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t i = ROWS && j >= x0 ? j + skip : j;
     float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
     for (int r = 0; r < DP_MAX_WORLD; ++r)
@@ -144,6 +207,7 @@ __global__ void __launch_bounds__(DP_THREADS, 1) dp_adam_kernel(DpAdam p) {
     for (int r = 0; r < DP_MAX_WORLD; ++r)
       if (r < p.world) { pp_[r][i] = w; gp[r][i] = z; }
   }
+  if constexpr (ROWS) dp_rows(p, rg, stamp, lo, hi, s_row_epoch, step_size, inv_sqrt_bc2);
   // ---- 3. loss (rank 0 owns the bucket's tail)
   if (p.rank == 0 && blockIdx.x == 0 && tid == 0) {
     float a = 0.f, b = 0.f;
@@ -198,9 +262,40 @@ extern "C" int srfrd_dp_adam_step(float* const* grad_ptrs_dev, float* const* par
   if (grid < 1) grid = 1;
   if (grid > num_sms()) grid = num_sms();            // every block must be resident (in-kernel grid barrier)
   if (l2)
-    SRFRD_CUDA(launch_pdl(dp_adam_kernel<true>, dim3((unsigned)grid), dim3(DP_THREADS), 0, (cudaStream_t)stream, p));
+    SRFRD_CUDA(launch_pdl(dp_adam_kernel<true, false>, dim3((unsigned)grid), dim3(DP_THREADS), 0, (cudaStream_t)stream, p,
+                          RowGate{}, (uint32_t* const*)nullptr));
   else
-    SRFRD_CUDA(launch_pdl(dp_adam_kernel<false>, dim3((unsigned)grid), dim3(DP_THREADS), 0, (cudaStream_t)stream, p));
+    SRFRD_CUDA(launch_pdl(dp_adam_kernel<false, false>, dim3((unsigned)grid), dim3(DP_THREADS), 0, (cudaStream_t)stream, p,
+                          RowGate{}, (uint32_t* const*)nullptr));
+  SRFRD_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int srfrd_dp_adam_step_rows(float* const* grad_ptrs_dev, float* const* param_ptrs_dev,
+                                       uint32_t* const* signal_ptrs_dev, int rank, int world, int64_t n, float* m, float* v,
+                                       float lr, float beta1, float beta2, float eps, float* state8, const float* norm2,
+                                       uint32_t* local4, int64_t table_off, int64_t table_rows, int D,
+                                       uint32_t* const* stamp_ptrs_dev, void* stream) {
+  SRFRD_REQUIRE(grad_ptrs_dev && param_ptrs_dev && signal_ptrs_dev && m && v && state8 && norm2 && local4 && stamp_ptrs_dev,
+                "dp_adam_step_rows: null pointer");
+  SRFRD_REQUIRE(world >= 1 && world <= DP_MAX_WORLD && rank >= 0 && rank < world, "dp_adam_step_rows: bad rank %d / world %d",
+                rank, world);
+  SRFRD_REQUIRE(n > 0 && n % 4 == 0, "dp_adam_step_rows: n must be a positive multiple of 4");
+  SRFRD_REQUIRE(table_off % 4 == 0 && table_off >= 0 && table_rows >= 0 && D >= 4 && D % 4 == 0 &&
+                table_off + table_rows * D <= n,
+                "dp_adam_step_rows: the table (offset %lld, %lld x %d) must start 4-aligned inside n = %lld, D a multiple of 4",
+                (long long)table_off, (long long)table_rows, D, (long long)n);
+  DpAdam p;
+  p.grad = grad_ptrs_dev; p.param = param_ptrs_dev; p.sig = signal_ptrs_dev; p.rank = rank; p.world = world; p.n = n;
+  p.m = m; p.v = v; p.lr = lr; p.beta1 = beta1; p.beta2 = beta2; p.eps = eps; p.state = state8; p.norm = norm2; p.local = local4;
+  p.l2s = L2Segments{};
+  const int64_t slice4 = (n / 4 + world - 1) / world;
+  const int64_t slice_rows = (table_rows + world - 1) / world;
+  int64_t grid = ((slice4 > slice_rows ? slice4 : slice_rows) + DP_THREADS - 1) / DP_THREADS;
+  if (grid < 1) grid = 1;
+  if (grid > num_sms()) grid = num_sms();            // every block must be resident (in-kernel grid barrier)
+  SRFRD_CUDA(launch_pdl(dp_adam_kernel<false, true>, dim3((unsigned)grid), dim3(DP_THREADS), 0, (cudaStream_t)stream, p,
+                        RowGate{table_off, table_rows, D, nullptr}, stamp_ptrs_dev));
   SRFRD_LAUNCH_CHECK();
   return 0;
 }

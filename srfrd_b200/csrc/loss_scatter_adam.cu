@@ -453,17 +453,23 @@ __global__ void __launch_bounds__(L2_THREADS) param_l2_kernel(const float* __res
 // block to finish publishes it -- by then every block has read the old state -- and block 0 finalises the loss.
 // state8 = {step, 1 - beta1^step, 1 - beta2^step, uint32 step bits, int blocks-done counter, -, -, -}.
 // L2: g += coef[tensor] * p (the gradient of l2 * ||p_t||, from the parameters before this update) and loss += reg.
-template <bool L2>
+// ROWS (lazy item-table Adam, RowGate): the grid-stride loop skips the table's float4s, the non-table floats of a float4
+// the table ends in are done one by one, and the table is walked row-parallel over its stamps: each warp loads 32 stamps,
+// and every stamped row among them is updated by the whole warp.  Same per-element arithmetic as the dense loop, so a
+// stamped row gets exactly the dense update; an unstamped row is not read (its gradient is zero: no kernel wrote it).
+template <bool L2, bool ROWS>
 __global__ void __launch_bounds__(256) adam_fused_kernel(float* __restrict__ p, float* __restrict__ g, float* __restrict__ m,
                                                          float* __restrict__ v, int64_t n, float lr, float beta1, float beta2,
                                                          float eps, float* state, int zero_grad, float* acc, const float* norm,
-                                                         float* loss, L2Segments l2s) {
+                                                         float* loss, L2Segments l2s, RowGate rg) {
   __shared__ float s_bc[2];
+  __shared__ uint32_t s_epoch;
   pdl_prologue_done();
   if (threadIdx.x == 0) {
     const float step = state[0] + 1.f;
     s_bc[0] = (float)(1.0 - pow((double)beta1, (double)step));
     s_bc[1] = (float)(1.0 - pow((double)beta2, (double)step));
+    if constexpr (ROWS) s_epoch = __float_as_uint(state[3]) + 1u;
   }
   if (blockIdx.x == 0 && threadIdx.x == 32 && acc) {
     const float a = norm[0] > 0.f ? acc[0] / norm[0] : 0.f;
@@ -485,7 +491,14 @@ __global__ void __launch_bounds__(256) adam_fused_kernel(float* __restrict__ p, 
   const int64_t n4 = n >> 2;
   int t = 0;
   if constexpr (L2) t = l2_find(s_off, l2s.n_seg, (int64_t)blockIdx.x * blockDim.x + threadIdx.x);
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
+  // ROWS: the table's float4s [t0, t1) are left to the row walk below; j counts the others
+  int64_t t0 = 0, skip = 0;
+  if constexpr (ROWS) {
+    t0 = rg.off >> 2;
+    skip = ((rg.off + rg.rows * rg.D + 3) >> 2) - t0;
+  }
+  for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < n4 - skip; j += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t i = ROWS && j >= t0 ? j + skip : j;
     float4 pp = reinterpret_cast<float4*>(p)[i], gg = reinterpret_cast<float4*>(g)[i];
     float4 mm = reinterpret_cast<float4*>(m)[i], vv = reinterpret_cast<float4*>(v)[i];
     float* pa = &pp.x; float* ga = &gg.x; float* ma = &mm.x; float* va = &vv.x;
@@ -513,6 +526,53 @@ __global__ void __launch_bounds__(256) adam_fused_kernel(float* __restrict__ p, 
     p[i] -= step_size * m[i] / (sqrtf(v[i]) * inv_sqrt_bc2 + eps);
     if (zero_grad) g[i] = 0.f;
   }
+  if constexpr (ROWS) {
+    const int64_t tend = rg.off + rg.rows * rg.D;
+    // the float4 the table ends in: its floats past the table are dense
+    if (blockIdx.x == 0 && threadIdx.x < ((4 - (tend & 3)) & 3)) {
+      const int64_t i = tend + threadIdx.x;
+      m[i] = beta1 * m[i] + (1.f - beta1) * g[i];
+      v[i] = beta2 * v[i] + (1.f - beta2) * g[i] * g[i];
+      p[i] -= step_size * m[i] / (sqrtf(v[i]) * inv_sqrt_bc2 + eps);
+      if (zero_grad) g[i] = 0.f;
+    }
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    const uint32_t epoch = s_epoch;
+    for (int64_t r0 = warp * 32; r0 < rg.rows; r0 += n_warps * 32) {
+      const int64_t r = r0 + lane;
+      unsigned hit = __ballot_sync(0xffffffffu, r < rg.rows && __ldcg(rg.stamp + r) == epoch);
+      while (hit) {
+        const int64_t e0 = rg.off + (r0 + __ffs(hit) - 1) * rg.D;
+        hit &= hit - 1;
+        if ((rg.D & 3) == 0) {
+          for (int64_t i = (e0 >> 2) + lane; i < ((e0 + rg.D) >> 2); i += 32) {
+            float4 pp = reinterpret_cast<float4*>(p)[i], gg = reinterpret_cast<float4*>(g)[i];
+            float4 mm = reinterpret_cast<float4*>(m)[i], vv = reinterpret_cast<float4*>(v)[i];
+            float* pa = &pp.x; float* ga = &gg.x; float* ma = &mm.x; float* va = &vv.x;
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+              ma[q] = beta1 * ma[q] + (1.f - beta1) * ga[q];
+              va[q] = beta2 * va[q] + (1.f - beta2) * ga[q] * ga[q];
+              pa[q] -= step_size * ma[q] / (sqrtf(va[q]) * inv_sqrt_bc2 + eps);
+            }
+            reinterpret_cast<float4*>(p)[i] = pp;
+            reinterpret_cast<float4*>(m)[i] = mm;
+            reinterpret_cast<float4*>(v)[i] = vv;
+            if (zero_grad) reinterpret_cast<float4*>(g)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+          }
+        } else {                                           // D % 4 != 0: rows straddle float4s, one float per lane
+          for (int64_t i = e0 + lane; i < e0 + rg.D; i += 32) {
+            m[i] = beta1 * m[i] + (1.f - beta1) * g[i];
+            v[i] = beta2 * v[i] + (1.f - beta2) * g[i] * g[i];
+            p[i] -= step_size * m[i] / (sqrtf(v[i]) * inv_sqrt_bc2 + eps);
+            if (zero_grad) g[i] = 0.f;
+          }
+        }
+      }
+    }
+  }
   __syncthreads();
   if (threadIdx.x == 0) {
     int* done = reinterpret_cast<int*>(state + 4);
@@ -523,6 +583,25 @@ __global__ void __launch_bounds__(256) adam_fused_kernel(float* __restrict__ p, 
       state[2] = s_bc[1];
       state[3] = __uint_as_float(__float_as_uint(state[3]) + 1u);
     }
+  }
+}
+
+// Lazy item-table Adam, part 1: stamp[id] = epoch for every id in 1..n_items of the step's id arrays (a, b, c: n_tok ids
+// each; list: n_list ids; null arrays are skipped).  epoch = the uint32 step bits + 1 = the value the next Adam launch
+// compares with, so nothing is ever cleared and a replayed graph stamps a new epoch without the host.
+__global__ void __launch_bounds__(256) touch_rows_kernel(const int64_t* __restrict__ a, const int64_t* __restrict__ b,
+                                                         const int64_t* __restrict__ c, int64_t n_tok,
+                                                         const int64_t* __restrict__ list, int64_t n_list, int64_t n_items,
+                                                         uint32_t* __restrict__ stamp, const float* __restrict__ state) {
+  pdl_prologue_done();
+  const uint32_t epoch = __float_as_uint(state[3]) + 1u;
+  const int64_t total = 3 * n_tok + n_list;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t s = i / n_tok < 3 && n_tok > 0 ? i / n_tok : 3;
+    const int64_t* src = s == 0 ? a : s == 1 ? b : s == 2 ? c : list;
+    if (!src) continue;
+    const int64_t id = src[s < 3 ? i - s * n_tok : i - 3 * n_tok];
+    if (id >= 1 && id <= n_items) stamp[id] = epoch;
   }
 }
 
@@ -755,11 +834,48 @@ extern "C" int srfrd_adam_step_fused(float* p, float* g, float* m, float* v, int
   if (blocks > num_sms() * 8) blocks = num_sms() * 8;
   const L2Segments l2s{l2_seg, l2_n_seg, l2_coef, l2_reg};
   if (l2)
-    SRFRD_CUDA(launch_pdl(adam_fused_kernel<true>, dim3((unsigned)blocks), dim3(256), 0, (cudaStream_t)stream, p, g, m, v, n,
-                          lr, beta1, beta2, eps, state8, zero_grad, acc2, norm2, loss, l2s));
+    SRFRD_CUDA(launch_pdl(adam_fused_kernel<true, false>, dim3((unsigned)blocks), dim3(256), 0, (cudaStream_t)stream, p, g, m,
+                          v, n, lr, beta1, beta2, eps, state8, zero_grad, acc2, norm2, loss, l2s, RowGate{}));
   else
-    SRFRD_CUDA(launch_pdl(adam_fused_kernel<false>, dim3((unsigned)blocks), dim3(256), 0, (cudaStream_t)stream, p, g, m, v, n,
-                          lr, beta1, beta2, eps, state8, zero_grad, acc2, norm2, loss, l2s));
+    SRFRD_CUDA(launch_pdl(adam_fused_kernel<false, false>, dim3((unsigned)blocks), dim3(256), 0, (cudaStream_t)stream, p, g, m,
+                          v, n, lr, beta1, beta2, eps, state8, zero_grad, acc2, norm2, loss, l2s, RowGate{}));
+  SRFRD_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int srfrd_touch_rows(const int64_t* a, const int64_t* b, const int64_t* c, int64_t n_tok, const int64_t* list,
+                                int64_t n_list, int64_t n_items, uint32_t* stamp, const float* state8, void* stream) {
+  SRFRD_REQUIRE(stamp && state8, "touch_rows: null pointer");
+  SRFRD_REQUIRE(n_tok >= 0 && n_list >= 0 && n_items >= 0, "touch_rows: negative count");
+  SRFRD_REQUIRE(n_list == 0 || list, "touch_rows: n_list > 0 needs the list");
+  const int64_t total = 3 * n_tok + n_list;
+  if (total == 0) return 0;
+  int64_t blocks = (total + 255) / 256;
+  if (blocks > num_sms() * 8) blocks = num_sms() * 8;
+  SRFRD_CUDA(launch_pdl(touch_rows_kernel, dim3((unsigned)blocks), dim3(256), 0, (cudaStream_t)stream, a, b, c, n_tok, list,
+                        n_list, n_items, stamp, state8));
+  SRFRD_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int srfrd_adam_step_fused_rows(float* p, float* g, float* m, float* v, int64_t n, float lr, float beta1,
+                                          float beta2, float eps, float* state8, int zero_grad, float* acc2,
+                                          const float* norm2, float* loss, int64_t table_off, int64_t table_rows, int D,
+                                          const uint32_t* stamp, void* stream) {
+  SRFRD_REQUIRE(p && g && m && v && state8 && stamp, "adam_step_fused_rows: null pointer");
+  SRFRD_REQUIRE(!acc2 || (norm2 && loss), "adam_step_fused_rows: the loss read-out needs norm and loss");
+  SRFRD_REQUIRE((((uintptr_t)p | (uintptr_t)g | (uintptr_t)m | (uintptr_t)v) & 15) == 0,
+                "adam_step_fused_rows: buffers must be 16-byte aligned");
+  SRFRD_REQUIRE(n % 4 == 0 && table_off % 4 == 0 && table_off >= 0 && table_rows >= 0 && D >= 1 &&
+                table_off + table_rows * D <= n,
+                "adam_step_fused_rows: the table (offset %lld, %lld x %d) must start 4-aligned inside n = %lld (a multiple of 4)",
+                (long long)table_off, (long long)table_rows, D, (long long)n);
+  const int64_t dense4 = n / 4 - (((table_off + table_rows * D + 3) >> 2) - (table_off >> 2));
+  int64_t blocks = (dense4 > table_rows ? dense4 : table_rows) / 256 + 1;
+  if (blocks > num_sms() * 8) blocks = num_sms() * 8;
+  SRFRD_CUDA(launch_pdl(adam_fused_kernel<false, true>, dim3((unsigned)blocks), dim3(256), 0, (cudaStream_t)stream, p, g, m, v,
+                        n, lr, beta1, beta2, eps, state8, zero_grad, acc2, norm2, loss, L2Segments{},
+                        RowGate{table_off, table_rows, D, stamp}));
   SRFRD_LAUNCH_CHECK();
   return 0;
 }

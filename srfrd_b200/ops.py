@@ -225,6 +225,34 @@ def adam_step_fused(p, g, m, v, lr, beta1, beta2, eps, state8, zero_grad=True, a
          _p(state8), int(zero_grad), _p(acc2), _p(norm2), _p(loss), _stream(), *_l2_args(l2))
 
 
+def touch_rows(stamp, state8, n_items: int, a=None, b=None, c=None, ids=None):
+    """Lazy item-table Adam: stamp[id] = epoch (the uint32 step bits of state8 + 1) for every id in 1..n_items of the int64
+    arrays a, b, c (same numel) and ids; stamp is an int32 / uint32 tensor of n_items + 1 words."""
+    _lib.require_device()
+    toks = [t for t in (a, b, c) if t is not None]
+    n_tok = toks[0].numel() if toks else 0
+    for t in toks + ([ids] if ids is not None else []):
+        _chk(t, torch.int64, "ids")
+        if not t.is_contiguous():
+            raise RuntimeError("srfrd_b200: touch_rows id arrays must be contiguous")
+    if any(t.numel() != n_tok for t in toks):
+        raise RuntimeError("srfrd_b200: touch_rows a, b and c must hold the same number of ids")
+    if stamp.numel() < n_items + 1:
+        raise RuntimeError(f"srfrd_b200: touch_rows needs {n_items + 1} stamps, got {stamp.numel()}")
+    call("srfrd_touch_rows", _p(a), _p(b), _p(c), n_tok, _p(ids), 0 if ids is None else ids.numel(), int(n_items),
+         _p(stamp), _p(state8), _stream())
+
+
+def adam_step_fused_rows(p, g, m, v, lr, beta1, beta2, eps, state8, table_off: int, table_rows: int, D: int, stamp,
+                         zero_grad=True, acc2=None, norm2=None, loss=None):
+    """adam_step_fused with the item table (table_rows x D floats at float table_off of p) updated only on the rows
+    ``touch_rows`` stamped in this step; every other row keeps p, m and v bit for bit."""
+    _lib.require_device()
+    call("srfrd_adam_step_fused_rows", _p(p), _p(g), _p(m), _p(v), p.numel(), float(lr), float(beta1), float(beta2),
+         float(eps), _p(state8), int(zero_grad), _p(acc2), _p(norm2), _p(loss), int(table_off), int(table_rows), int(D),
+         _p(stamp), _stream())
+
+
 class ParamL2:
     """The l2_emb regulariser's per-tensor norms over a flat parameter buffer (srfrd_param_l2): ``segments`` = the
     (offset, numel) of every parameter tensor in the buffer.  ``launch(p)`` writes ``coef[t] = l2 / ||p_t||`` (0 for a
@@ -463,6 +491,16 @@ def dp_adam_step(grad_ptrs_dev: int, param_ptrs_dev: int, signal_ptrs_dev: int, 
     _lib.require_device()
     call("srfrd_dp_adam_step", grad_ptrs_dev, param_ptrs_dev, signal_ptrs_dev, int(rank), int(world), int(n), _p(m), _p(v),
          float(lr), float(beta1), float(beta2), float(eps), _p(state8), _p(norm2), _p(local4), _stream(), *_l2_args(l2))
+
+
+def dp_adam_step_rows(grad_ptrs_dev: int, param_ptrs_dev: int, signal_ptrs_dev: int, rank, world, n, m, v, lr, beta1, beta2,
+                      eps, state8, norm2, local4, table_off: int, table_rows: int, D: int, stamp_ptrs_dev: int):
+    """dp_adam_step with the lazy item table of adam_step_fused_rows: stamp_ptrs_dev = device address of the array of
+    every rank's peer-mapped stamp pointers; a table row moves only when some rank stamped it this step."""
+    _lib.require_device()
+    call("srfrd_dp_adam_step_rows", grad_ptrs_dev, param_ptrs_dev, signal_ptrs_dev, int(rank), int(world), int(n), _p(m),
+         _p(v), float(lr), float(beta1), float(beta2), float(eps), _p(state8), _p(norm2), _p(local4), int(table_off),
+         int(table_rows), int(D), stamp_ptrs_dev, _stream())
 
 
 def _parts(parts):

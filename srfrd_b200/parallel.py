@@ -40,6 +40,15 @@ def allreduce_sum_(t: torch.Tensor, group=None) -> torch.Tensor:
     return t
 
 
+def union_row_stamps_(stamp: torch.Tensor, group=None) -> torch.Tensor:
+    """In-place MAX all-reduce of the lazy item-table Adam's int32 row stamps (no-op without a process group / at world
+    size 1).  The current step's epoch is the largest stamp any rank has written, so afterwards a row carries it on every
+    rank exactly when some rank looked the row up: the row set of the global batch, as one rank on B sequences sees it."""
+    if group is not None and dist.is_initialized() and dist.get_world_size(group) > 1:
+        dist.all_reduce(stamp, op=dist.ReduceOp.MAX, group=group)
+    return stamp
+
+
 def broadcast_parameters(flat_params: torch.Tensor, src: int = 0, group=None) -> None:
     if dist.is_initialized() and dist.get_world_size(group) > 1:
         dist.broadcast(flat_params, src, group=group)

@@ -110,15 +110,29 @@ class FusedTrainer:
                    A negative that occurs in a position's sequence (its seq or pos ids) is left out of that position's
                    loss.  Same discriminator weights and normaliser as the BCE; the kernels are csrc/gbce.cu.  Every
                    data-parallel rank draws the same negatives.  w_neg and SRFRN are refused as for "ce".
+    lazy_item_adam: update only the item-table rows the step looks up (SparseAdam's rule; default False = dense Adam
+                   over the whole flat buffer).  A step looks up the non-zero ids of the batch's seq, pos and neg for
+                   "bce", of seq and pos plus the drawn negatives for "gbce", and data parallel the union over ranks.
+                   Those rows get exactly the dense update (torch.optim.Adam's m_hat / (sqrt(v_hat) + eps), bias
+                   corrections of the trainer's global step) even when their gradient is zero; every other row keeps
+                   its parameters and moments bit for bit.  Every other parameter tensor stays dense.  When a step looks
+                   up every row, the result is bit-identical to the dense step.  Refused with l2_emb != 0 (the
+                   regulariser's gradient reaches every row) and with loss="ce" (every row is a candidate).
     """
 
     def __init__(self, model, lr: float = 1e-3, betas=(0.9, 0.98), eps: float = 1e-8, process_group=None,
                  use_graph: bool = True, l2_emb: float = 0.0, packed: Optional[bool] = None, loss: str = "bce",
-                 num_negatives: Optional[int] = None, gbce_t: Optional[float] = None):
+                 num_negatives: Optional[int] = None, gbce_t: Optional[float] = None, lazy_item_adam: bool = False):
         if loss not in ("bce", "ce", "gbce"):
             raise ValueError(f"unknown loss {loss!r} (expected 'bce', 'ce' or 'gbce')")
         if loss != "gbce" and (num_negatives is not None or gbce_t is not None):
             raise ValueError(f"num_negatives / gbce_t configure loss='gbce', not loss={loss!r}")
+        if lazy_item_adam and l2_emb != 0.0:
+            raise ValueError("lazy_item_adam needs l2_emb == 0: the regulariser's gradient reaches every item row on every "
+                             "step, so no row is left untouched")
+        if lazy_item_adam and loss == "ce":
+            raise ValueError("lazy_item_adam does not apply to loss='ce': every item is a candidate of every step, so every "
+                             "row is updated and lazy equals dense")
         if loss in ("ce", "gbce") and model.spec.kind == "SRFRN":
             raise ValueError(f"loss={loss!r} does not support SRFRN: its logits need each candidate's fake label "
                              "(SRFR_model.py:225-233), which unobserved items do not have")
@@ -131,9 +145,14 @@ class FusedTrainer:
             check_gbce(self.num_negatives, self.gbce_t, n_items, model.spec.D)
         self.loss_kind = loss
         self.model = model
+        self.lazy = bool(lazy_item_adam)
+        item_rows = dict(model.named_parameters())[model.spec.item_key].shape[0]
         self._dp = None
-        if process_group is not None and torch.distributed.get_world_size(process_group) > 1:
-            self._dp = self._setup_fused_dp(model, process_group)
+        # the fused data-parallel kernel's lazy row walk moves whole float4 rows (D % 4 == 0); other widths take the NCCL
+        # all-reduce + the single-GPU gated Adam, which handles any D
+        if process_group is not None and torch.distributed.get_world_size(process_group) > 1 and \
+                not (self.lazy and model.spec.D % 4):
+            self._dp = self._setup_fused_dp(model, process_group, item_rows if self.lazy else 0)
         self.eng: HotPath = model._sync_flat()
         self.P = self.eng.P
         self.spec = self.eng.spec
@@ -159,6 +178,12 @@ class FusedTrainer:
         self._gbce_ws: Optional[Dict[str, torch.Tensor]] = None
         if loss == "ce":
             self.eng.enable_ce_table()
+        # lazy item-table Adam: one uint32 epoch stamp per item row (srfrd_touch_rows); in symmetric memory under the fused
+        # data-parallel optimizer, which ORs every rank's stamps
+        self.stamp: Optional[torch.Tensor] = None
+        if self.lazy:
+            self.stamp = self._dp["stamp"] if self._dp is not None else torch.zeros(item_rows, dtype=torch.int32, device=dev)
+            self._table = (self.P.offsets[self.spec.item_key][0], item_rows, self.spec.D)
         self.P.grad_bucket.zero_()
         self.eng.refresh_shadows()
         self.steps = 0
@@ -206,11 +231,11 @@ class FusedTrainer:
 
     # ------------------------------------------------------------------
     @staticmethod
-    def _setup_fused_dp(model, pg):
+    def _setup_fused_dp(model, pg, stamp_rows: int = 0):
         """Place the flat parameter buffer and the gradient bucket in symmetric memory (mapped into every rank of the
         node) so that ONE kernel per rank can do reduce-scatter -> Adam -> all-gather through NVLink peer pointers
         (csrc/dp_adam.cu).  Returns None -- the NCCL all-reduce path stays -- when symmetric memory is unavailable or
-        SRFRD_FUSED_DP=0."""
+        SRFRD_FUSED_DP=0.  stamp_rows > 0 (lazy_item_adam): the item rows' epoch stamps are placed there too."""
         import os
         if os.environ.get("SRFRD_FUSED_DP", "1") == "0":
             return None
@@ -230,6 +255,11 @@ class FusedTrainer:
             dp = dict(g=int(hg.buffer_ptrs_dev), p=int(hp.buffer_ptrs_dev), s=int(hs.buffer_ptrs_dev), rank=int(hg.rank),
                       world=int(hg.world_size), keep=(hg, hp, hs, sig),
                       local=torch.zeros(4, dtype=torch.int32, device=dev))
+            if stamp_rows > 0:
+                stamp = symm.empty(stamp_rows, dtype=torch.int32, device=dev).zero_()
+                torch.cuda.synchronize()
+                hst = symm.rendezvous(stamp, gname)
+                dp.update(stamp=stamp, st=int(hst.buffer_ptrs_dev), keep=dp["keep"] + (hst, stamp))
             torch.cuda.synchronize()
             torch.distributed.barrier(group=pg)
             return dp
@@ -281,6 +311,10 @@ class FusedTrainer:
             ops.weight_sums(pos, w_pos, w_neg, norm)
             if self.pg is not None:
                 parallel.allreduce_sum_(norm, self.pg)
+            if self.lazy:
+                # the rows this step's forward and loss gather (gBCE leaves neg unused; its drawn ids are stamped below)
+                ops.touch_rows(self.stamp, eng.step_state, self._table[1] - 1, st["seq"].view(-1), pos,
+                               neg if self.loss_kind == "bce" else None)
             if self._l2 is not None:
                 # the norms of the parameters the previous step left behind, next to the forward pass; the join below
                 # orders them before Adam (in the fused data-parallel kernel, peers overwrite this buffer once this rank
@@ -309,6 +343,10 @@ class FusedTrainer:
             # the same (seed, step) on every data-parallel rank: every rank draws the same negatives
             ops.gbce_draw(E, gb["ids"], gb["nb"], gb["excl"][:B], st["seq"], st["pos"], seed=eng.drop_seed,
                           step=eng.step_state[3:4])
+            if self.lazy:
+                self.comm.wait_stream(torch.cuda.current_stream())
+                with torch.cuda.stream(self.comm):
+                    ops.touch_rows(self.stamp, eng.step_state, E.shape[0] - 1, ids=gb["ids"])
             ops.gbce_loss(hb, gb["nb"], gb["ids"], E, pos, w_pos, norm, gb["excl"], L,
                           gbce_beta(self.num_negatives, E.shape[0] - 1, self.gbce_t), acc, ws["dh"][:rows],
                           P.view(s.item_key, grad=True), gb["part"], plan)
@@ -319,7 +357,14 @@ class FusedTrainer:
             ops.score_loss_fused(ws["hfin"][:rows], P.view(s.item_key), ft, pos, neg, prs_, nrs_, w_pos, w_neg, norm, acc,
                                  ws["dh"][:rows], P.view(s.item_key, grad=True), eng.fake_table_grad())
         eng.backward(ws["dh"][:rows])
-        if self._dp is not None:
+        if self.lazy:
+            torch.cuda.current_stream().wait_stream(self.comm)           # every stamp of the step is written
+        if self._dp is not None and self.lazy:
+            d = self._dp
+            ops.dp_adam_step_rows(d["g"], d["p"], d["s"], d["rank"], d["world"], P.numel, self.m, self.v, self.lr,
+                                  self.betas[0], self.betas[1], self.eps, eng.step_state, norm, d["local"], *self._table,
+                                  d["st"])
+        elif self._dp is not None:
             # reduce-scatter -> Adam on this rank's slice -> all-gather of the new parameters + loss, one kernel over NVLink
             # peer memory (csrc/dp_adam.cu) instead of an NCCL all-reduce followed by the same Adam on every rank
             d = self._dp
@@ -328,9 +373,16 @@ class FusedTrainer:
         else:
             if self.pg is not None:
                 parallel.allreduce_sum_(P.grad_bucket, self.pg)           # ONE NCCL sum over NVLink: gradients + loss sums
-            # Adam tick + dense Adam + loss read-out (consumes acc: zero again for the next step) in one launch
-            ops.adam_step_fused(P.data, P.grad, self.m, self.v, self.lr, self.betas[0], self.betas[1], self.eps,
-                                eng.step_state, zero_grad=True, acc2=acc, norm2=norm, loss=loss, l2=self._l2)
+                if self.lazy:
+                    parallel.union_row_stamps_(self.stamp, self.pg)       # the rows of the global batch on every rank
+            if self.lazy:
+                ops.adam_step_fused_rows(P.data, P.grad, self.m, self.v, self.lr, self.betas[0], self.betas[1], self.eps,
+                                         eng.step_state, *self._table, self.stamp, zero_grad=True, acc2=acc, norm2=norm,
+                                         loss=loss)
+            else:
+                # Adam tick + dense Adam + loss read-out (consumes acc: zero again for the next step) in one launch
+                ops.adam_step_fused(P.data, P.grad, self.m, self.v, self.lr, self.betas[0], self.betas[1], self.eps,
+                                    eng.step_state, zero_grad=True, acc2=acc, norm2=norm, loss=loss, l2=self._l2)
         eng.refresh_shadows()
 
     # ------------------------------------------------------------------

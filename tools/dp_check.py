@@ -4,7 +4,9 @@ and row-sharded catalogue top-10 (NCCL all-gather + merge) == unsharded top-10.
 `--topk-k K` checks the sharded top-K (1 <= K <= 64) instead of the top-10.
 `--loss ce` trains both with the full-catalogue cross-entropy (FusedTrainer(loss="ce")) instead of the BCE.
 `--loss gbce [--negatives K] [--t T]` trains both with gSASRec's gBCE (FusedTrainer(loss="gbce")); every rank draws the
-same K negatives per step, so the check is the same.  Its loss is about K times the BCE's, so its bound is relative."""
+same K negatives per step, so the check is the same.  Its loss is about K times the BCE's, so its bound is relative.
+`--lazy` trains both with FusedTrainer(lazy_item_adam=True) (combinable with `--loss gbce`): the G ranks update the union
+of their batches' item rows, so they still reproduce one rank on the concatenated batch."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -41,6 +43,8 @@ gb = {}
 if loss == "gbce":
     gb = dict(num_negatives=int(sys.argv[sys.argv.index("--negatives") + 1]) if "--negatives" in sys.argv else 256,
               gbce_t=float(sys.argv[sys.argv.index("--t") + 1]) if "--t" in sys.argv else 0.75)
+if "--lazy" in sys.argv:
+    gb["lazy_item_adam"] = True
 tr_dp = FusedTrainer(m_dp, process_group=dist.group.WORLD, use_graph=use_graph, l2_emb=l2_emb, loss=loss, **gb)
 if rank == 0:
     print("fused reduce-scatter/Adam/all-gather kernel:", tr_dp._dp is not None, "graph:", use_graph, "l2_emb:", l2_emb,

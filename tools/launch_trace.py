@@ -2,8 +2,8 @@
 
 For each configuration of a fixed matrix (model kind and widths, heads, maxlen, dropout, the SRFRD_* switches) and each
 entry path (the autograd model call + backward, an eval forward, encode_last, eager FusedTrainer steps with loss "bce",
-"ce" and "gbce", each on the dense and the packed token layout where it has one), every call into libsrfrd_b200.so is written
-as one line:
+"ce" and "gbce", each on the dense and the packed token layout where it has one, then "bce" and "gbce" with
+lazy_item_adam=True), every call into libsrfrd_b200.so is written as one line:
   - the entry point's name;
   - the stream it was enqueued on: "main", "side", "side2" (HotPath's branch streams) or "comm" (FusedTrainer's);
   - every scalar argument;
@@ -187,6 +187,14 @@ def run_config(make, L, seed):
         for packed in (False, True):
             tr = FusedTrainer(m, use_graph=False, packed=packed, loss=loss)
             trace(f"trainer {loss} {'packed' if packed else 'dense'}", lambda: tr.step(b, w_pos=w),
+                  {tr.comm.cuda_stream: "comm"})
+    # lazy item-table Adam, after every other entry so that their allocations (and traces) are unchanged
+    for loss in ("bce", "gbce"):
+        if loss != "bce" and s.kind == "SRFRN":
+            continue
+        for packed in (False, True):
+            tr = FusedTrainer(m, use_graph=False, packed=packed, loss=loss, lazy_item_adam=True)
+            trace(f"trainer {loss} lazy {'packed' if packed else 'dense'}", lambda: tr.step(b, w_pos=w),
                   {tr.comm.cuda_stream: "comm"})
     return dict(meta=meta, entries=entries)
 
